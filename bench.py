@@ -15,6 +15,11 @@ bundle.  Rays are generated on the device (Philox), so nothing but the replicate
 
 After the timed region rank 0 traces a sub-sample of the SAME rays through the SAME field with the CPU oracle
 (oracle/, the checker) and prints the comparison under "parity".
+
+--dump-outputs DIR: rank 0 writes what the last timed step handed its caller as DIR/<name>.npy (float64): one file per
+detector channel (the image as ``image.result()`` returns it) and stats.npy (``engine.STAT_NAMES`` order), at most
+64 MB in all (see ``dump_outputs``).  Field and rays are seeded, so two builds run with the same arguments can be
+compared file for file.
 """
 import argparse
 import hashlib
@@ -74,7 +79,13 @@ def parse(argv=None):
                          "report them under extra.c5; auto = when 8 GPUs run the default C2 workload")
     ap.add_argument("--rtol", type=float, default=1e-3)
     ap.add_argument("--atol", type=float, default=1e-6)
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the detector images and stats of the last timed step to DIR/<name>.npy (float64, <= 64 MB)")
     a = ap.parse_args(argv)
+    if a.steps < 1:
+        ap.error("--steps must be at least 1")
+    if a.dump_outputs and a.impl != "ours":
+        ap.error("--dump-outputs writes the outputs of the CUDA arm (--impl ours)")
     grid, rays, bs = workload_defaults(a.workload)
     a.grid = grid if a.grid is None else a.grid
     a.rays = rays if a.rays is None else a.rays
@@ -512,6 +523,41 @@ def attach_ncu_static(roof, a, n_rays):
             pass
 
 
+# ------------------------------------------------------------------------------------------------- output dump
+DUMP_BYTES = 64_000_000
+_NPY_HEADER = 256          # upper bound of np.save's header for a 1-D or 2-D float64 array
+
+
+def dump_outputs(out_dir, arrays, budget=DUMP_BYTES):
+    """Write ``arrays`` (name -> array) as ``out_dir/<name>.npy`` in float64, ``budget`` bytes in all.  Arrays are
+    taken smallest first and each gets an equal share of what is left; one that does not fit its share is replaced by
+    its values at a fixed, seeded sample of flat indices (sorted, written beside it as ``<name>_index.npy``), so the
+    same outputs always produce the same files."""
+    os.makedirs(out_dir, exist_ok=True)
+    items = sorted(((k, np.asarray(v, dtype=np.float64)) for k, v in arrays.items()), key=lambda kv: kv[1].size)
+    left = budget
+    for i, (name, v) in enumerate(items):
+        share = left // (len(items) - i)
+        if v.nbytes + _NPY_HEADER <= share:
+            files = {name: v}
+        else:
+            k = (share - 2 * _NPY_HEADER) // 16                      # a float64 value and its float64 index per entry
+            idx = np.sort(np.random.default_rng(0).choice(v.size, size=k, replace=False))
+            files = {name: v.reshape(-1)[idx], name + "_index": idx.astype(np.float64)}
+        for fn, arr in files.items():
+            path = os.path.join(out_dir, fn + ".npy")
+            np.save(path, arr)
+            left -= os.path.getsize(path)
+
+
+def last_step_outputs(a, specs, stats):
+    """What one timed ``solve_and_image`` call hands its caller: each channel's image and the stats dict."""
+    from synthpy_b200 import engine
+    out = {name: s.image.result().cpu().numpy() for s, (name, _) in zip(specs, chain_names(a))}
+    out["stats"] = np.array([stats[k] for k in engine.STAT_NAMES], dtype=np.float64)
+    return out
+
+
 # ------------------------------------------------------------------------------------------------- our arm
 def run_c5_passes(a, rank, world, barrier, passes=2):
     """BASELINE configs[4] as a side measurement of a multi-GPU run: 1024^3 seed-3 field replicated on every GPU,
@@ -636,6 +682,8 @@ def run_ours(a):
         img_total = sum(int(s.image.total().sum().item()) for s in specs)
         allreduce_check = {"sum_images": img_total, "sum_rays_binned_over_ranks": int(tot[1].item()),
                            "equal": img_total == int(tot[1].item())}
+    if a.dump_outputs and rank == 0:                   # before the e2e passes below reuse the image buffers
+        dump_outputs(a.dump_outputs, last_step_outputs(a, specs, stats))
 
     # ---- e2e: host ray bundle in pinned memory -> H2D -> fused trace -> images D2H, every step
     e2e = None

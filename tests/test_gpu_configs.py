@@ -299,6 +299,34 @@ def test_bench_contract_on_a_small_workload():
     assert p["n"] == 500 and p["max_rel"] < 1e-9 and p["steps_equal"] and p["hist_equal"]
 
 
+def test_bench_dump_outputs_and_step_count(tmp_path):
+    """--steps sets the number of timed passes (launches scale with it), and --dump-outputs writes the same images and
+    stats for the same arguments whatever the step count: every pass traces the same seeded rays through the same field."""
+    import json
+    import os
+    import subprocess
+    import sys
+    root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+    lines = {}
+    for steps in (2, 3):
+        out = subprocess.run([sys.executable, os.path.join(root, "bench.py"), "--grid", "64", "--rays", "2e5", "--steps", str(steps),
+                              "--warmup", "3", "--no-cpu-baseline", "--no-parity", "--no-e2e", "--dump-outputs",
+                              str(tmp_path / f"s{steps}")], capture_output=True, text=True, timeout=900)
+        assert out.returncode == 0, out.stderr[-3000:]
+        lines[steps] = json.loads([l for l in out.stdout.strip().splitlines() if l.startswith("{")][0])
+        assert lines[steps]["steps"] == steps
+    assert lines[2]["gpu_launches"] * 3 == lines[3]["gpu_launches"] * 2 and lines[2]["gpu_launches"] > 0
+    files = sorted(os.listdir(tmp_path / "s2"))
+    assert files == ["schlieren_DF.npy", "schlieren_DF_index.npy", "shadow_two.npy", "shadow_two_index.npy", "stats.npy"]
+    assert sum(os.path.getsize(tmp_path / "s2" / f) for f in files) <= 64_000_000
+    for f in files:
+        a, b = np.load(tmp_path / "s2" / f), np.load(tmp_path / "s3" / f)
+        assert a.dtype == np.float64 and np.array_equal(a, b), f
+    stats = dict(zip(("ray_steps", "ray_steps_acc", "rays_capped", "rays_binned", "rays_rejected", "rhs_evals"),
+                     np.load(tmp_path / "s2" / "stats.npy")))
+    assert stats["ray_steps"] == lines[2]["ray_steps_per_pass_per_gpu"] and stats["rays_binned"] == lines[2]["rays_binned_last_pass"]
+
+
 def test_bench_C1_line():
     """--workload C1 (BASELINE configs[0], the reference's own CPU-runnable case) prints a full line with parity over ALL
     its rays' first 2000."""

@@ -220,6 +220,37 @@ def test_bench_parity_helpers_and_lattice():
         assert prm.h == h and prm.n_steps == n, w
 
 
+def test_bench_dump_outputs_budget_and_sample(tmp_path):
+    """bench.dump_outputs: float64 files within the byte budget, small arrays whole, a larger one as a fixed seeded sample
+    whose index file says where every value came from; the same arrays always give the same files."""
+    import bench
+    big = np.random.default_rng(1).integers(0, 50, size=(300, 500))
+    stats = np.arange(6)
+    for d in ("a", "b"):
+        bench.dump_outputs(str(tmp_path / d), {"img": big, "stats": stats}, budget=600_000)
+    files = sorted(os.listdir(tmp_path / "a"))
+    assert files == ["img.npy", "img_index.npy", "stats.npy"]
+    assert sum(os.path.getsize(tmp_path / "a" / f) for f in files) <= 600_000
+    got = {f: np.load(tmp_path / "a" / f) for f in files}
+    for f in files:
+        assert got[f].dtype == np.float64 and np.array_equal(got[f], np.load(tmp_path / "b" / f))
+    idx = got["img_index.npy"].astype(np.int64)
+    assert len(idx) > 30_000 and np.all(np.diff(idx) > 0)
+    assert np.array_equal(got["img.npy"], big.ravel()[idx]) and np.array_equal(got["stats.npy"], stats)
+    bench.dump_outputs(str(tmp_path / "c"), {"img": big, "stats": stats})
+    assert np.array_equal(np.load(tmp_path / "c" / "img.npy"), big)         # fits the default budget: written whole
+    assert sorted(os.listdir(tmp_path / "c")) == ["img.npy", "stats.npy"]
+
+
+def test_bench_rejects_step_counts_below_one_and_dumps_of_the_reference_arm():
+    import bench
+    import pytest
+    assert bench.parse(["--steps", "7"]).steps == 7
+    for argv in (["--steps", "0"], ["--impl", "reference", "--dump-outputs", "out"]):
+        with pytest.raises(SystemExit):
+            bench.parse(argv)
+
+
 def test_numa_binding_is_best_effort():
     """distributed.bind_to_local_numa never raises: without a GPU (or without sysfs NUMA information, as inside the GPU
     pool's containers: numa_node = -1) it reports that nothing was bound and the run proceeds unbound."""
