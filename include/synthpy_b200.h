@@ -143,6 +143,17 @@ typedef struct sp_optic_op {
 #define SP_PLANE_FRAC_BITS 40  /* interferogram planes hold round(value * 2^40): integer sums are exact and
                                  order-independent (run-to-run and GPU-count invariant images), quantisation
                                  9e-13 per contribution, range +-8.4e6 per pixel (|E| per ray is <= ~2)       */
+#define SP_IMG_STOKES 2        /* polarimetry: histogram bins (np.histogram2d semantics, as SP_IMG_HISTOGRAM) of the
+                                 ray count and of Stokes I, Q, U of the Jones vector E at the detector, summed
+                                 incoherently over the rays of a pixel:  I = |Ex|^2 + |Ey|^2,  Q = |Ex|^2 - |Ey|^2,
+                                 U = 2 Re(Ex conj(Ey)).  For the reference's E = amp e^{i phase} (-sin pol, cos pol)
+                                 (full_solver.py:883-890): I = amp^2, Q = -amp^2 cos 2pol, U = -amp^2 sin 2pol.
+                                 Stokes V = 2 Im(Ex conj(Ey)) is identically 0 for that Jones form: not stored.
+                                 planes_dev [4][ny][nx] int64: count, then I, Q, U in fixed point
+                                 (SP_STOKES_FRAC_BITS).  Channels must not contain SP_OP_REF_BEAM.            */
+#define SP_STOKES_FRAC_BITS 32 /* Stokes planes hold round(value * 2^32): quantisation 2.3e-10 per contribution,
+                                 range +-2^31 per pixel (2^31 unit contributions: every ray of a 1e9 bundle in
+                                 one pixel); a contribution beyond +-2^20 saturates                           */
 
 typedef struct sp_image {
     int32_t kind;
@@ -151,7 +162,8 @@ typedef struct sp_image {
     double x_lo, x_hi;        /* edges = np.linspace(lo, hi, nx+1) in both modes (digitize: nx = n_edges - 1)  */
     double y_lo, y_hi;
     uint64_t* counts_dev;     /* [ny][nx], histogram only (caller zeroes; calls accumulate)                  */
-    int64_t* planes_dev;      /* [4][ny][nx]: Re Ex, Im Ex, Re Ey, Im Ey, fixed point (SP_PLANE_FRAC_BITS)    */
+    int64_t* planes_dev;      /* [4][ny][nx], caller zeroes; calls accumulate.  Interferogram: Re Ex, Im Ex, Re Ey,
+                                 Im Ey (SP_PLANE_FRAC_BITS); Stokes: count, I, Q, U (SP_STOKES_FRAC_BITS)         */
 } sp_image;
 
 /* One detector channel: an optical train ending in an image.  Several channels can share one bundle of
@@ -166,12 +178,14 @@ typedef struct sp_channel {
 
 /* Optics + binning on exit rays that already exist in HBM: Diagnostic.*_solve() + histogram()/interferogram()
  * (diagnostics.py:388-640, rtm_solver.py:191-453).  rf_dev is 4 x n in METRES as returned by the solver
- * (m_to_mm is applied inside, diagnostics.py:313).  jf_dev (2 x n complex128 interleaved) may be NULL.
+ * (m_to_mm is applied inside, diagnostics.py:313).  jf_dev (2 x n complex128 interleaved) may be NULL, except for an
+ * interferogram or Stokes image.
  * rf_out_dev / jf_out_dev (may be NULL) receive the rays at the detector plane (NaN = rejected). */
 int sp_optics_image(const double* rf_dev, const double* jf_dev, uint64_t n, const sp_channel* chan,
                     double* rf_out_dev, double* jf_out_dev, void* stream);
 
-/* Interferogram magnitude  H = sqrt(Re(sum Ex)^2 + Re(sum Ey)^2)  (rtm_solver.py:450-453). */
+/* SP_IMG_INTERFEROGRAM: H_dev [ny][nx] = sqrt(Re(sum Ex)^2 + Re(sum Ey)^2)  (rtm_solver.py:450-453).
+ * SP_IMG_STOKES:        H_dev [4][ny][nx] float64 = N, I, Q, U (the fixed-point format stays inside the library). */
 int sp_image_finalize(const sp_image* img, double* H_dev, void* stream);
 
 /* ------------------------------------------------------------------------------------------- propagate */

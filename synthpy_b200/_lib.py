@@ -13,8 +13,9 @@ LIB_PATH = os.environ.get("SYNTHPY_B200_LIB") or os.path.join(_HERE, "csrc", "li
 FIELD_PHASE, FIELD_PHASE_F64 = 1, 2
 BEAM_CIRCULAR_FOLD, BEAM_CIRCULAR_POW2, BEAM_SQUARE, BEAM_RECTANGULAR, BEAM_LINEAR = range(5)
 OP_TRAVEL, OP_TRAVEL_NOE, OP_LENS, OP_CIRC_AP, OP_CIRC_STOP, OP_RECT_AP, OP_KNIFE, OP_REF_BEAM = range(8)
-IMG_HISTOGRAM, IMG_INTERFEROGRAM = 0, 1
+IMG_HISTOGRAM, IMG_INTERFEROGRAM, IMG_STOKES = 0, 1, 2
 PLANE_FRAC_BITS = 40          # SP_PLANE_FRAC_BITS: interferogram planes are int64 in units of 2^-40
+STOKES_FRAC_BITS = 32         # SP_STOKES_FRAC_BITS: Stokes I, Q, U planes are int64 in units of 2^-32
 METHOD_RK4, METHOD_RK45, METHOD_RK45_JOINT, METHOD_TSIT5 = 0, 1, 2, 6
 FLAG_PHASE, FLAG_EARLY_EXIT, FLAG_FP32, FLAG_PHASE_F64, FLAG_NO_SORT, FLAG_ATTEN, FLAG_FARADAY, FLAG_BUNDLE_STEP = 1, 2, 4, 8, 16, 32, 64, 128
 

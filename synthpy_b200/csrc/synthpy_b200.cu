@@ -368,8 +368,13 @@ static int channel_to_dev(const sp_channel* c, ChannelDev& d) {
     d.counts = (unsigned long long*)c->image.counts_dev; d.planes = (long long*)c->image.planes_dev;
     d.with_E = (c->image.kind == SP_IMG_INTERFEROGRAM);
     d.kwave = c->wavelength > 0 ? 2.0 * 3.14159265358979323846 / c->wavelength : 0.0;
+    if (d.kind < SP_IMG_HISTOGRAM || d.kind > SP_IMG_STOKES) return fail(SP_EINVAL, "unknown image kind");
     if (d.kind == SP_IMG_HISTOGRAM && !d.counts && d.nx > 0) return fail(SP_EINVAL, "histogram channel without counts buffer");
     if (d.kind == SP_IMG_INTERFEROGRAM && !d.planes && d.nx > 0) return fail(SP_EINVAL, "interferogram channel without planes buffer");
+    if (d.kind == SP_IMG_STOKES && !d.planes && d.nx > 0) return fail(SP_EINVAL, "Stokes channel without planes buffer");
+    if (d.kind == SP_IMG_STOKES)
+        for (int i = 0; i < d.n_ops; ++i)     // a reference beam added to Ey would be counted as a polarisation change
+            if (d.ops[i].kind == SP_OP_REF_BEAM) return fail(SP_EINVAL, "Stokes channel cannot contain a reference beam (ref_beam)");
     return SP_OK;
 }
 
@@ -380,19 +385,25 @@ static int channel_to_dev(const sp_channel* c, ChannelDev& d) {
 // SP_PLANE_FRAC_BITS fractional bits): integer addition is associative, so an image does not depend on the order in
 // which warps, kernels, chunks or GPUs contribute -- run-to-run and partition-to-partition identical, like the
 // counts -- at a quantisation of 2^-40 per contribution (|E| <= amp + 1 ~ 2; range +-2^23 per pixel).
+// Stokes: one 64-bit count and I, Q, U of the ray's Jones vector at the detector, fixed point with SP_STOKES_FRAC_BITS
+// fractional bits (a pixel holds +-2^31: 2^31 contributions of unit intensity).  The
+// optics are ray-transfer matrices and the E-phase advance multiplies both Jones components by the same unit factor,
+// so the Stokes parameters do not depend on it: Stokes channels run with with_E = 0.
 // Returns 1 if binned.
 // (a NaN amplitude contributes nothing -- the reference would poison the pixel with NaN -- and values beyond the
-// per-contribution range +-2^22 saturate instead of wrapping)
-__device__ __forceinline__ long long to_plane_fixed(double v) {
-    const double lim = 4194304.0;
+// per-contribution range (+-2^22 for interferogram planes, +-2^20 for Stokes planes) saturate instead of wrapping)
+template <int FRAC_BITS>
+__device__ __forceinline__ long long to_fixed(double v, double lim) {
     v = (v == v) ? fmin(fmax(v, -lim), lim) : 0.0;
-    return __double2ll_rn(v * (double)(1ll << SP_PLANE_FRAC_BITS));
+    return __double2ll_rn(v * (double)(1ll << FRAC_BITS));
 }
+__device__ __forceinline__ long long to_plane_fixed(double v) { return to_fixed<SP_PLANE_FRAC_BITS>(v, 4194304.0); }
+__device__ __forceinline__ long long to_stokes_fixed(double v) { return to_fixed<SP_STOKES_FRAC_BITS>(v, 1048576.0); }
 
 __device__ __forceinline__ int bin_ray(const ChannelDev& ch, const DetRay& d, bool active) {
     int pix = -1;
     if (active && d.alive && ch.nx > 0) {
-        const bool hist = (ch.kind == SP_IMG_HISTOGRAM);
+        const bool hist = (ch.kind != SP_IMG_INTERFEROGRAM);        // histogram edges for counts and Stokes images
         const int ix = bin_index(d.x, ch.x_lo, ch.x_hi, ch.nx, hist);
         const int iy = bin_index(d.y, ch.y_lo, ch.y_hi, ch.ny, hist);
         if (ix >= 0 && iy >= 0) pix = iy * ch.nx + ix;
@@ -404,7 +415,15 @@ __device__ __forceinline__ int bin_ray(const ChannelDev& ch, const DetRay& d, bo
         if (leader) atomicAdd(ch.counts + pix, (unsigned long long)__popc(peers));
     } else {
         long long v0 = 0, v1 = 0, v2 = 0, v3 = 0;
-        if (pix >= 0) { v0 = to_plane_fixed(d.ex_re); v1 = to_plane_fixed(d.ex_im); v2 = to_plane_fixed(d.ey_re); v3 = to_plane_fixed(d.ey_im); }
+        if (pix >= 0) {
+            if (ch.kind == SP_IMG_STOKES) {         // count, I = |Ex|^2 + |Ey|^2, Q = |Ex|^2 - |Ey|^2, U = 2 Re(Ex conj(Ey))
+                const double xx = d.ex_re * d.ex_re + d.ex_im * d.ex_im, yy = d.ey_re * d.ey_re + d.ey_im * d.ey_im;
+                const double u = 2.0 * (d.ex_re * d.ey_re + d.ex_im * d.ey_im);
+                v0 = 1; v1 = to_stokes_fixed(xx + yy); v2 = to_stokes_fixed(xx - yy); v3 = to_stokes_fixed(u);
+            } else {
+                v0 = to_plane_fixed(d.ex_re); v1 = to_plane_fixed(d.ex_im); v2 = to_plane_fixed(d.ey_re); v3 = to_plane_fixed(d.ey_im);
+            }
+        }
         if (peers & (peers - 1)) {                       // more than one lane on this pixel (coarse images): sum the group
             long long s0 = 0, s1 = 0, s2 = 0, s3 = 0;
             for (unsigned m = peers; m; m &= m - 1) {
@@ -1255,7 +1274,8 @@ __global__ void k_optics_image(const double* __restrict__ rf, const double* __re
             const double unit = ch.input_mm ? 1.0 : 1e3;      // m_to_mm (diagnostics.py:122-127)
             d.x = xm * unit; d.th = rf[n + i]; d.y = ym * unit; d.ph = rf[3 * n + i];
             if (jf) { d.ex_re = jf[2 * i]; d.ex_im = jf[2 * i + 1]; d.ey_re = jf[2 * (n + i)]; d.ey_im = jf[2 * (n + i) + 1]; }
-            run_optics(d, xm, ym, ch.ops, ch.n_ops, jf != nullptr, ch.kwave);
+            // a Stokes image does not need the E-phase advance (see bin_ray); the Jones vectors handed back do
+            run_optics(d, xm, ym, ch.ops, ch.n_ops, jf != nullptr && (ch.kind != SP_IMG_STOKES || jf_out != nullptr), ch.kwave);
         }
         if (valid && rf_out) {
             const double nanv = __longlong_as_double(0x7ff8000000000000ULL);
@@ -1324,6 +1344,14 @@ __global__ void k_finalize(const long long* __restrict__ planes, double* __restr
     const double q = 1.0 / (double)(1ll << SP_PLANE_FRAC_BITS);
     const double a = (double)planes[i] * q, b = (double)planes[2 * npix + i] * q;     // Re(sum Ex), Re(sum Ey)
     H[i] = sqrt(a * a + b * b);
+}
+
+__global__ void k_finalize_stokes(const long long* __restrict__ planes, double* __restrict__ H, size_t npix) {
+    size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= npix) return;
+    const double q = 1.0 / (double)(1ll << SP_STOKES_FRAC_BITS);
+    H[i] = (double)planes[i];                                                          // N
+    for (int k = 1; k < 4; ++k) H[k * npix + i] = (double)planes[k * npix + i] * q;    // I, Q, U
 }
 
 template <bool PHASE, bool AUX64>
@@ -1859,6 +1887,7 @@ extern "C" int sp_optics_image(const double* rf_dev, const double* jf_dev, uint6
     int rc = channel_to_dev(chan, ch);
     if (rc) return rc;
     if (ch.kind == SP_IMG_INTERFEROGRAM && ch.nx > 0 && !jf_dev) return fail(SP_EINVAL, "interferogram needs Jones vectors");
+    if (ch.kind == SP_IMG_STOKES && ch.nx > 0 && !jf_dev) return fail(SP_EINVAL, "Stokes image needs Jones vectors");
     uint64_t blocks = (n + 255) / 256;
     const size_t nbins = (size_t)ch.nx * ch.ny;
     if (ch.kind == SP_IMG_HISTOGRAM && nbins > 0 && nbins <= 12288) {
@@ -1889,7 +1918,10 @@ extern "C" int sp_image_finalize(const sp_image* img, double* H_dev, void* strea
     if (!img || !H_dev || !img->planes_dev) return fail(SP_EINVAL, "null argument");
     const size_t npix = (size_t)img->nx * img->ny;
     if (npix == 0) return SP_OK;
-    k_finalize<<<(unsigned)((npix + 255) / 256), 256, 0, (cudaStream_t)stream>>>((const long long*)img->planes_dev, H_dev, npix);
+    if (img->kind == SP_IMG_STOKES)
+        k_finalize_stokes<<<(unsigned)((npix + 255) / 256), 256, 0, (cudaStream_t)stream>>>((const long long*)img->planes_dev, H_dev, npix);
+    else
+        k_finalize<<<(unsigned)((npix + 255) / 256), 256, 0, (cudaStream_t)stream>>>((const long long*)img->planes_dev, H_dev, npix);
     LAUNCH_CHECK();
     return SP_OK;
 }

@@ -2,7 +2,7 @@
 ``src/simulator/diagnostics.py`` (legacy twin: ``src/solvers-legacy/rtm_solver.py``).
 
 Every ``*_solve`` is one pass of the fused optics kernel over the rays (``sp_optics_image``); ``histogram`` /
-``interferogram`` is one binning pass.  ``spec()`` returns the same optical train as data so that
+``interferogram`` / ``polarimetry`` is one binning pass.  ``spec()`` returns the same optical train as data so that
 ``propagator.solve_and_image`` can run it in the propagation kernel's epilogue instead.
 Units: ``rf`` arrives in metres, is converted with ``m_to_mm`` (diagnostics.py:313), lengths L, R, Lx, Ly in mm.
 """
@@ -130,12 +130,18 @@ def chain_ops(name, L=400, R=25, focal_plane=0, **kw):
 
 
 def spec(name, *, bin_scale=1, pix_x=3448, pix_y=2574, L=400, R=25, Lx=18, Ly=13.5, focal_plane=0, wavelength=0.0,
-         interferogram=False, ref_beam=None, **kw):
-    """A fused-path diagnostic: optical train ``name`` + a fresh detector image."""
+         interferogram=False, stokes=False, ref_beam=None, **kw):
+    """A fused-path diagnostic: optical train ``name`` + a fresh detector image (a ray-count histogram, an interferogram,
+    or with ``stokes=True`` the ray count and Stokes I, Q, U of a polarimeter, see ``Polarimetry``)."""
+    if stokes and interferogram:
+        raise ValueError("a channel records either an interferogram or a Stokes image, not both")
+    if stokes and ref_beam is not None:
+        raise ValueError("a reference beam has no polarimetric meaning: stokes=True takes no ref_beam")
     ops = chain_ops(name, L=L, R=R, focal_plane=focal_plane, **kw)
     if ref_beam is not None:
         ops = [("ref_beam", ref_beam[0], ref_beam[1])] + ops
-    mk = engine.ImageBuffer.for_interferogram if interferogram else engine.ImageBuffer.for_histogram
+    mk = (engine.ImageBuffer.for_interferogram if interferogram else
+          engine.ImageBuffer.for_stokes if stokes else engine.ImageBuffer.for_histogram)
     return DiagnosticSpec(ops, mk(bin_scale, pix_x, pix_y, Lx, Ly), wavelength, name)
 
 
@@ -286,3 +292,56 @@ class Interferometry(Diagnostic):
 
     def interferogram(self, bin_scale=1, pix_x=3448, pix_y=2574, clear_mem=False):   # diagnostics.py:640
         self.histogram_legacy(bin_scale=bin_scale, pix_x=pix_x, pix_y=pix_y, clear_mem=clear_mem)
+
+
+class Polarimetry(Diagnostic):
+    """Faraday-rotation polarimetry (no upstream counterpart): per detector pixel the ray count ``N`` and the Stokes
+    parameters ``I``, ``Q``, ``U`` of the rays' Jones vectors, summed incoherently, which is what a camera behind a
+    polariser integrates.  For the reference's Jones vector ``E = amp e^{i phase} (-sin pol, cos pol)``
+    (full_solver.py:883-890) a ray contributes ``I = amp^2``, ``Q = -amp^2 cos 2pol`` and ``U = -amp^2 sin 2pol``; Stokes V
+    is identically 0.  ``pol`` is the Faraday rotation integrated by ``ScalarDomain(B_on=True)`` and ``amp`` the
+    inverse-bremsstrahlung attenuation (``inv_brems=True``).  Needs ``Jf`` (``solve(..., return_E=True)``)."""
+
+    def __init__(self, wavelength, rf, Jf=None, **kw):
+        if Jf is None:
+            raise ValueError("This diagnostic requires a calculated Jf matrix.")
+        super().__init__(wavelength, rf, Jf, **kw)
+
+    def single_lens_solve(self):                     # the shadowgraphy imaging trains
+        self._run("shadow_single")
+
+    def two_lens_solve(self):
+        self._run("shadow_two")
+
+    def polarimetry(self, bin_scale=1, pix_x=3448, pix_y=2574, clear_mem=False):
+        """Bins the rays on the histogram's edges (np.histogram2d semantics); sets ``N``, ``I``, ``Q``, ``U`` (ny, nx) and
+        ``H = I``, the attenuation-weighted shadowgram.  The Jones vectors are binned as they left the plasma: the optics
+        multiply both components by the same phase factor, which the Stokes parameters do not see."""
+        if self._Jf is None:
+            raise ValueError("This diagnostic requires a calculated Jf matrix.")
+        img = engine.ImageBuffer.for_stokes(bin_scale, pix_x, pix_y, self.Lx, self.Ly)
+        src = self._rf_det if self._rf_det is not None else m_to_mm(self._rf_m)
+        engine.optics_image(src, [], jf=self._Jf, image=img, input_mm=True, want_rays=False)
+        self.xedges = np.linspace(-self.Lx / 2, self.Lx / 2, img.nx + 1)
+        self.yedges = np.linspace(-self.Ly / 2, self.Ly / 2, img.ny + 1)
+        S = img.stokes()
+        self.N, self.I, self.Q, self.U = (self._view(S[k]) for k in "NIQU")
+        self.H = self.I
+        if clear_mem:
+            clear_rays(self)
+
+    def rotation_angle(self):
+        """Intensity-weighted polarisation angle per pixel in the convention of ``pol``: ``0.5 atan2(-U, -Q)``, in
+        (-pi/2, pi/2]; NaN where no ray landed."""
+        if isinstance(self.I, torch.Tensor):
+            a = 0.5 * torch.atan2(-self.U, -self.Q)
+            return torch.where(self.N > 0, a, torch.full_like(a, float("nan")))
+        with np.errstate(invalid="ignore"):
+            return np.where(self.N > 0, 0.5 * np.arctan2(-self.U, -self.Q), np.nan)
+
+    def analyser_image(self, angle):
+        """What a camera behind a linear analyser at ``angle`` (radians, the convention of ``pol``) records:
+        ``0.5 (I - Q cos 2 angle - U sin 2 angle)``; a ray of angle ``pol`` passes ``amp^2 cos^2(pol - angle)`` (Malus).
+        Two calls at ``pi/2 +- delta`` give the two images of the usual two-camera polarimeter."""
+        m = torch if isinstance(angle, torch.Tensor) else np          # angle: a number or a per-pixel array
+        return 0.5 * (self.I - self.Q * m.cos(2 * angle) - self.U * m.sin(2 * angle))

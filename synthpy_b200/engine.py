@@ -216,10 +216,14 @@ def make_beam(beam_type, size, divergence, ne_extent, probing_direction="z", see
                   divergence=float(divergence), start=-float(ne_extent), seed=int(seed))
 
 
+IMAGE_KINDS = {"histogram": L.IMG_HISTOGRAM, "interferogram": L.IMG_INTERFEROGRAM, "stokes": L.IMG_STOKES}
+
+
 class ImageBuffer:
     """Detector image accumulator in HBM.  ``kind`` 'histogram' -> uint64 counts (np.histogram2d semantics),
-    'interferogram' -> four int64 fixed-point planes (2^-40 units) of summed complex E (digitize semantics): integer
-    sums are exact, so the image is identical from run to run and for any partition of the rays over GPUs."""
+    'interferogram' -> four int64 fixed-point planes (2^-40 units) of summed complex E (digitize semantics), 'stokes' ->
+    int64 ray count plus Stokes I, Q, U of the rays' Jones vectors in fixed point (2^-32 units; histogram semantics):
+    integer sums are exact, so the image is identical from run to run and for any partition of the rays over GPUs."""
 
     def __init__(self, kind, nx, ny, x_range, y_range):
         require_cuda()
@@ -229,7 +233,7 @@ class ImageBuffer:
         self._global = None            # sum over ranks attached by distributed.combine_images (out of place)
         if kind == "histogram":
             self.counts = torch.zeros((self.ny, self.nx), dtype=torch.int64, device="cuda")
-        elif kind == "interferogram":
+        elif kind in ("interferogram", "stokes"):
             self.planes = torch.zeros((4, self.ny, self.nx), dtype=torch.int64, device="cuda")
         else:
             raise ValueError(kind)
@@ -245,8 +249,13 @@ class ImageBuffer:
         return cls("interferogram", pix_x // bin_scale - 1, pix_y // bin_scale - 1, (-Lx // 2, Lx // 2),
                    (-Ly // 2, Ly // 2))
 
+    @classmethod
+    def for_stokes(cls, bin_scale=1, pix_x=3448, pix_y=2574, Lx=18, Ly=13.5):
+        # the histogram's edges: np.histogram2d(..., weights=) of I, Q, U is the image
+        return cls("stokes", pix_x // bin_scale, pix_y // bin_scale, (-Lx / 2, Lx / 2), (-Ly / 2, Ly / 2))
+
     def struct(self):
-        return L.Image(kind=L.IMG_HISTOGRAM if self.kind == "histogram" else L.IMG_INTERFEROGRAM, nx=self.nx,
+        return L.Image(kind=IMAGE_KINDS[self.kind], nx=self.nx,
                        ny=self.ny, x_lo=self.x_range[0], x_hi=self.x_range[1], y_lo=self.y_range[0],
                        y_hi=self.y_range[1], counts_dev=None if self.counts is None else self.counts.data_ptr(),
                        planes_dev=None if self.planes is None else self.planes.data_ptr())
@@ -272,10 +281,23 @@ class ImageBuffer:
         return self._global if self._global is not None else self.tensors()[0]
 
     def result(self):
-        """H as the reference returns it: float64 counts (ny, nx), or sqrt(Re(sum Ex)^2 + Re(sum Ey)^2)."""
+        """H as the reference returns it: float64 counts (ny, nx), or sqrt(Re(sum Ex)^2 + Re(sum Ey)^2); for a Stokes
+        image the intensity I (ny, nx), i.e. the attenuation-weighted shadowgram."""
         if self.counts is not None:
             return self.total().to(torch.float64)
-        H = torch.empty((self.ny, self.nx), dtype=torch.float64, device="cuda")
+        if self.kind == "stokes":
+            return self.stokes()["I"]
+        return self._finalize((self.ny, self.nx))
+
+    def stokes(self):
+        """Stokes image as float64 (ny, nx) tensors: {'N': ray count, 'I', 'Q', 'U'} (include/synthpy_b200.h SP_IMG_STOKES)."""
+        if self.kind != "stokes":
+            raise ValueError(f"stokes() needs a 'stokes' image, this one is '{self.kind}'")
+        H = self._finalize((4, self.ny, self.nx))
+        return dict(zip("NIQU", H.unbind(0)))
+
+    def _finalize(self, shape):
+        H = torch.empty(shape, dtype=torch.float64, device="cuda")
         img = self.struct()
         img.planes_dev = self.total().data_ptr()
         L.check(L.lib.sp_image_finalize(C.byref(img), _ptr(H), _stream()))
