@@ -327,6 +327,24 @@ int sp_fresnel_transfer(double* spec_dev, int m0, int m1, double d0, double d1, 
 int sp_fresnel_finish(const double* u_pad_dev, int n0, int n1, int pad_factor, double scale_re, double scale_im,
                       double* out_dev, void* stream);
 
+/* ----------------------------------------------------------------------------------- turbulent-field noise */
+/*
+ * Band-limited turbulence (gaussian3D.domain_fft, src/field_generator/gaussian3D.py:215-271) is Re ifftn(Z sqrt(S)) for
+ * complex white noise Z.  This writes the Hermitian half spectrum whose inverse real FFT is that field, drawing Z on the
+ * device from (seed, grid index):
+ *   noise   Z at full-grid element (i, j, l) of the (n0, n1, n2) grid, flat = (i n1 + j) n2 + l: one Philox4x32-10 block
+ *           with key (seed lo, seed hi) and counter (flat lo, flat hi, 0, 0xf1e1d) (the beam's tag is 0x5eed, so one seed
+ *           gives unrelated beam and field streams); U0, U1 = the block's two 53-bit uniforms;
+ *           Z = sqrt(-2 log(1 - U0)) (cos 2 pi U1 + i sin 2 pi U1).  Re Z, Im Z ~ N(0, 1), independent.
+ *   output  H[i][j][l] = (double)sqrtf(S[i][j][l]) (Z(i, j, l) + conj Z((n0 - i) % n0, (n1 - j) % n1, (n2 - l) % n2)) / 2
+ *           for l < n2/2 + 1; exactly real at self-conjugate elements.
+ *   S_dev   float32 [n0][n1][n2/2 + 1], the power spectrum on the half grid (0 outside the band)
+ *   H_dev   complex128 interleaved [n0][n1][n2/2 + 1], 16-byte aligned: the layout torch.fft.irfftn(H, s=(n0, n1, n2))
+ *           and cuFFT C2R take
+ * Every element of H is written.  The field is a function of the seed alone: it does not depend on the GPU or launch.
+ */
+int sp_noise_spectrum(const float* S_dev, int n0, int n1, int n2, uint64_t seed, double* H_dev, void* stream);
+
 /* Measurement aid for bench.py's roofline (no reference counterpart: the reference has no device code).  Enqueues
  * one launch in which every resident thread of every SM runs 8 independent DFMA chains of `iters` links and writes
  * one double to out_dev[thread] (thread < out_len); *n_dfma_out = DFMA thread-instructions of the launch.  The caller

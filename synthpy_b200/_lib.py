@@ -90,6 +90,7 @@ EXPORTS = {
     "sp_fresnel_finish": (C.c_int, [C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_double, C.c_double, C.c_void_p, C.c_void_p]),
     "sp_rhs": (C.c_int, [C.c_void_p, C.POINTER(Params), C.c_void_p, C.c_uint64, C.c_void_p, C.c_void_p]),
     "sp_fp64_peak": (C.c_int, [C.c_int, C.c_void_p, C.c_uint64, C.POINTER(C.c_uint64), C.c_void_p]),
+    "sp_noise_spectrum": (C.c_int, [C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_uint64, C.c_void_p, C.c_void_p]),
 }
 
 

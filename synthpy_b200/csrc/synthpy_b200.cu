@@ -6,8 +6,9 @@
 //   k_propagate<T, METHOD, PHASE, AUX64>                 : persistent ray integrator + fused optics/binning
 //   k_joint_*                                           : the reference's joint-step RK45 (one h for all rays)
 //   k_optics_image / k_finalize / k_rhs / k_beam        : stand-alone entry points
+//   k_noise_spectrum                                    : turbulent-field noise as a Hermitian half spectrum
 //
-// Per-ray arithmetic lives in ray_core.h (shared with the CPU self-test build).
+// Per-ray arithmetic lives in ray_core.h (shared with the CPU self-test build), the noise's in noise_core.h.
 #include <cuda_runtime.h>
 #include <stdio.h>
 #include <stdlib.h>
@@ -2141,6 +2142,44 @@ extern "C" int sp_fresnel_finish(const double* u_pad_dev, int n0, int n1, int pa
     k_fresnel_finish<<<stream_grid((unsigned long long)n0 * n1), 256, 0, (cudaStream_t)stream>>>((const d2*)u_pad_dev, n0, n1,
                                                                                                 pad_factor, scale_re, scale_im,
                                                                                                 (d2*)out_dev);
+    LAUNCH_CHECK();
+    return SP_OK;
+}
+
+// ------------------------------------------------------------------------------- turbulent-field noise (SURVEY 8f-1)
+// The Hermitian half spectrum of band-limited turbulence, written straight from (seed, grid index): no noise is drawn
+// on the host and nothing of grid size is copied to the device.  Per-element math is noise_core.h.
+#include "noise_core.h"
+
+// Grid-stride over the half grid [n0][n1][nh]; (i, j, l) of the element advance by the stride's own mixed-radix digits,
+// so the loop does no 64-bit division.  Every element is written (S is already 0 outside the band).
+__global__ void __launch_bounds__(256) k_noise_spectrum(const float* __restrict__ S, int n0, int n1, int n2, uint64_t seed,
+                                                        d2* __restrict__ H) {
+    const int nh = n2 / 2 + 1;
+    const uint64_t total = (uint64_t)n0 * n1 * nh, stride = (uint64_t)gridDim.x * blockDim.x;
+    uint64_t h = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (h >= total) return;
+    int l = (int)(h % nh), j = (int)((h / nh) % n1), i = (int)(h / nh / n1);
+    const int dl = (int)(stride % nh), dj = (int)((stride / nh) % n1);
+    const uint64_t di = stride / nh / n1;
+    for (; h < total; h += stride) {
+        H[h] = noise_half(__ldg(S + h), n0, n1, n2, seed, i, j, l);
+        l += dl;
+        int carry = l >= nh;
+        l -= carry ? nh : 0;
+        j += dj + carry;
+        carry = j >= n1;
+        j -= carry ? n1 : 0;
+        i += (int)di + carry;                  // past n0 only when h has passed `total` as well
+    }
+}
+
+extern "C" int sp_noise_spectrum(const float* S_dev, int n0, int n1, int n2, uint64_t seed, double* H_dev, void* stream) {
+    if (!S_dev || !H_dev) return fail(SP_EINVAL, "null argument");
+    if (n0 < 2 || n1 < 2 || n2 < 2) return fail(SP_EINVAL, "need n0, n1, n2 >= 2");
+    if ((uintptr_t)H_dev % 16) return fail(SP_EINVAL, "H_dev must be 16-byte aligned (complex128)");
+    const unsigned long long total = (unsigned long long)n0 * n1 * (n2 / 2 + 1);
+    k_noise_spectrum<<<stream_grid(total), 256, 0, (cudaStream_t)stream>>>(S_dev, n0, n1, n2, seed, (d2*)H_dev);
     LAUNCH_CHECK();
     return SP_OK;
 }

@@ -396,6 +396,22 @@ def beam_generate(beam, n, ray_offset=0):
     return s0
 
 
+def noise_spectrum(S, shape, seed):
+    """sp_noise_spectrum: the Hermitian half spectrum sqrt(S) (Z + conj Z(-k)) / 2 of Philox complex white noise for a
+    ``shape`` = (n0, n1, n2) grid.  S: contiguous float32 CUDA tensor (n0, n1, n2 // 2 + 1); returns complex128 of the
+    same shape on S's device, ready for ``torch.fft.irfftn(H, s=shape)``."""
+    require_cuda()
+    n0, n1, n2 = (int(n) for n in shape)
+    if not (S.is_cuda and S.dtype == torch.float32 and S.is_contiguous() and tuple(S.shape) == (n0, n1, n2 // 2 + 1)):
+        raise ValueError(f"S must be a contiguous float32 CUDA tensor of shape {(n0, n1, n2 // 2 + 1)}")
+    if not 0 <= int(seed) < 2 ** 64:
+        raise ValueError("seed must be in [0, 2**64)")
+    with torch.cuda.device(S.device):
+        H = torch.empty(S.shape, dtype=torch.complex128, device=S.device)
+        L.check(L.lib.sp_noise_spectrum(_ptr(S), n0, n1, n2, int(seed), _ptr(H), _stream()))
+    return H
+
+
 def optics_image(rf, ops, *, jf=None, image=None, wavelength=0.0, input_mm=False, want_rays=True):
     """Optical train (+ optional binning) on existing rays.  rf: (4,N) CUDA float64; jf: (2,N) complex128.
     Returns (rf_out, jf_out) at the detector plane (mm; NaN columns = rejected), or (None, None)."""
