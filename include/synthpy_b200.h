@@ -345,6 +345,23 @@ int sp_fresnel_finish(const double* u_pad_dev, int n0, int n1, int pad_factor, d
  */
 int sp_noise_spectrum(const float* S_dev, int n0, int n1, int n2, uint64_t seed, double* H_dev, void* stream);
 
+/*
+ * The same H on a box of the full grid, stored in a chosen axis order, so that a field too large for one spectrum can be
+ * built piece by piece (field_generator.domain_fft_slabs: the Hermitian half along an axis other than the probing one):
+ *   order   host int[3], a permutation of 0, 1, 2: box axis t runs along grid axis order[t]
+ *   lo, cnt host int[3] per GRID axis: the box is [lo[a], lo[a] + cnt[a]) along grid axis a
+ *   output  H_dev[a][b][c] (complex128 interleaved, dims cnt[order[0]] x cnt[order[1]] x cnt[order[2]], 16-byte aligned)
+ *           = H at the grid index k with lo[order[t]] + (a, b, c)[t] along grid axis order[t]: for k in the half grid
+ *           (last index l <= n2/2) the value sp_noise_spectrum writes there, bit for bit; above it conj H(-k) of the
+ *           mirrored half-grid element, bit for bit (given S(-k) == S(k) bit for bit).  The box is therefore exactly
+ *           the Hermitian extension of sp_noise_spectrum's half spectrum, in any axis order.
+ *   S_dev   float32 in the output's box layout, the power spectrum at each element (0 outside the band)
+ * SP_EINVAL before any CUDA call for a null pointer, any n < 2, an order that is not a permutation, lo < 0, cnt < 1 or
+ * lo + cnt > n on any axis, or a misaligned H_dev.  Every element of the box is written.
+ */
+int sp_noise_spectrum_box(const float* S_dev, int n0, int n1, int n2, const int* order, const int* lo, const int* cnt,
+                          uint64_t seed, double* H_dev, void* stream);
+
 /* Measurement aid for bench.py's roofline (no reference counterpart: the reference has no device code).  Enqueues
  * one launch in which every resident thread of every SM runs 8 independent DFMA chains of `iters` links and writes
  * one double to out_dev[thread] (thread < out_len); *n_dfma_out = DFMA thread-instructions of the launch.  The caller

@@ -91,6 +91,8 @@ EXPORTS = {
     "sp_rhs": (C.c_int, [C.c_void_p, C.POINTER(Params), C.c_void_p, C.c_uint64, C.c_void_p, C.c_void_p]),
     "sp_fp64_peak": (C.c_int, [C.c_int, C.c_void_p, C.c_uint64, C.POINTER(C.c_uint64), C.c_void_p]),
     "sp_noise_spectrum": (C.c_int, [C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_uint64, C.c_void_p, C.c_void_p]),
+    "sp_noise_spectrum_box": (C.c_int, [C.c_void_p, C.c_int, C.c_int, C.c_int, C.POINTER(C.c_int), C.POINTER(C.c_int),
+                                        C.POINTER(C.c_int), C.c_uint64, C.c_void_p, C.c_void_p]),
 }
 
 

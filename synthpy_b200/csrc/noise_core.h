@@ -7,8 +7,8 @@
 // (S(-k) == S(k) bit for bit: fftfreq gives exact negatives).  A counter-based generator evaluates Z(-k) where it is
 // needed, so H is written in one pass and nothing of grid size exists before it.
 //
-// SP_HD like ray_core.h: the same source is inlined into the sm_100a kernel and compiled by g++ into
-// tests/noise_harness.cpp.
+// SP_HD like ray_core.h: the same source is inlined into the sm_100a kernels and compiled by g++ into
+// tests/noise_harness.cpp and tests/noise_box_harness.cpp.
 #pragma once
 #include "ray_core.h"
 
@@ -49,6 +49,36 @@ SP_HD d2 noise_half(float s32, int n0, int n1, int n2, uint64_t seed, int i, int
     d2 h;
     h.x = s * (0.5 * (are + bre));
     h.y = s * (0.5 * (aim - bim));
+    return h;
+}
+
+// A box of the full grid stored in axis order `order` (a permutation of 0, 1, 2): element (a, b, c) of the box is grid
+// index lo[order[t]] + (a, b, c)[t] along grid axis order[t].  lo is per grid axis, dim per box axis.
+struct NoiseBox {
+    int order[3], lo[3], dim[3];
+};
+
+// the box coordinate that runs along grid axis `axis` (selects, no indexed access: the kernel keeps it in registers)
+SP_HD int box_coord(const NoiseBox& B, int axis, int a, int b, int c) {
+    return B.order[0] == axis ? a : B.order[1] == axis ? b : c;
+}
+
+// H at box element (a, b, c).  Inside the half grid (l <= n2/2) this is noise_half at the element, the value
+// k_noise_spectrum writes.  Above it, it is conj H(-k) with H(-k) from noise_half at the mirrored half-grid element: the
+// formula would give the same value at k itself, but a device build may fuse the sum of the two draws' real parts into
+// an FMA in either order, so only the mirror makes the box the Hermitian extension of k_noise_spectrum's half spectrum
+// bit for bit.  s32 is S at k, which equals S(-k) bit for bit.
+SP_HD d2 noise_box(float s32, int n0, int n1, int n2, uint64_t seed, const NoiseBox& B, int a, int b, int c) {
+    int i = B.lo[0] + box_coord(B, 0, a, b, c), j = B.lo[1] + box_coord(B, 1, a, b, c);
+    int l = B.lo[2] + box_coord(B, 2, a, b, c);
+    const bool upper = 2 * l > n2;
+    if (upper) {
+        i = i ? n0 - i : 0;
+        j = j ? n1 - j : 0;
+        l = n2 - l;
+    }
+    d2 h = noise_half(s32, n0, n1, n2, seed, i, j, l);
+    if (upper) h.y = -h.y;
     return h;
 }
 

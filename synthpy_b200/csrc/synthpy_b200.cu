@@ -7,6 +7,7 @@
 //   k_joint_*                                           : the reference's joint-step RK45 (one h for all rays)
 //   k_optics_image / k_finalize / k_rhs / k_beam        : stand-alone entry points
 //   k_noise_spectrum                                    : turbulent-field noise as a Hermitian half spectrum
+//   k_noise_spectrum_box                                : the same noise on a box of the full grid, any axis order
 //
 // Per-ray arithmetic lives in ray_core.h (shared with the CPU self-test build), the noise's in noise_core.h.
 #include <cuda_runtime.h>
@@ -2180,6 +2181,55 @@ extern "C" int sp_noise_spectrum(const float* S_dev, int n0, int n1, int n2, uin
     if ((uintptr_t)H_dev % 16) return fail(SP_EINVAL, "H_dev must be 16-byte aligned (complex128)");
     const unsigned long long total = (unsigned long long)n0 * n1 * (n2 / 2 + 1);
     k_noise_spectrum<<<stream_grid(total), 256, 0, (cudaStream_t)stream>>>(S_dev, n0, n1, n2, seed, (d2*)H_dev);
+    LAUNCH_CHECK();
+    return SP_OK;
+}
+
+// The same H on a box of the full grid in any axis order (out-of-core generation fills its spectrum chunk by chunk,
+// with the Hermitian half along whichever axis is not probed).  Same loop as k_noise_spectrum over [dim0][dim1][dim2].
+__global__ void __launch_bounds__(256) k_noise_spectrum_box(const float* __restrict__ S, int n0, int n1, int n2, NoiseBox B,
+                                                            uint64_t seed, d2* __restrict__ H) {
+    const int d1 = B.dim[1], d2_ = B.dim[2];
+    const uint64_t total = (uint64_t)B.dim[0] * d1 * d2_, stride = (uint64_t)gridDim.x * blockDim.x;
+    uint64_t h = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (h >= total) return;
+    int c = (int)(h % d2_), b = (int)((h / d2_) % d1), a = (int)(h / d2_ / d1);
+    const int dc = (int)(stride % d2_), db = (int)((stride / d2_) % d1);
+    const uint64_t da = stride / d2_ / d1;
+    for (; h < total; h += stride) {
+        H[h] = noise_box(__ldg(S + h), n0, n1, n2, seed, B, a, b, c);
+        c += dc;
+        int carry = c >= d2_;
+        c -= carry ? d2_ : 0;
+        b += db + carry;
+        carry = b >= d1;
+        b -= carry ? d1 : 0;
+        a += (int)da + carry;                  // past dim0 only when h has passed `total` as well
+    }
+}
+
+extern "C" int sp_noise_spectrum_box(const float* S_dev, int n0, int n1, int n2, const int* order, const int* lo,
+                                     const int* cnt, uint64_t seed, double* H_dev, void* stream) {
+    if (!S_dev || !H_dev || !order || !lo || !cnt) return fail(SP_EINVAL, "null argument");
+    if (n0 < 2 || n1 < 2 || n2 < 2) return fail(SP_EINVAL, "need n0, n1, n2 >= 2");
+    const int n[3] = {n0, n1, n2};
+    bool seen[3] = {false, false, false};
+    for (int t = 0; t < 3; ++t) {
+        if (order[t] < 0 || order[t] > 2 || seen[order[t]]) return fail(SP_EINVAL, "order must be a permutation of 0, 1, 2");
+        seen[order[t]] = true;
+    }
+    for (int t = 0; t < 3; ++t)
+        if (lo[t] < 0 || cnt[t] < 1 || (long long)lo[t] + cnt[t] > n[t])
+            return fail(SP_EINVAL, "box out of the grid: need lo >= 0, cnt >= 1 and lo + cnt <= n on every axis");
+    if ((uintptr_t)H_dev % 16) return fail(SP_EINVAL, "H_dev must be 16-byte aligned (complex128)");
+    NoiseBox B;
+    for (int t = 0; t < 3; ++t) {
+        B.order[t] = order[t];
+        B.lo[t] = lo[t];
+        B.dim[t] = cnt[order[t]];
+    }
+    const unsigned long long total = (unsigned long long)B.dim[0] * B.dim[1] * B.dim[2];
+    k_noise_spectrum_box<<<stream_grid(total), 256, 0, (cudaStream_t)stream>>>(S_dev, n0, n1, n2, B, seed, (d2*)H_dev);
     LAUNCH_CHECK();
     return SP_OK;
 }

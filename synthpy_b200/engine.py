@@ -412,6 +412,35 @@ def noise_spectrum(S, shape, seed):
     return H
 
 
+def noise_spectrum_box(S, shape, order, lo, cnt, seed, out=None):
+    """sp_noise_spectrum_box: ``noise_spectrum``'s H on the box [lo, lo + cnt) (per grid axis) of the full ``shape`` grid,
+    stored with box axis t along grid axis order[t].  S: contiguous float32 CUDA tensor of the box shape
+    (cnt[order[0]], cnt[order[1]], cnt[order[2]]); ``out``: a contiguous complex128 tensor (or view) of that shape on S's
+    device to write into, else a new one.  Returns the written tensor."""
+    require_cuda()
+    n = tuple(int(v) for v in shape)
+    order, lo, cnt = (tuple(int(v) for v in a) for a in (order, lo, cnt))
+    if len(n) != 3 or len(order) != 3 or len(lo) != 3 or len(cnt) != 3:
+        raise ValueError("shape, order, lo and cnt need three entries each")
+    if sorted(order) != [0, 1, 2]:
+        raise ValueError(f"order {order} is not a permutation of 0, 1, 2")
+    if any(a < 0 or c < 1 or a + c > m for a, c, m in zip(lo, cnt, n)):
+        raise ValueError(f"box lo={lo} cnt={cnt} is not inside the grid {n}")
+    box = tuple(cnt[o] for o in order)
+    if not (S.is_cuda and S.dtype == torch.float32 and S.is_contiguous() and tuple(S.shape) == box):
+        raise ValueError(f"S must be a contiguous float32 CUDA tensor of shape {box}")
+    if not 0 <= int(seed) < 2 ** 64:
+        raise ValueError("seed must be in [0, 2**64)")
+    if out is not None and not (out.device == S.device and out.dtype == torch.complex128 and out.is_contiguous()
+                                and tuple(out.shape) == box):
+        raise ValueError(f"out must be a contiguous complex128 tensor of shape {box} on {S.device}")
+    ints = lambda v: (C.c_int * 3)(*v)
+    with torch.cuda.device(S.device):
+        H = torch.empty(box, dtype=torch.complex128, device=S.device) if out is None else out
+        L.check(L.lib.sp_noise_spectrum_box(_ptr(S), *n, ints(order), ints(lo), ints(cnt), int(seed), _ptr(H), _stream()))
+    return H
+
+
 def optics_image(rf, ops, *, jf=None, image=None, wavelength=0.0, input_mm=False, want_rays=True):
     """Optical train (+ optional binning) on existing rays.  rf: (4,N) CUDA float64; jf: (2,N) complex128.
     Returns (rf_out, jf_out) at the detector plane (mm; NaN columns = rejected), or (None, None)."""

@@ -20,7 +20,8 @@ that nothing about the result depends on it:
     widened until its probing axis makes the same choice as the full axis.
 
 The slab source is a callable ``source(k0, k1) -> ne[..., k0:k1 along the probing axis]`` (NumPy array, ``np.memmap`` of a
-raw dump, or CUDA tensor): ``array_source`` wraps an array-like.  One slab is resident at a time; the next is packed after
+raw dump, or CUDA tensor): ``array_source`` wraps an array-like; ``field_generator.turbulent_ne_slabs`` generates a
+turbulent field on the device slab by slab.  One slab is resident at a time; the next is packed after
 the rays have left the current one.  ``PrefetchingSource`` overlaps the host-side read of the next slab with the tracing;
 upload and packing are not overlapped yet.
 """
@@ -91,6 +92,8 @@ class PrefetchingSource:
         if out is None:
             out = self._source(k0, k1)
             self.misses += 1
+            if getattr(out, "is_cuda", False):          # before any worker thread has called the source
+                raise ValueError("prefetch=True is for host sources: this source returns CUDA tensors (use prefetch=False)")
         if k1 < self._n:
             n0 = max(0, k1 - self._back)
             self._start(n0, min(self._n, n0 + (k1 - k0) + self._back))
