@@ -8,7 +8,7 @@
 // needed, so H is written in one pass and nothing of grid size exists before it.
 //
 // SP_HD like ray_core.h: the same source is inlined into the sm_100a kernels and compiled by g++ into
-// tests/noise_harness.cpp and tests/noise_box_harness.cpp.
+// tests/host_harness.cpp.
 #pragma once
 #include "ray_core.h"
 

@@ -28,14 +28,11 @@ import torch
 def domain_fft(k_func, l_max, l_min, extent, res, factor=1, *, noise="numpy", seed=0, device="cuda"):
     """Returns the (2res, 2res, int(2res*factor)) field as a float64 torch tensor on ``device``, normalised to
     max |f| = 1.  k_func maps a float32 torch tensor of |k| to the power spectrum."""
-    nx = ny = 2 * res
-    nz = int(2 * res * factor)
-    dx = extent / res
-    kx = 2 * np.pi * np.fft.fftfreq(nx, d=dx)
-    kz = 2 * np.pi * np.fft.fftfreq(nz, d=dx)
+    k_axes = _k_axes(extent, res, factor)
     dev = torch.device(device)
     if noise == "philox":
-        return _philox_field(k_func, l_max, l_min, kx, kz, seed, dev)
+        return _philox_field(k_func, l_max, l_min, k_axes, seed, dev)
+    kx, _, kz = k_axes
     kxt, kzt = torch.from_numpy(kx).to(dev), torch.from_numpy(kz).to(dev)
     # np.meshgrid(kx, ky, kz) uses 'xy' indexing: axis 0 <- ky, axis 1 <- kx   (gaussian3D.py:238)
     k2 = kxt[None, :, None] ** 2 + kxt[:, None, None] ** 2 + kzt[None, None, :] ** 2
@@ -46,7 +43,7 @@ def domain_fft(k_func, l_max, l_min, extent, res, factor=1, *, noise="numpy", se
     S = torch.zeros_like(k)
     S[mask] = k_func(k[mask])
     del mask, k
-    shape = (ny, nx, nz)
+    shape = (len(kx), len(kx), len(kz))                        # (ny, nx, nz)
     if noise == "numpy":
         re = torch.from_numpy(np.random.normal(0, 1, shape)).to(dev)
         im = torch.from_numpy(np.random.normal(0, 1, shape)).to(dev)
@@ -60,6 +57,13 @@ def domain_fft(k_func, l_max, l_min, extent, res, factor=1, *, noise="numpy", se
     field = torch.fft.ifftn(spec).real
     del spec
     return field / field.abs().max()
+
+
+def _k_axes(extent, res, factor):
+    """The 2 pi fftfreq axes (kx, ky, kz) of domain_fft's (2res, 2res, int(2res * factor)) grid, spacing extent / res."""
+    dx = extent / res
+    kx = 2 * np.pi * np.fft.fftfreq(2 * res, d=dx)
+    return kx, kx, 2 * np.pi * np.fft.fftfreq(int(2 * res * factor), d=dx)
 
 
 def half_spectrum(k_func, l_max, l_min, k_axes, device="cuda"):
@@ -92,13 +96,13 @@ def spectrum_box(k_func, l_max, l_min, k_axes, order, lo, cnt, device="cuda"):
     return S.masked_fill_(~mask, 0.0)
 
 
-def _philox_field(k_func, l_max, l_min, kx, kz, seed, dev):
+def _philox_field(k_func, l_max, l_min, k_axes, seed, dev):
     if dev.type != "cuda":
         raise RuntimeError("noise='philox' is generated by a CUDA kernel and has no CPU path: use device='cuda' "
                            "(or noise='torch' / 'numpy' on the CPU)")
     from . import engine
-    shape = (len(kx), len(kx), len(kz))
-    S = half_spectrum(k_func, l_max, l_min, (kx, kx, kz), dev)
+    shape = tuple(len(k) for k in k_axes)
+    S = half_spectrum(k_func, l_max, l_min, k_axes, dev)
     H = engine.noise_spectrum(S, shape, seed)
     del S
     field = _irfftn_slabs(H, shape)
@@ -224,12 +228,7 @@ def domain_fft_slabs(k_func, l_max, l_min, extent, res, factor=1, *, axis, seed,
     another order); every plane is the same bits whatever window it is asked in.  ``source.shape`` is the grid,
     ``source.max_abs`` the normalisation, ``source.build_seconds`` the two construction passes.  Device memory: about 8
     bytes per grid point for the life of the source, plus a few blocks of ``block_planes`` planes.  CUDA only."""
-    nx = 2 * res
-    nz = int(2 * res * factor)
-    dx = extent / res
-    kx = 2 * np.pi * np.fft.fftfreq(nx, d=dx)
-    kz = 2 * np.pi * np.fft.fftfreq(nz, d=dx)
-    return _slabs(k_func, l_max, l_min, (kx, kx, kz), axis, seed, block_planes, device)
+    return _slabs(k_func, l_max, l_min, _k_axes(extent, res, factor), axis, seed, block_planes, device)
 
 
 def _slabs(k_func, l_max, l_min, k_axes, axis, seed, block_planes, device, **kw):
@@ -259,7 +258,5 @@ def turbulent_ne_slabs(res, *, probing_direction="z", ne0=1e25, dne=9e24, l_max=
     held but ``domain_fft_slabs``'s spectrum (about 8 bytes per point: 68.8 GB at 2048^3).  The values agree with
     turbulent_ne's to FFT rounding and are the same bits whatever window is asked for."""
     from . import engine
-    nx = 2 * res
-    k = 2 * np.pi * np.fft.fftfreq(nx, d=extent / res)
-    return _slabs(kolmogorov, l_max, l_min, (k, k, k), engine.AXIS[probing_direction], seed, block_planes, device,
-                  ne0=ne0, dne=dne)
+    return _slabs(kolmogorov, l_max, l_min, _k_axes(extent, res, 1), engine.AXIS[probing_direction], seed,
+                  block_planes, device, ne0=ne0, dne=dne)

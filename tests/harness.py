@@ -10,7 +10,8 @@ SO = os.path.join(HERE, "_build", "libhost_harness.so")
 SRC = os.path.join(HERE, "host_harness.cpp")
 DEPS = [SRC, os.path.join(HERE, "..", "synthpy_b200", "csrc", "ray_core.h"),
         os.path.join(HERE, "..", "synthpy_b200", "csrc", "field_prep.h"),
-        os.path.join(HERE, "..", "synthpy_b200", "csrc", "fresnel_core.h")]
+        os.path.join(HERE, "..", "synthpy_b200", "csrc", "fresnel_core.h"),
+        os.path.join(HERE, "..", "synthpy_b200", "csrc", "noise_core.h")]
 
 OPK = {"travel": 0, "travel_noE": 1, "lens": 2, "circ_ap": 3, "circ_stop": 4, "rect_ap": 5, "knife": 6, "ref_beam": 7}
 
@@ -77,6 +78,32 @@ class Harness:
     def philox(self, key, ctr):
         out = np.empty(4, dtype=np.uint32)
         self.lib.hh_philox(*(C.c_uint32(k) for k in key), *(C.c_uint32(c) for c in ctr), _p(out))
+        return out
+
+    def noise_full(self, shape, seed):
+        """Z of the turbulent-field noise at every full-grid index: complex128 of ``shape``."""
+        out = np.empty(shape, dtype=np.complex128)
+        self.lib.hh_noise_full(*(C.c_int(n) for n in shape), C.c_uint64(seed), _p(out))
+        return out
+
+    def noise_half(self, S, shape, seed):
+        """The half spectrum k_noise_spectrum writes: complex128 (n0, n1, n2 // 2 + 1) from float32 S of that shape."""
+        n0, n1, n2 = shape
+        S = np.ascontiguousarray(S, dtype=np.float32)
+        assert S.shape == (n0, n1, n2 // 2 + 1)
+        out = np.empty(S.shape, dtype=np.complex128)
+        self.lib.hh_noise_half(_p(S), *(C.c_int(n) for n in shape), C.c_uint64(seed), _p(out))
+        return out
+
+    def noise_box(self, S, shape, order, lo, cnt, seed):
+        """The box k_noise_spectrum_box writes: complex128 of shape (cnt[order[0]], cnt[order[1]], cnt[order[2]]) from
+        float32 S of that shape; lo, cnt per grid axis."""
+        S = np.ascontiguousarray(S, dtype=np.float32)
+        assert S.shape == tuple(cnt[o] for o in order)
+        ints = lambda v: (C.c_int * 3)(*(int(x) for x in v))
+        out = np.empty(S.shape, dtype=np.complex128)
+        self.lib.hh_noise_box(_p(S), *(C.c_int(n) for n in shape), ints(order), ints(lo), ints(cnt), C.c_uint64(seed),
+                              _p(out))
         return out
 
 

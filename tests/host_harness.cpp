@@ -1,4 +1,5 @@
-// CPU self-test build of the product's per-ray math (synthpy_b200/csrc/ray_core.h, field_prep.h).
+// CPU self-test build of the product's per-ray math (synthpy_b200/csrc/ray_core.h, field_prep.h), wave optics
+// (fresnel_core.h) and turbulent-field noise (noise_core.h).
 // The build container has no GPU; this harness lets the CPU test-suite run the very same source that is
 // inlined into the sm_100a kernels against the golden vectors.  It is TEST code: nothing in synthpy_b200/
 // loads it, and it is not a fallback.
@@ -505,4 +506,40 @@ extern "C" void hh_window(int M, double alpha, double* w) {
 
 extern "C" void hh_reflect(int n, int lo, int hi, int32_t* out) {
     for (int i = lo; i < hi; ++i) out[i - lo] = (int32_t)reflect_idx(i, n);
+}
+
+// ---- turbulent-field noise (noise_core.h): the loops of k_noise_spectrum / k_noise_spectrum_box run serially -------
+#include "../synthpy_b200/csrc/noise_core.h"
+
+// Z at every full-grid index, complex128 interleaved [n0][n1][n2]
+extern "C" void hh_noise_full(int n0, int n1, int n2, uint64_t seed, double* out) {
+    const uint64_t n = (uint64_t)n0 * n1 * n2;
+    for (uint64_t f = 0; f < n; ++f) noise_z(seed, f, out[2 * f], out[2 * f + 1]);
+}
+
+// the half spectrum H that k_noise_spectrum writes, from S float32 [n0][n1][n2/2+1]
+extern "C" void hh_noise_half(const float* S, int n0, int n1, int n2, uint64_t seed, double* out) {
+    const int nh = n2 / 2 + 1;
+    for (int i = 0; i < n0; ++i)
+        for (int j = 0; j < n1; ++j)
+            for (int l = 0; l < nh; ++l) {
+                const uint64_t h = ((uint64_t)i * n1 + j) * nh + l;
+                const d2 v = noise_half(S[h], n0, n1, n2, seed, i, j, l);
+                out[2 * h] = v.x; out[2 * h + 1] = v.y;
+            }
+}
+
+// the box k_noise_spectrum_box writes: grid box [lo, lo + cnt) (per grid axis) in axis order `order`, from S float32 in the
+// same box layout
+extern "C" void hh_noise_box(const float* S, int n0, int n1, int n2, const int* order, const int* lo, const int* cnt,
+                             uint64_t seed, double* out) {
+    NoiseBox B;
+    for (int t = 0; t < 3; ++t) { B.order[t] = order[t]; B.lo[t] = lo[t]; B.dim[t] = cnt[order[t]]; }
+    for (int a = 0; a < B.dim[0]; ++a)
+        for (int b = 0; b < B.dim[1]; ++b)
+            for (int c = 0; c < B.dim[2]; ++c) {
+                const uint64_t h = ((uint64_t)a * B.dim[1] + b) * B.dim[2] + c;
+                const d2 v = noise_box(S[h], n0, n1, n2, seed, B, a, b, c);
+                out[2 * h] = v.x; out[2 * h + 1] = v.y;
+            }
 }

@@ -1,9 +1,9 @@
 """Turbulent-field noise drawn on the device (field_generator noise='philox', sp_noise_spectrum / k_noise_spectrum).
 
-CPU: the per-element source (noise_core.h) built by g++ (tests/noise_harness.cpp): the Hermitian half spectrum it writes is
-the full complex path's field after irfftn, its noise is N(0, 1) and independent, and the C ABI validates its arguments
-before any CUDA call.  GPU (-m gpu): the kernel against the host build, the product path against the full complex path,
-the spectrum at 512^3, memory and host-to-device traffic at 256^3, a traced field, and two GPUs."""
+CPU: the per-element source (noise_core.h) built by g++ (tests/host_harness.cpp): the Hermitian half spectrum it writes
+is the full complex path's field after irfftn, its noise is N(0, 1) and independent, and the C ABI validates its
+arguments before any CUDA call.  GPU (-m gpu): the kernel against the host build, the product path against the full
+complex path, the spectrum at 512^3, memory and host-to-device traffic at 256^3, a traced field, and two GPUs."""
 import ctypes as C
 import json
 import os
@@ -24,15 +24,14 @@ BAND = (4.0, 1.0)           # l_max, l_min: a band that cuts both ends of the sm
 
 @pytest.fixture(scope="module")
 def H():
-    from noise_harness import NoiseHarness
-    return NoiseHarness()
+    from harness import Harness
+    return Harness()
 
 
 @pytest.fixture(scope="module")
-def philox():
+def philox(H):
     """The Philox4x32-10 block function of the host build (ray_core.h)."""
-    from harness import Harness
-    return Harness().philox
+    return H.philox
 
 
 def _k(shape, extent=5.0):

@@ -26,12 +26,9 @@ BAND = (4.0, 1.0)           # l_max, l_min: a band that cuts both ends of the sm
 
 @pytest.fixture(scope="module")
 def H():
-    """The host builds of noise_core.h: noise_half / noise_full (noise_harness) and noise_box (noise_box_harness)."""
-    from noise_box_harness import NoiseBoxHarness
-    from noise_harness import NoiseHarness
-    h = NoiseHarness()
-    h.noise_box = NoiseBoxHarness().noise_box
-    return h
+    """The host build of noise_core.h: noise_half, noise_full and noise_box."""
+    from harness import Harness
+    return Harness()
 
 
 def _k(shape, extent=5.0):
