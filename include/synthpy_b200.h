@@ -266,6 +266,33 @@ int sp_propagate(const sp_field* field, const sp_params* params, sp_workspace* w
                  double* jf_dev, uint32_t* steps_dev, const sp_channel* channels_host, int n_channels,
                  sp_stats* stats_dev, void* stream);
 
+/* One slab of an out-of-core adaptive solve (synthpy_b200/out_of_core.py): SP_METHOD_RK45 per ray or SP_METHOD_TSIT5,
+ * resumable, on a field that holds only some planes of the probing axis.  [w_lo, w_hi] (probing-axis coordinate; +-inf
+ * at a grid edge) is where the slab's field equals the whole grid's.  A ray whose next attempt -- or RK45's initial-step
+ * probe -- would evaluate the field outside it, at a point inside the whole grid, PARKS: the attempt is dropped and the controller record keeps the state of
+ * the top of that loop iteration, so the next launch, over a slab that holds the point, resumes exactly.  Every committed
+ * attempt is the arithmetic of sp_propagate, so the per-slab launches give its results bit for bit.  [g_lo, g_hi] is the
+ * whole grid's probing-axis range: points beyond it read the fill value 0 from any slab, as from the whole grid.
+ *   state_dev (9 x n float64)  the ODE state, read and written (parked and finished rays alike)
+ *   idx_dev   n_idx uint32 indices of the rays to process, or NULL for all n (finished rays are skipped either way)
+ *   ctl_dev   (3 x n float64)  record rows: t (RK45) / tau (Tsit5); h_abs / dt; w of the point that parked the ray
+ *   ctl_flags_dev (n uint32)   SP_CTL_* bits;  steps_dev (n uint32) attempts so far.  All three start zeroed.
+ *   rf_dev, jf_dev, channels: written / binned for the rays that FINISH in this launch (t == t_end, early exit, or
+ *           failed) -- images are integer sums, so binning each ray in the launch it finishes in gives the in-core image.
+ *   stats_dev: ray_steps, ray_steps_acc, rays_capped, rays_binned and rays_rejected count committed work and sum over the
+ *           launches to sp_propagate's values; rhs_evals counts every evaluation, those of dropped attempts included (the
+ *           out-of-core overhead).
+ * SP_EINVAL before any CUDA call: other methods, SP_FLAG_BUNDLE_STEP / SP_FLAG_ATTEN / SP_FLAG_FARADAY, w_lo > w_hi, a
+ * field not marched along the probing axis, null pointers. */
+#define SP_CTL_STARTED 1u     /* RK45: initial step chosen / Tsit5: dt holds the controller's step                     */
+#define SP_CTL_PENDING 2u     /* RK45: a rejected attempt is pending                                                    */
+#define SP_CTL_FINISHED 4u    /* the ray is done and its epilogue has run                                               */
+#define SP_CTL_FAILED 8u      /* attempt cap, step below min_step, or NaN error norm                                    */
+int sp_propagate_window(const sp_field* field, const sp_params* params, sp_workspace* ws, double* state_dev, uint64_t n,
+                        const uint32_t* idx_dev, uint64_t n_idx, double* ctl_dev, uint32_t* ctl_flags_dev,
+                        uint32_t* steps_dev, double w_lo, double w_hi, double g_lo, double g_hi, double* rf_dev, double* jf_dev,
+                        const sp_channel* channels_host, int n_channels, sp_stats* stats_dev, void* stream);
+
 /* Device time of the k_propagate launches issued through `ws` since the last call (CUDA events recorded
  * around each launch on its stream; this call waits for the last one).  bench.py's roofline figure. */
 int sp_workspace_propagate_ms(sp_workspace* ws, double* total_ms, int* n_launches);

@@ -710,9 +710,23 @@ template <typename T> struct StageSmem {
 };
 #define SP_STAGE_DOUBLES 19
 
-template <typename T, bool PHASE, bool AUX64, typename Store>
+// ---- windowed integration (out-of-core tracing) ------------------------------------------------------------------
+// [lo, hi] along kernel axis w (the probing axis) is where the resident slab's field equals the whole grid's; so does every
+// point outside the whole grid (w outside [g_lo, g_hi], the grid's w range, or u / v outside the axes the slab shares with
+// the grid), where both give the fill value 0.  An attempt with a point anywhere else is abandoned before that point is
+// evaluated (WIN instantiations only): *out is set to the point's w and the caller discards the attempt.  NaN is never
+// outside, so a NaN ray fails as it does in core.
+struct Window { double lo, hi, g_lo, g_hi; };
+template <typename T> SP_HD bool outside(const Window& W, const FieldView<T>& F, const T* p) {
+    const double w = (double)p[2];
+    if (!(w < W.lo || w > W.hi)) return false;
+    if (w < W.g_lo || w > W.g_hi) return false;
+    return !(p[0] < F.ax[0].lo || p[0] > F.ax[0].hi || p[1] < F.ax[1].lo || p[1] > F.ax[1].hi);
+}
+
+template <typename T, bool PHASE, bool AUX64, typename Store, bool WIN = false>
 SP_HD int dp5_attempt(const FieldView<T>& F, T omega, T h, T rtol, T atol, const Ray<T>& r, const Deriv<T>& k1,
-                      Ray<T>& rn, Deriv<T>& k7, T& err_sq, Store& S) {
+                      Ray<T>& rn, Deriv<T>& k7, T& err_sq, Store& S, const Window* W = nullptr, double* out = nullptr) {
     T n7 = (T)0;
     const T* K1 = k1.dv;
     const T h2 = h * h;
@@ -762,6 +776,7 @@ SP_HD int dp5_attempt(const FieldView<T>& F, T omega, T h, T rtol, T atol, const
                 rn.ph = r.ph + h * ((T)DP::b1 * k1.dph + omega * ((T)DP::b3 * S.N(0) + (T)DP::b4 * S.N(1) + (T)DP::b5 * S.N(2) + (T)DP::b6 * S.N(3)));
             break;
         }
+        if (WIN && outside(*W, F, p)) { *out = (double)p[2]; return touched; }
         T a0, a1, a2, nn;
         touched += rhs_direct<T, PHASE, AUX64>(F, p[0], p[1], p[2], a0, a1, a2, nn);
         switch (s) {
@@ -828,9 +843,9 @@ template <typename T> SP_HD T dp5_factor(T en, bool accepted, bool rejected_befo
 
 // Hairer's initial step as coded in scipy/integrate/_ivp/common.py::select_initial_step (order = 4), with
 // the RMS norms taken over the ray's own n_state components (amp contributes (amp/scale)^2 to d0 only).
-template <typename T, bool PHASE, bool AUX64>
+template <typename T, bool PHASE, bool AUX64, bool WIN = false>
 SP_HD T dp5_initial_step(const FieldView<T>& F, T omega, T t_end, T rtol, T atol, int n_state, T amp, T pol,
-                         const Ray<T>& r, const Deriv<T>& f0, int& touched) {
+                         const Ray<T>& r, const Deriv<T>& f0, int& touched, const Window* W = nullptr, double* out = nullptr) {
     if (t_end == (T)0) return (T)0;
     const T inv_n = (T)1 / (T)n_state;
     T s0 = (T)0, s1 = (T)0;
@@ -856,6 +871,7 @@ SP_HD T dp5_initial_step(const FieldView<T>& F, T omega, T t_end, T rtol, T atol
     T p1[3], v1[3];
 #pragma unroll
     for (int c = 0; c < 3; ++c) { p1[c] = r.p[c] + h0 * f0.dp[c]; v1[c] = r.v[c] + h0 * f0.dv[c]; }
+    if (WIN && outside(*W, F, p1)) { *out = (double)p1[2]; return (T)0; }
     Deriv<T> f1;
     touched += deriv_direct<T, PHASE, AUX64>(F, omega, p1, v1, f1);
     T s2 = (T)0;
@@ -891,8 +907,9 @@ SP_HD int tsit5_f(const FieldView<T>& F, T omega, const T* y, T* f) {
     return t;
 }
 
-template <typename T, bool PHASE, bool AUX64>
-SP_HD int tsit5_attempt(const FieldView<T>& F, T omega, T h, T rtol, T atol, const T* y, const T* k1, T* yn, T* k7, T& err_sq) {
+template <typename T, bool PHASE, bool AUX64, bool WIN = false>
+SP_HD int tsit5_attempt(const FieldView<T>& F, T omega, T h, T rtol, T atol, const T* y, const T* k1, T* yn, T* k7, T& err_sq,
+                        const Window* W = nullptr, double* out = nullptr) {
     const double A[5][5] = {{0.161, 0, 0, 0, 0},
                             {-0.008480655492356989, 0.335480655492357, 0, 0, 0},
                             {2.8971530571054935, -6.359448489975075, 4.3622954328695815, 0, 0},
@@ -910,6 +927,7 @@ SP_HD int tsit5_attempt(const FieldView<T>& F, T omega, T h, T rtol, T atol, con
             for (int j = 1; j < s; ++j) acc += (T)A[s - 1][j] * K[j][i];
             ys[i] = y[i] + acc * h;
         }
+        if (WIN && outside(*W, F, ys)) { *out = (double)ys[2]; return touched; }
         touched += tsit5_f<T, PHASE, AUX64>(F, omega, ys, K[s]);
     }
     for (int i = 0; i < 7; ++i) {
@@ -917,6 +935,7 @@ SP_HD int tsit5_attempt(const FieldView<T>& F, T omega, T h, T rtol, T atol, con
         for (int j = 1; j < 6; ++j) acc += (T)B[j] * K[j][i];
         yn[i] = y[i] + h * acc;
     }
+    if (WIN && outside(*W, F, yn)) { *out = (double)yn[2]; return touched; }
     touched += tsit5_f<T, PHASE, AUX64>(F, omega, yn, K[6]);
     T tot = (T)0;
     for (int i = 0; i < 7; ++i) {
@@ -938,6 +957,148 @@ template <typename T> SP_HD T pid_factor(T err, bool keep) {
     if (err == (T)0) return (T)10;
     const T f = (T)0.9 * pow(err, (T)-0.2);
     return f < fmin_ ? fmin_ : (f > (T)10 ? (T)10 : f);
+}
+
+// ---- the per-ray adaptive solves restricted to a window (out-of-core tracing, sp_propagate_window) -----------------
+// The controller loops of k_propagate's SP_METHOD_RK45 and SP_METHOD_TSIT5 branches, resumable: a ray PARKS when its
+// next attempt (or RK45's initial-step probe p + h0 f0) would evaluate the field outside the window W.  The attempt is
+// dropped -- no attempt counted, no state committed -- and the record is left exactly as it was at the top of that loop
+// iteration (h before the clip to t_end: storing the clipped one would move the final step by an ulp on resume; the
+// min_step clamp is idempotent).  The next launch, over a slab that holds the point, resumes from the record: the FSAL
+// derivative is recomputed at the committed state (rhs_direct has no cache, so it is the same bits) and min_step from t.
+// Every committed attempt therefore does exactly the in-core arithmetic.  One code for the kernels and the CPU test
+// build; the warp vote only keeps the lanes converged.
+#define SP_CTL_STARTED 1u     // RK45: initial step chosen / Tsit5: dt holds the controller's step
+#define SP_CTL_PENDING 2u     // RK45: a rejected attempt is pending (the retry keeps min_step and the rejected flag)
+#define SP_CTL_FINISHED 4u    // t == t_end, escaped (early exit) or failed: the epilogue has run
+#define SP_CTL_FAILED 8u      // attempt cap, step below min_step, or NaN error norm
+struct WinCtl {
+    double t, h;              // RK45: t, h_abs / Tsit5: tau, dt
+    double w_park;            // w of the point that parked the ray (the next window must hold it)
+    unsigned n_att, flags;
+};
+
+#if defined(__CUDA_ARCH__)
+#define SP_WIN_VOTE(lanes, go) __any_sync(lanes, go)
+#else
+#define SP_WIN_VOTE(lanes, go) (go)
+#endif
+
+template <typename T, bool PHASE, bool AUX64, typename Store>
+SP_HD int dp5_window(const FieldView<T>& F, const Window& W, T omega, T t_end, T rtol, T atol, int n_state, T amp, T pol,
+                     unsigned cap, bool early, unsigned lanes, Ray<T>& r, WinCtl& c, Store& S, unsigned& acc, unsigned& capped) {
+    int touched = 0;
+    const bool skip = (c.flags & SP_CTL_FINISHED) != 0;   // finished in an earlier launch: takes part in the votes only
+    double pw = NAN;                                       // set (not NaN) once the ray parks
+    if (skip) pw = 0.0;
+    else if (outside(W, F, r.p)) pw = (double)r.p[2];   // before the escape test: the slab's w bounds are not the grid's
+    T t = (T)c.t, h_abs = (T)c.h;
+    unsigned n_att = c.n_att;
+    bool failed = false, rejected = (c.flags & SP_CTL_PENDING) != 0, fresh = !rejected, started = (c.flags & SP_CTL_STARTED) != 0;
+    T min_step = (T)10 * (nextafter(t, (T)INFINITY) - t);
+    const T inv_n = (T)1 / (T)n_state;
+    Deriv<T> f;
+    f.dp[0] = f.dp[1] = f.dp[2] = f.dv[0] = f.dv[1] = f.dv[2] = f.dph = (T)0;
+    if (pw != pw) {
+        touched += deriv_direct<T, PHASE, AUX64>(F, omega, r.p, r.v, f);
+        if (!started) {
+            const T h0 = dp5_initial_step<T, PHASE, AUX64, true>(F, omega, t_end, rtol, atol, n_state, amp, pol, r, f, touched, &W, &pw);
+            if (pw != pw) { h_abs = h0; started = true; }
+        }
+    }
+    for (;;) {
+        bool go = (pw != pw) && (t < t_end) && !failed;
+        const T h_top = h_abs;
+        const bool fresh_top = fresh;
+        if (go && fresh) {
+            if (early && escaped(F, r)) go = false;
+            else {
+                min_step = (T)10 * (nextafter(t, (T)INFINITY) - t);
+                if (h_abs < min_step) h_abs = min_step;
+                rejected = false; fresh = false;
+            }
+        }
+        if (go && (n_att >= cap || h_abs < min_step)) { failed = true; capped += 1; go = false; }
+        if (!SP_WIN_VOTE(lanes, go)) break;
+        if (go) {
+            T t_new = t + h_abs;
+            if (t_new - t_end > (T)0) t_new = t_end;
+            const T h = t_new - t;
+            h_abs = fabs(h);
+            Ray<T> rn; Deriv<T> fn; T esq;
+            touched += dp5_attempt<T, PHASE, AUX64, Store, true>(F, omega, h, rtol, atol, r, f, rn, fn, esq, S, &W, &pw);
+            if (pw == pw) { h_abs = h_top; fresh = fresh_top; }          // parked: the record as at the top of this iteration
+            else {
+                ++n_att;
+                const T en = sqrt(esq * inv_n);
+                if (!(en == en)) { failed = true; capped += 1; }
+                else {
+                    const bool acc_ = en < (T)1;
+                    h_abs *= dp5_factor<T>(en, acc_, rejected);
+                    if (acc_) { t = t_new; r = rn; f = fn; acc += 1; fresh = true; }
+                    else rejected = true;
+                }
+            }
+        }
+    }
+    if (skip) return touched;
+    c.t = (double)t; c.h = (double)h_abs; c.n_att = n_att; c.w_park = pw;
+    c.flags = (started ? SP_CTL_STARTED : 0u) | (fresh ? 0u : SP_CTL_PENDING) | (pw != pw ? SP_CTL_FINISHED : 0u) | (failed ? SP_CTL_FAILED : 0u);
+    return touched;
+}
+
+// Tsit5 + PID per ray (k_propagate's SP_METHOD_TSIT5 branch), resumable in the same way; dt0 is taken when !STARTED.
+template <typename T, bool PHASE, bool AUX64>
+SP_HD int tsit5_window(const FieldView<T>& F, const Window& W, T omega, T t_end, T dt0, T rtol, T atol, int n_state,
+                       unsigned cap, unsigned lanes, Ray<T>& r, WinCtl& c, unsigned& acc, unsigned& capped) {
+    int touched = 0;
+    const bool skip = (c.flags & SP_CTL_FINISHED) != 0;
+    double pw = NAN;
+    if (skip) pw = 0.0;
+    else if (outside(W, F, r.p)) pw = (double)r.p[2];
+    T y[7], f[7], yn[7], fn[7];
+#pragma unroll
+    for (int k = 0; k < 3; ++k) { y[k] = r.p[k]; y[3 + k] = r.v[k]; }
+    y[6] = r.ph;
+#pragma unroll
+    for (int k = 0; k < 7; ++k) f[k] = (T)0;
+    if (pw != pw) touched += tsit5_f<T, PHASE, AUX64>(F, omega, y, f);
+    T tau = (T)c.t, dt = (c.flags & SP_CTL_STARTED) ? (T)c.h : dt0;
+    unsigned n_att = c.n_att;
+    const T inv_n = (T)1 / (T)n_state;
+    bool failed = false;
+    for (;;) {
+        bool go = (pw != pw) && (tau < (T)1) && !failed;
+        if (go && n_att >= cap) { failed = true; capped += 1; go = false; }
+        if (!SP_WIN_VOTE(lanes, go)) break;
+        if (go) {
+            const bool last = tau + dt >= (T)1;
+            const T d = last ? (T)1 - tau : dt;
+            T esq;
+            touched += tsit5_attempt<T, PHASE, AUX64, true>(F, omega, d * t_end, rtol, atol, y, f, yn, fn, esq, &W, &pw);
+            if (pw != pw) {
+                ++n_att;
+                const T en = sqrt(esq * inv_n);
+                if (!(en == en)) { failed = true; capped += 1; }
+                else {
+                    const bool keep = en < (T)1;
+                    dt = d * pid_factor<T>(en, keep);
+                    if (keep) {
+                        tau = last ? (T)1 : tau + d; acc += 1;
+#pragma unroll
+                        for (int i = 0; i < 7; ++i) { y[i] = yn[i]; f[i] = fn[i]; }
+                    }
+                }
+            }
+        }
+    }
+    if (skip) return touched;
+#pragma unroll
+    for (int k = 0; k < 3; ++k) { r.p[k] = y[k]; r.v[k] = y[3 + k]; }
+    r.ph = y[6];
+    c.t = (double)tau; c.h = (double)dt; c.n_att = n_att; c.w_park = pw;
+    c.flags = SP_CTL_STARTED | (pw != pw ? SP_CTL_FINISHED : 0u) | (failed ? SP_CTL_FAILED : 0u);
+    return touched;
 }
 
 // ---- Dormand-Prince on the full 9-component state (attenuation / Faraday channels on; slow path) ----------------

@@ -345,6 +345,8 @@ extern "C" int sp_field_export_gradients(const sp_field* f, float* gx_dev, float
 #define SP_METHOD_RK4X 3      // internal: RK4 with the attenuation / Faraday channels (float64)
 #define SP_METHOD_RK45X 4     // internal: per-ray Dormand-Prince over all nine rows (channels on, float64)
 #define SP_METHOD_RK45B 5     // internal: Dormand-Prince with one step size per 32-ray bundle (SP_FLAG_BUNDLE_STEP)
+#define SP_METHOD_RK45W 7     // internal: per-ray Dormand-Prince restricted to a window along w (sp_propagate_window)
+#define SP_METHOD_TSIT5W 8    // internal: per-ray Tsit5 restricted to a window along w (sp_propagate_window)
 #define SP_MAX_OPS 16
 #define SP_MAX_CHANNELS 4
 
@@ -451,6 +453,9 @@ struct Epilogue {
     double* sf; double* rf; double* jf; uint32_t* steps;
     int n_channels;
     ChannelDev ch[SP_MAX_CHANNELS];
+    // SP_METHOD_RK45W / SP_METHOD_TSIT5W only: the window, and the controller record (ctl: t, h, w_park rows of n_total
+    // doubles; ctl_flags: SP_CTL_* bits).  sf is then the state itself and steps the attempt count, both read and written.
+    Window win; double* ctl; uint32_t* ctl_flags;
 };
 
 // --------------------------------------------------------------------------------------------- ray sorting
@@ -864,7 +869,8 @@ __global__ void __launch_bounds__(128, (METHOD == SP_METHOD_RK4 && sizeof(T) == 
 #pragma unroll
         for (int k = 0; k < 3; ++k) { r.p[k] = (T)s[A.perm[k]]; r.v[k] = (T)s[3 + A.perm[k]]; }
         r.ph = (T)ph0;
-        unsigned n_att = 0;
+        unsigned n_att = 0, n_att0 = 0;           // n_att0: attempts of earlier launches (windowed methods)
+        bool fin = true;                          // windowed methods: the ray finishes in this launch (it did not park)
         CellCache<T, PHASE> cc;
         double amp_x = 1.0, pol_x = 0.0;
         if (METHOD == SP_METHOD_RK45B) {
@@ -918,6 +924,28 @@ __global__ void __launch_bounds__(128, (METHOD == SP_METHOD_RK4 && sizeof(T) == 
                 r.ph = y[6];
             } else if (METHOD == SP_METHOD_RK45B) {
                 // handled above (whole-warp path)
+            } else if (METHOD == SP_METHOD_RK45W || METHOD == SP_METHOD_TSIT5W) {
+                // one slab of an out-of-core solve: resume from the record, park at the window (ray_core.h dp5_window)
+                const uint64_t N = A.n_total;
+                WinCtl c;
+                c.t = E.ctl[gi]; c.h = E.ctl[N + gi]; c.w_park = E.ctl[2 * N + gi]; c.n_att = E.steps[gi]; c.flags = E.ctl_flags[gi];
+                n_att0 = c.n_att;
+                const bool before = (c.flags & SP_CTL_FINISHED) != 0;         // finished in an earlier launch: a no-op
+                unsigned acc = 0, capped = 0;
+                if (METHOD == SP_METHOD_RK45W) {
+                    const unsigned cap = A.n_steps > 0 ? (unsigned)A.n_steps : (1u << 30);
+                    ls.evals += dp5_window<T, PHASE, AUX64, StageSmem<T> >(A.F, E.win, A.omega, A.t_end, A.rtol, A.atol, A.n_state,
+                                                                          (T)A.s0[6 * N + gi], (T)A.s0[8 * N + gi], cap, early, vmask,
+                                                                          r, c, S, acc, capped);
+                } else {
+                    const unsigned cap = A.n_steps > 0 ? (unsigned)A.n_steps : 10000u;
+                    ls.evals += tsit5_window<T, PHASE, AUX64>(A.F, E.win, A.omega, A.t_end, A.h, A.rtol, A.atol, A.n_state, cap, vmask,
+                                                              r, c, acc, capped);
+                }
+                ls.acc += acc; ls.capped += capped;
+                n_att = c.n_att;
+                fin = !before && (c.flags & SP_CTL_FINISHED) != 0;
+                E.ctl[gi] = c.t; E.ctl[N + gi] = c.h; E.ctl[2 * N + gi] = c.w_park; E.ctl_flags[gi] = c.flags;
             } else if (METHOD == SP_METHOD_RK4) {
                 for (int it = 0; it < A.n_steps; ++it) {
                     const int t = rk4_step<T, PHASE, AUX64>(A.F, cc, A.rk, A.omega, r, early);
@@ -975,7 +1003,7 @@ __global__ void __launch_bounds__(128, (METHOD == SP_METHOD_RK4 && sizeof(T) == 
                 }
                 ls.evals += touched;
             }
-            ls.steps += n_att;
+            ls.steps += n_att - n_att0;
         }
         // ---- epilogue: exit plane, outputs, fused optics + binning ----
         T xa = 0, tha = 0, xb = 0, thb = 0;
@@ -1009,15 +1037,17 @@ __global__ void __launch_bounds__(128, (METHOD == SP_METHOD_RK4 && sizeof(T) == 
                 E.jf[2 * gi] = ex_re; E.jf[2 * gi + 1] = ex_im;
                 E.jf[2 * (N + gi)] = ey_re; E.jf[2 * (N + gi) + 1] = ey_im;
             }
+            // windowed methods: rf / jf of a parked ray are overwritten in the launch it finishes in, but it is binned only there
+            const bool done = (METHOD == SP_METHOD_RK45W || METHOD == SP_METHOD_TSIT5W) ? (valid && fin) : valid;
             for (int c = 0; c < E.n_channels; ++c) {
                 const ChannelDev& ch = E.ch[c];
                 DetRay d;
                 d.x = (double)xa * 1e3; d.th = (double)tha; d.y = (double)xb * 1e3; d.ph = (double)thb;   // m_to_mm
-                d.ex_re = ex_re; d.ex_im = ex_im; d.ey_re = ey_re; d.ey_im = ey_im; d.alive = valid;
-                if (valid) run_optics(d, (double)xa, (double)xb, ch.ops, ch.n_ops, ch.with_E != 0, ch.kwave);
-                const int b = bin_ray(ch, d, valid);
+                d.ex_re = ex_re; d.ex_im = ex_im; d.ey_re = ey_re; d.ey_im = ey_im; d.alive = done;
+                if (done) run_optics(d, (double)xa, (double)xb, ch.ops, ch.n_ops, ch.with_E != 0, ch.kwave);
+                const int b = bin_ray(ch, d, done);
                 ls.binned += b;
-                ls.rejected += (valid && !d.alive) ? 1 : 0;
+                ls.rejected += (done && !d.alive) ? 1 : 0;
             }
         }
         if (A.stats) {
@@ -1511,7 +1541,7 @@ static int kernel_index_of(const sp_field* f, int caller_axis) {
 }
 
 template <typename T, int METHOD> static constexpr size_t stage_smem_bytes() {
-    return (METHOD == SP_METHOD_RK45 || METHOD == SP_METHOD_RK45B) ? (size_t)SP_STAGE_DOUBLES * 128 * sizeof(T) : 0;
+    return (METHOD == SP_METHOD_RK45 || METHOD == SP_METHOD_RK45B || METHOD == SP_METHOD_RK45W) ? (size_t)SP_STAGE_DOUBLES * 128 * sizeof(T) : 0;
 }
 
 template <typename T, int METHOD>
@@ -1695,6 +1725,76 @@ extern "C" int sp_propagate(const sp_field* field, const sp_params* P, sp_worksp
             FILL(double)
             rc = (P->method == SP_METHOD_RK4) ? launch_propagate<double, SP_METHOD_RK4>(A, E, g, st)
                  : (bundle_step ? launch_propagate<double, SP_METHOD_RK45B>(A, E, g, st) : launch_propagate<double, SP_METHOD_RK45>(A, E, g, st));
+        }
+#undef FILL
+        if (rc) return rc;
+        rc = ws_event(ws, st);
+        if (rc) return rc;
+    }
+    return SP_OK;
+}
+
+extern "C" int sp_propagate_window(const sp_field* field, const sp_params* P, sp_workspace* ws, double* state_dev, uint64_t n,
+                                   const uint32_t* idx_dev, uint64_t n_idx, double* ctl_dev, uint32_t* ctl_flags_dev,
+                                   uint32_t* steps_dev, double w_lo, double w_hi, double g_lo, double g_hi, double* rf_dev, double* jf_dev,
+                                   const sp_channel* channels_host, int n_channels, sp_stats* stats_dev, void* stream) {
+    if (!field || !P || !ws) return fail(SP_EINVAL, "null field / params / workspace");
+    if (!state_dev || !ctl_dev || !ctl_flags_dev || !steps_dev) return fail(SP_EINVAL, "null state / controller record / steps");
+    if (!(w_lo <= w_hi)) return fail(SP_EINVAL, "window needs w_lo <= w_hi");
+    if (!(g_lo <= g_hi)) return fail(SP_EINVAL, "grid range needs g_lo <= g_hi");
+    if (P->method != SP_METHOD_RK45 && P->method != SP_METHOD_TSIT5)
+        return fail(SP_EINVAL, "sp_propagate_window takes SP_METHOD_RK45 (per ray) or SP_METHOD_TSIT5");
+    if (P->flags & (SP_FLAG_BUNDLE_STEP | SP_FLAG_ATTEN | SP_FLAG_FARADAY))
+        return fail(SP_EINVAL, "sp_propagate_window: no bundle-step RK45 and no attenuation / Faraday channels");
+    if (n_channels < 0 || n_channels > SP_MAX_CHANNELS) return fail(SP_EINVAL, "at most 4 detector channels");
+    if (P->probing_axis < 0 || P->probing_axis > 2 || P->out_axis_a < 0 || P->out_axis_a > 2 || P->out_axis_b < 0 ||
+        P->out_axis_b > 2)
+        return fail(SP_EINVAL, "axis index out of range");
+    if (kernel_index_of(field, P->probing_axis) != 2) return fail(SP_EINVAL, "the field must march along the probing axis (the window is along it)");
+    if (P->method == SP_METHOD_TSIT5 && (!(P->h > 0) || !(P->t_end > 0))) return fail(SP_EINVAL, "tsit5 needs h = dt0 > 0 (units of t_end) and t_end > 0");
+    if ((P->flags & SP_FLAG_PHASE_F64) && !field->aux64) return fail(SP_ESTATE, "field was built without SP_FIELD_PHASE_F64");
+    const uint64_t m = idx_dev ? n_idx : n;
+    if (m == 0) return SP_OK;
+    cudaStream_t st = (cudaStream_t)stream;
+    Epilogue E; memset(&E, 0, sizeof(E));
+    E.sf = state_dev; E.rf = rf_dev; E.jf = jf_dev; E.steps = steps_dev; E.n_channels = n_channels;
+    E.win.lo = w_lo; E.win.hi = w_hi; E.win.g_lo = g_lo; E.win.g_hi = g_hi; E.ctl = ctl_dev; E.ctl_flags = ctl_flags_dev;
+    for (int c = 0; c < n_channels; ++c) {
+        int rc = channel_to_dev(channels_host + c, E.ch[c]);
+        if (rc) return rc;
+    }
+    const bool fp32 = (P->flags & SP_FLAG_FP32) != 0, tsit = P->method == SP_METHOD_TSIT5;
+    int grid = 0, rc;
+    if (tsit) rc = fp32 ? occupancy_grid<float, SP_METHOD_TSIT5W>(ws->sm_count, P->flags, grid) : occupancy_grid<double, SP_METHOD_TSIT5W>(ws->sm_count, P->flags, grid);
+    else rc = fp32 ? occupancy_grid<float, SP_METHOD_RK45W>(ws->sm_count, P->flags, grid) : occupancy_grid<double, SP_METHOD_RK45W>(ws->sm_count, P->flags, grid);
+    if (rc) return rc;
+    const uint64_t CHUNK = 1ull << 25;
+    for (uint64_t off = 0; off < m; off += CHUNK) {
+        const uint32_t cn = (uint32_t)((m - off) < CHUNK ? (m - off) : CHUNK);
+        CU(cudaMemsetAsync(ws->cursor, 0, sizeof(unsigned long long), st));
+        const uint64_t bundles = (cn + 31) / 32;
+        int g = grid;
+        if ((uint64_t)g * 4 > bundles) g = (int)((bundles + 3) / 4);
+        if (g < 1) g = 1;
+#define FILL(T)                                                                                          \
+        PropArgs<T> A; memset(&A, 0, sizeof(A));                                                         \
+        A.F = make_view<T>(field); A.s0 = state_dev; A.n_total = n;                                      \
+        A.chunk_off = idx_dev ? 0 : off; A.chunk_n = cn; A.order = idx_dev ? idx_dev + off : nullptr;    \
+        A.cursor = ws->cursor;                                                                           \
+        for (int k = 0; k < 3; ++k) A.perm[k] = field->perm[k];                                          \
+        A.kp = kernel_index_of(field, P->probing_axis); A.ka = kernel_index_of(field, P->out_axis_a);    \
+        A.kb = kernel_index_of(field, P->out_axis_b);                                                    \
+        A.method = P->method; A.flags = P->flags; A.n_steps = P->n_steps; A.n_state = P->n_state > 0 ? P->n_state : 9; \
+        A.h = (T)P->h; A.t_end = (T)P->t_end; A.rtol = (T)P->rtol; A.atol = (T)P->atol; A.omega = (T)P->omega; \
+        A.extent = (T)P->extent; A.stats = stats_dev;
+        rc = ws_event(ws, st);
+        if (rc) return rc;
+        if (fp32) {
+            FILL(float)
+            rc = tsit ? launch_propagate<float, SP_METHOD_TSIT5W>(A, E, g, st) : launch_propagate<float, SP_METHOD_RK45W>(A, E, g, st);
+        } else {
+            FILL(double)
+            rc = tsit ? launch_propagate<double, SP_METHOD_TSIT5W>(A, E, g, st) : launch_propagate<double, SP_METHOD_RK45W>(A, E, g, st);
         }
 #undef FILL
         if (rc) return rc;

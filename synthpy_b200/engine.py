@@ -362,6 +362,42 @@ def propagate(field, params, *, s0=None, beam=None, n=None, ray_offset=0, want_s
     return out
 
 
+def controller_record(n):
+    """Zeroed controller record of ``propagate_window`` for n rays: 'ctl' (3, n) float64 (t or tau, h_abs or dt, w of the
+    point that parked the ray), 'flags' (n,) int32 of SP_CTL_* bits, 'steps' (n,) int32 attempts so far."""
+    require_cuda()
+    return dict(ctl=torch.zeros((3, n), dtype=torch.float64, device="cuda"),
+                flags=torch.zeros(n, dtype=torch.int32, device="cuda"), steps=torch.zeros(n, dtype=torch.int32, device="cuda"))
+
+
+def propagate_window(field, params, state, record, w_lo, w_hi, grid_range, *, idx=None, rf=None, jf=None, channels=(),
+                     stats=None):
+    """One call of ``sp_propagate_window``: advance the rays ``idx`` (int32 CUDA tensor of indices, None = all) of the
+    (9, N) CUDA float64 ``state`` in place, each until it finishes or parks at the window [w_lo, w_hi] of the probing
+    axis (``grid_range``: the whole grid's extent along it).  ``record`` from ``controller_record``; ``rf`` (4, N) / ``jf`` (2, N) complex128 receive the rays that finish;
+    ``stats`` an int64 (6,) CUDA tensor accumulated into.  No sync."""
+    require_cuda()
+    if not (isinstance(state, torch.Tensor) and state.is_cuda and state.dtype == torch.float64 and state.is_contiguous()
+            and state.ndim == 2 and state.shape[0] == 9):
+        raise TypeError("state must be a contiguous (9, N) CUDA float64 tensor")
+    n = state.shape[1]
+    if idx is not None and not (idx.is_cuda and idx.dtype == torch.int32 and idx.is_contiguous()):
+        raise TypeError("idx must be a contiguous CUDA int32 tensor")
+    keep, structs = [], []
+    for ops, image, wl in channels:
+        if image is not None:
+            image.touched()
+        ch, k = make_channel(ops, image, wl)
+        structs.append(ch)
+        keep.append(k)
+    ch_arr = (L.Channel * max(1, len(structs)))(*structs)
+    L.check(L.lib.sp_propagate_window(field._h, C.byref(params), workspace(), _ptr(state), n, _ptr(idx),
+                                      0 if idx is None else idx.numel(), _ptr(record["ctl"]), _ptr(record["flags"]),
+                                      _ptr(record["steps"]), float(w_lo), float(w_hi), float(grid_range[0]),
+                                      float(grid_range[1]), _ptr(rf), _ptr(jf), ch_arr,
+                                      len(structs), _ptr(stats), _stream()))
+
+
 STAT_NAMES = ("ray_steps", "ray_steps_acc", "rays_capped", "rays_binned", "rays_rejected", "rhs_evals")
 
 

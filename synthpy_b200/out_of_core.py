@@ -6,9 +6,12 @@ progress upstream (the section bounds are hard-coded, domain.py:247-252).  On a 
 180 GB, so this is needed only from ~2048^3 upwards (137 GB packed) or when several fields share a GPU; it is built so
 that nothing about the result depends on it:
 
-  * fixed-step RK4 only (the ray ODE has no explicit time dependence, so N steps through the whole grid are N_1 + N_2 +
-    ... steps through consecutive slabs, the (9, N) state carried over exactly; an adaptive per-ray controller would see
-    different step sequences);
+  * fixed-step RK4: the ray ODE has no explicit time dependence, so N steps through the whole grid are N_1 + N_2 + ...
+    steps through consecutive slabs, the (9, N) state carried over exactly;
+  * the per-ray adaptive solves (method='rk45', 'tsit5'; ``trace_slabs_adaptive`` over ``sp_propagate_window``): a ray
+    parks when its next attempt would evaluate the field inside the grid but outside the slab's window, with its
+    controller record as at the top of that loop iteration, and resumes in a later slab; every committed attempt is the
+    in-core arithmetic (see ray_core.h dp5_window).  Joint and bundle-step RK45 stay in core;
   * a slab holds the planes [a, b] of the probing axis.  The float32 gradient stencil (field_prep.h) at plane k reads
     planes k-1 and k+1, so the edge planes of a slab carry one-sided differences that the whole grid would not: the
     planner keeps every RK stage of every live ray at least two planes inside (``plan_slab``), checks it afterwards on
@@ -111,13 +114,10 @@ def axis_is_uniform(a32):
     return bool(np.all(d == d[0])) if d.size else True
 
 
-def plan_slab(zc, zmin, zmax, vmax, h, steps_left, slab_planes):
-    """Which planes [a, b] to load and how many RK4 steps to take in them.
-
-    zc          the probing axis (float32 values as float64), n planes
-    zmin, zmax  extreme probing-axis positions of the live rays now;  vmax  their largest speed along that axis
-    Returns (a, b, m, z_stop): after m steps no live ray may be beyond z_stop (checked by the driver); ``b == n - 1``
-    means the slab reaches the end of the grid and takes all remaining steps."""
+def slab_planes_for(zc, zmin, slab_planes):
+    """The planes [a, b] of the next slab: from MARGIN planes behind the cell holding ``zmin`` (the slowest live ray),
+    ``slab_planes`` long, widened until its probing axis makes the same uniform / non-uniform stencil choice as the whole
+    axis (zc: the probing axis, float32 values as float64)."""
     n = len(zc)
     cell = int(np.clip(np.searchsorted(zc, zmin, side="right") - 1, 0, n - 2))       # cell holding the last ray
     a = max(0, cell - MARGIN)
@@ -128,6 +128,18 @@ def plan_slab(zc, zmin, zmax, vmax, h, steps_left, slab_planes):
             b += 1
         else:
             a -= 1
+    return a, b
+
+
+def plan_slab(zc, zmin, zmax, vmax, h, steps_left, slab_planes):
+    """Which planes [a, b] to load and how many RK4 steps to take in them.
+
+    zc          the probing axis (float32 values as float64), n planes
+    zmin, zmax  extreme probing-axis positions of the live rays now;  vmax  their largest speed along that axis
+    Returns (a, b, m, z_stop): after m steps no live ray may be beyond z_stop (checked by the driver); ``b == n - 1``
+    means the slab reaches the end of the grid and takes all remaining steps."""
+    n = len(zc)
+    a, b = slab_planes_for(zc, zmin, slab_planes)
     if b == n - 1:
         return a, b, int(steps_left), np.inf
     z_stop = float(zc[b - MARGIN])
@@ -228,23 +240,157 @@ def trace_slabs(backend, s0, source, axes, probing_direction, n_steps, h, slab_p
             return s, steps_total, rf, jf, log, stats_total
 
 
+class _AdaptiveDeviceBackend:
+    """The product path of the adaptive solves: packed slab field in HBM, ``sp_propagate_window`` per slab."""
+
+    def __init__(self, params, lwl, probing_direction, phase, phase_f64, want_jf):
+        import torch
+        self.torch, self.P, self.lwl, self.phase, self.phase_f64 = torch, params, lwl, phase, phase_f64
+        self.p = engine.AXIS[probing_direction]
+        self.want_jf = want_jf
+        self.stats = torch.zeros(6, dtype=torch.int64, device="cuda")
+
+    def to_state(self, s0):
+        s = engine.to_device(s0, self.torch.float64)
+        return s.clone() if isinstance(s0, self.torch.Tensor) else s        # advanced in place: never the caller's tensor
+
+    def record(self, n):
+        t = self.torch
+        rec = engine.controller_record(n)
+        rec["ctl"][2].fill_(np.inf)
+        self.rf = t.empty((4, n), dtype=t.float64, device="cuda")
+        self.jf = t.empty((2, n), dtype=t.complex128, device="cuda") if self.want_jf else None
+        return rec
+
+    def slowest(self, s, rec):
+        todo = (rec["flags"] & engine.L.CTL_FINISHED) == 0
+        if not bool(todo.any()):
+            return None
+        z = self.torch.minimum(s[self.p][todo], rec["ctl"][2][todo])
+        z = z[self.torch.isfinite(z)]
+        return float(z.min()) if z.numel() else -np.inf
+
+    def select(self, s, rec, w_lo, w_hi):
+        w = s[self.p]
+        ok = ((rec["flags"] & engine.L.CTL_FINISHED) == 0) & ~(w < w_lo) & ~(w > w_hi)      # NaN positions are inside
+        return self.torch.nonzero(ok).squeeze(1).to(self.torch.int32)
+
+    def summary(self, rec, idx, t_stop):
+        f, c = rec["flags"][idx.long()], rec["ctl"][:, idx.long()]
+        L = engine.L
+        parked = (f & L.CTL_FINISHED) == 0
+        return dict(attempts=int(rec["steps"].sum()), finished=int(((rec["flags"] & L.CTL_FINISHED) != 0).sum()),
+                    pending=int((parked & ((f & L.CTL_PENDING) != 0)).sum()),
+                    clip=int((parked & (c[0] + c[1] - t_stop > 0)).sum()))
+
+    def field(self, ne_slab, axes):
+        return engine.DeviceField.from_ne(ne_slab, axes[0], axes[1], axes[2], engine.omega_of(self.lwl), march_axis=self.p,
+                                          phase=self.phase, phase_f64=self.phase_f64)
+
+    def launch(self, field, s, rec, idx, w_lo, w_hi, grid_range, channels):
+        engine.propagate_window(field, self.P, s, rec, w_lo, w_hi, grid_range, idx=idx, rf=self.rf, jf=self.jf, channels=channels,
+                                stats=self.stats)
+
+    def release(self, field):
+        self.torch.cuda.current_stream().synchronize()
+        field.close()
+        self.torch.cuda.empty_cache()
+
+
+def trace_slabs_adaptive(backend, s0, source, axes, probing_direction, slab_planes, t_stop, *, max_slab_planes=None,
+                         channels=()):
+    """The slab loop of the adaptive solves (``backend``: the device, or the host build of the same ray code in the tests).
+    Each pass loads the slab from MARGIN planes behind the slowest unfinished ray (or the lowest point a parked ray needs)
+    and launches once over the unfinished rays inside its window; a ray runs until it finishes or parks at the window, and
+    resumes in a later slab from its controller record.  Returns (state, record, log): ``log`` one dict per slab with its
+    planes, window, rays launched, finished, parked, parked with a pending rejection ('parked_pending'), parked right
+    before their final step, the one clipped to the end of the interval ('parked_clip'), and committed attempts.
+    ``t_stop`` is where that clip happens in the record's time (t_end for RK45, 1 for Tsit5's normalised time).
+
+    A launch in which no ray commits an attempt or finishes leaves the state as it was: some attempt spans more planes than
+    the window.  The slab then doubles, up to ``max_slab_planes`` (default ``slab_planes``: no growth), and returns to
+    ``slab_planes`` after the next launch that makes progress.  SciPy's initial step is one such attempt: 100 h0 is of
+    the order of the distance from the origin, so the first (rejected) attempts of RK45 span much of the box.  A second
+    launch without progress at the largest slab raises ``ValueError`` instead of looping."""
+    p = engine.AXIS[probing_direction]
+    zc = np.asarray(np.float32(axes[p]), dtype=np.float64)
+    n = len(zc)
+    if int(slab_planes) < 2 * MARGIN + 2:
+        raise ValueError(f"slab_planes must be at least {2 * MARGIN + 2}: the window is the slab less {MARGIN} planes per side")
+    top = max(int(slab_planes), int(max_slab_planes or slab_planes))
+    grid_range = (float(zc[0]), float(zc[-1]))
+    s = backend.to_state(s0)
+    rec = backend.record(s.shape[1])
+    log, stalls, planes = [], 0, int(slab_planes)
+    while True:
+        zmin = backend.slowest(s, rec)
+        if zmin is None:
+            return s, rec, log
+        a, b = slab_planes_for(zc, zmin, planes)
+        w_lo = -np.inf if a == 0 else float(zc[a + MARGIN])
+        w_hi = np.inf if b == n - 1 else float(zc[b - MARGIN])
+        idx = backend.select(s, rec, w_lo, w_hi)
+        before = backend.summary(rec, idx, t_stop)
+        slab_axes = list(axes)
+        slab_axes[p] = np.asarray(axes[p])[a:b + 1]
+        field = backend.field(source(a, b + 1), slab_axes)
+        backend.launch(field, s, rec, idx, w_lo, w_hi, grid_range, channels)
+        backend.release(field)
+        after = backend.summary(rec, idx, t_stop)
+        done, att = after["finished"] - before["finished"], after["attempts"] - before["attempts"]
+        log.append(dict(planes=(a, b), window=(w_lo, w_hi), launched=len(idx), finished=done, parked=len(idx) - done,
+                        parked_pending=after["pending"], parked_clip=after["clip"], attempts=att))
+        # Nothing committed and nothing finished: the state is what it was, so the next window is this one or (once) the
+        # one that holds the point a ray parked at below it.  Grow the slab; at the largest, a second such launch means an
+        # attempt wider than the window.
+        if att > 0 or done > 0:
+            stalls, planes = 0, int(slab_planes)
+        elif planes < top:
+            planes = min(top, 2 * planes)
+        else:
+            stalls += 1
+            if stalls >= 2:
+                raise ValueError(f"slab of {b - a + 1} planes is too thin for the adaptive steps: no ray can take its next "
+                                 f"attempt inside the window ({w_lo:.4g} .. {w_hi:.4g} m): increase slab_planes "
+                                 "(or max_slab_planes)")
+
+
 def solve_out_of_core(s0_import, source, lengths, dims, probing_depth, *, slab_planes, probing_direction="z", lwl=1064e-9,
                       return_E=False, phaseshift=False, phase_f64=False, n_steps=None, ds=None, sort=True,
-                      axis_convention="current", diagnostics=(), return_state=False, prefetch=False):
-    """``propagator.solve(..., method='rk4')`` for a grid delivered in slabs of ``slab_planes`` planes of the probing axis
+                      axis_convention="current", diagnostics=(), return_state=False, prefetch=False, method="rk4",
+                      rtol=None, atol=None, max_steps=None, precision="fp64", early_exit=True, save_steps=2,
+                      max_slab_planes=None):
+    """``propagator.solve(..., method=...)`` for a grid delivered in slabs of ``slab_planes`` planes of the probing axis
     by ``source(k0, k1)``.  ``lengths`` / ``dims`` describe the whole grid as ``ScalarDomain`` takes them (axes
     ``linspace(-L/2, L/2, n)`` rounded to float32).  Same outputs as ``solve``: ``(rf, Jf, duration)`` (+ a dict with
-    'sf', 'steps', 'slabs', 'stats' when ``return_state``); ``diagnostics`` (``DiagnosticSpec`` list) are binned by the
-    last slab's launch, fused as in ``solve_and_image``.  ``prefetch=True`` (host sources only) reads the next slab on a
-    worker thread while the current one is traced (``PrefetchingSource``)."""
+    'sf', 'steps', 'slabs', 'stats' when ``return_state``); ``diagnostics`` (``DiagnosticSpec`` list) are binned fused as
+    in ``solve_and_image`` (RK4: by the last slab's launch; adaptive: each ray by the launch it finishes in).
+    ``prefetch=True`` (host sources only) reads the next slab on a worker thread while the current one is traced
+    (``PrefetchingSource``).
+
+    ``method='rk4'`` (default; ``n_steps`` / ``ds``) or the per-ray adaptive solves ``'rk45'`` and ``'tsit5'`` with
+    ``rtol`` / ``atol`` / ``max_steps`` / ``precision`` / ``early_exit`` / ``save_steps`` as ``propagator.solve`` takes
+    them; every result equals the in-core solve's bit for bit.  'rk45_joint' and 'rk45_bundle' are not available out of
+    core (one step size per batch / per bundle), nor are the attenuation and Faraday channels.  ``max_slab_planes`` lets
+    an adaptive solve grow a slab while no ray can take its next attempt inside it (``trace_slabs_adaptive``)."""
     import torch
     from . import propagator
+    if method in ("rk45_joint", "rk45_bundle"):
+        raise ValueError(f"method={method!r} is not available out of core: its step size is shared by a whole batch / "
+                         "bundle of rays; use 'rk45' (per ray), 'tsit5' or 'rk4'")
+    if method not in ("rk4", "rk45", "tsit5"):
+        raise ValueError(f"unknown method {method!r}")
+    if method == "rk4" and (precision != "fp64" or not early_exit):
+        raise ValueError("out-of-core RK4 runs in float64 with early exit (precision='fp64', early_exit=True)")
     engine.require_cuda()
-    if np.ndim(lengths) == 0:
-        lengths = [lengths] * 3
-    if np.ndim(dims) == 0:
-        dims = [dims] * 3
-    axes = [np.float32(np.linspace(-float(L_) / 2, float(L_) / 2, int(n))) for L_, n in zip(lengths, dims)]
+    if method in ("rk45", "tsit5"):
+        return _solve_adaptive(s0_import, source, lengths, dims, probing_depth, slab_planes=slab_planes,
+                               probing_direction=probing_direction, lwl=lwl, return_E=return_E, phaseshift=phaseshift,
+                               phase_f64=phase_f64, axis_convention=axis_convention, diagnostics=diagnostics,
+                               return_state=return_state, prefetch=prefetch, method=method, rtol=rtol, atol=atol,
+                               max_steps=max_steps, precision=precision, early_exit=early_exit, save_steps=save_steps,
+                               sort=sort, max_slab_planes=max_slab_planes)
+    lengths, dims, axes = _grid_axes(lengths, dims)
     extent = float(probing_depth)
     t_end = np.sqrt(8.0) * extent / C_LIGHT
     if ds is None and n_steps is None:
@@ -279,6 +425,53 @@ def solve_out_of_core(s0_import, source, lengths, dims, probing_depth, *, slab_p
     if return_state:
         extra = dict(sf=sf.cpu().numpy() if as_numpy else sf, steps=steps.cpu().numpy() if as_numpy else steps, slabs=log,
                      stats=engine.stats_dict(stats))
+        return rf, jf, duration, extra
+    return rf, jf, duration
+
+
+def _grid_axes(lengths, dims):
+    if np.ndim(lengths) == 0:
+        lengths = [lengths] * 3
+    if np.ndim(dims) == 0:
+        dims = [dims] * 3
+    axes = [np.float32(np.linspace(-float(L_) / 2, float(L_) / 2, int(n))) for L_, n in zip(lengths, dims)]
+    return list(lengths), list(dims), axes
+
+
+def _solve_adaptive(s0_import, source, lengths, dims, probing_depth, *, slab_planes, probing_direction, lwl, return_E,
+                    phaseshift, phase_f64, axis_convention, diagnostics, return_state, prefetch, method, rtol, atol,
+                    max_steps, precision, early_exit, save_steps, sort, max_slab_planes):
+    import torch
+    from . import propagator
+    lengths, dims, axes = _grid_axes(lengths, dims)
+    pa = engine.AXIS[probing_direction]
+    need_phase = any(d.image.kind == "interferogram" for d in diagnostics)
+    phase = bool(phaseshift) or need_phase
+    P = propagator._solver_params(probing_direction, float(lengths[pa]) / (int(dims[pa]) - 1), False, False, probing_depth,
+                                  lwl, method, None, None, rtol, atol, precision, early_exit, phase, phase_f64, sort,
+                                  axis_convention, max_steps, save_steps)
+    backend = _AdaptiveDeviceBackend(P, lwl, probing_direction, phase, phase_f64, return_E)
+    chans = [(d.ops, d.image, d.wavelength if d.wavelength else lwl) for d in diagnostics]
+    as_numpy = not isinstance(s0_import, torch.Tensor)
+    if prefetch:
+        source = PrefetchingSource(source, int(dims[pa]), pa)
+    torch.cuda.synchronize()
+    start = time()
+    try:
+        sf, rec, log = trace_slabs_adaptive(backend, s0_import, source, axes, probing_direction, slab_planes,
+                                            1.0 if method == "tsit5" else P.t_end, max_slab_planes=max_slab_planes,
+                                            channels=chans)
+    finally:
+        if prefetch:
+            source.close()
+    torch.cuda.synchronize()
+    duration = time() - start
+    rf, jf, steps = backend.rf, backend.jf, rec["steps"]
+    if as_numpy:
+        rf, jf = rf.cpu().numpy(), (None if jf is None else jf.cpu().numpy())
+    if return_state:
+        extra = dict(sf=sf.cpu().numpy() if as_numpy else sf, steps=steps.cpu().numpy() if as_numpy else steps, slabs=log,
+                     stats=engine.stats_dict(backend.stats))
         return rf, jf, duration, extra
     return rf, jf, duration
 

@@ -35,6 +35,15 @@ def _out_axes(probing_direction, convention):
 
 def _params(domain, probing_depth, lwl, method, n_steps, ds, rtol, atol, precision, early_exit, phase, phase_f64,
             sort, convention, max_steps, save_steps=2):
+    return _solver_params(domain.probing_direction, domain.cell_size(), bool(domain.inv_brems), bool(domain.B_on),
+                          probing_depth, lwl, method, n_steps, ds, rtol, atol, precision, early_exit, phase, phase_f64,
+                          sort, convention, max_steps, save_steps)
+
+
+def _solver_params(probing_direction, cell_size, atten, faraday, probing_depth, lwl, method, n_steps, ds, rtol, atol,
+                   precision, early_exit, phase, phase_f64, sort, convention, max_steps, save_steps=2):
+    """``sp_params`` of a solve from what it reads of the domain: the probing direction, the cell size along it (RK4's
+    default ``ds``) and whether the attenuation / Faraday channels are on (``out_of_core`` has no domain object)."""
     extent = float(probing_depth)
     t_end = np.sqrt(8.0) * extent / c
     h, n = 0.0, 0
@@ -47,7 +56,7 @@ def _params(domain, probing_depth, lwl, method, n_steps, ds, rtol, atol, precisi
         n = int(max_steps or 10000)                            # propagator.py:572
     elif method == "rk4":
         if ds is None and n_steps is None:
-            ds = 0.5 * domain.cell_size()
+            ds = 0.5 * cell_size
         if ds is not None:
             h = float(ds) / c
             n = int(np.ceil(t_end / h)) if n_steps is None else int(n_steps)
@@ -56,12 +65,12 @@ def _params(domain, probing_depth, lwl, method, n_steps, ds, rtol, atol, precisi
             h = t_end / n
     else:
         n = int(max_steps or 0)
-    return engine.make_params(method, probing_direction=domain.probing_direction, extent=extent,
+    return engine.make_params(method, probing_direction=probing_direction, extent=extent,
                               omega=engine.omega_of(lwl), n_steps=n, h=h, t_end=t_end, rtol=rtol, atol=atol,
                               phase=phase, phase_f64=phase_f64, early_exit=early_exit, fp32=(precision == "fp32"),
-                              sort=sort, out_axes=_out_axes(domain.probing_direction, convention),
-                              atten=bool(domain.inv_brems), faraday=bool(domain.B_on),
-                              verdet=2.62e-13 * lwl ** 2 if domain.B_on else 0.0)      # propagator.py:353-355
+                              sort=sort, out_axes=_out_axes(probing_direction, convention),
+                              atten=atten, faraday=faraday,
+                              verdet=2.62e-13 * lwl ** 2 if faraday else 0.0)      # propagator.py:353-355
 
 
 def solve(s0_import, ScalarDomain, probing_depth, *, return_E=False, parallelise=True, jitted=True, save_steps=2,
