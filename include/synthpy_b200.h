@@ -293,6 +293,19 @@ int sp_propagate_window(const sp_field* field, const sp_params* params, sp_works
                         uint32_t* steps_dev, double w_lo, double w_hi, double g_lo, double g_hi, double* rf_dev, double* jf_dev,
                         const sp_channel* channels_host, int n_channels, sp_stats* stats_dev, void* stream);
 
+/* sp_propagate_window with the attenuation and / or Faraday channels (SP_FLAG_ATTEN, SP_FLAG_FARADAY): the per-ray
+ * Dormand-Prince over all nine rows that sp_propagate runs for SP_METHOD_RK45 with a channel flag, resumable in the same way
+ * and with the same arguments, record layout and stats.  amp (row 6) and pol (row 8) of state_dev are integrated and carried
+ * from launch to launch.  The slab's field needs the grids of the flags (sp_field_attach_channels on the slab's planes).
+ * A separate entry point because sp_propagate_window refuses the channel flags.
+ * SP_EINVAL before any CUDA call: a method other than SP_METHOD_RK45 (Tsit5 included), neither channel flag, SP_FLAG_FP32
+ * or SP_FLAG_BUNDLE_STEP, and every window, grid-range, axis and null-pointer case sp_propagate_window refuses.
+ * SP_ESTATE: the field lacks the kappa grid (SP_FLAG_ATTEN) or the ne and B grids (SP_FLAG_FARADAY). */
+int sp_propagate_window_channels(const sp_field* field, const sp_params* params, sp_workspace* ws, double* state_dev, uint64_t n,
+                                 const uint32_t* idx_dev, uint64_t n_idx, double* ctl_dev, uint32_t* ctl_flags_dev,
+                                 uint32_t* steps_dev, double w_lo, double w_hi, double g_lo, double g_hi, double* rf_dev,
+                                 double* jf_dev, const sp_channel* channels_host, int n_channels, sp_stats* stats_dev, void* stream);
+
 /* Device time of the k_propagate launches issued through `ws` since the last call (CUDA events recorded
  * around each launch on its stream; this call waits for the last one).  bench.py's roofline figure. */
 int sp_workspace_propagate_ms(sp_workspace* ws, double* total_ms, int* n_launches);

@@ -84,6 +84,10 @@ EXPORTS = {
     "sp_propagate_window": (C.c_int, [C.c_void_p, C.POINTER(Params), C.c_void_p, C.c_void_p, C.c_uint64, C.c_void_p, C.c_uint64,
                                       C.c_void_p, C.c_void_p, C.c_void_p, C.c_double, C.c_double, C.c_double, C.c_double,
                                       C.c_void_p, C.c_void_p, C.POINTER(Channel), C.c_int, C.c_void_p, C.c_void_p]),
+    "sp_propagate_window_channels": (C.c_int, [C.c_void_p, C.POINTER(Params), C.c_void_p, C.c_void_p, C.c_uint64, C.c_void_p,
+                                               C.c_uint64, C.c_void_p, C.c_void_p, C.c_void_p, C.c_double, C.c_double, C.c_double,
+                                               C.c_double, C.c_void_p, C.c_void_p, C.POINTER(Channel), C.c_int, C.c_void_p,
+                                               C.c_void_p]),
     "sp_exit_plane": (C.c_int, [C.c_void_p, C.c_uint64, C.c_int, C.c_int, C.c_int, C.c_double, C.c_int, C.c_void_p, C.c_void_p,
                                 C.c_void_p, C.c_void_p]),
     "sp_scatter_to_grid": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_uint64, C.c_void_p, C.c_uint64, C.c_void_p,

@@ -1118,10 +1118,10 @@ SP_HD int deriv9(const FieldView<double>& F, const ExtView& X, CellCache<double,
     return in;
 }
 
-template <bool PHASE, bool AUX64>
+template <bool PHASE, bool AUX64, bool WIN = false>
 SP_HD int dp5_attempt9(const FieldView<double>& F, const ExtView& X, CellCache<double, PHASE>& cc, double omega, bool with_phase,
                        double h, double rtol, double atol, const double* y, const double* k1, double* yn, double* k7,
-                       double& err_sq) {
+                       double& err_sq, const Window* W = nullptr, double* out = nullptr) {
     const double A[5][5] = {{DP::a21, 0, 0, 0, 0}, {DP::a31, DP::a32, 0, 0, 0}, {DP::a41, DP::a42, DP::a43, 0, 0},
                             {DP::a51, DP::a52, DP::a53, DP::a54, 0}, {DP::a61, DP::a62, DP::a63, DP::a64, DP::a65}};
     const double Bc[6] = {DP::b1, 0.0, DP::b3, DP::b4, DP::b5, DP::b6};
@@ -1135,6 +1135,7 @@ SP_HD int dp5_attempt9(const FieldView<double>& F, const ExtView& X, CellCache<d
             for (int j = 1; j < s; ++j) acc += A[s - 1][j] * K[j][i];
             ys[i] = y[i] + acc * h;
         }
+        if (WIN && outside(*W, F, ys)) { *out = ys[2]; return touched; }
         touched += deriv9<PHASE, AUX64>(F, X, cc, omega, with_phase, ys, K[s]);
     }
     for (int i = 0; i < 9; ++i) {
@@ -1142,6 +1143,7 @@ SP_HD int dp5_attempt9(const FieldView<double>& F, const ExtView& X, CellCache<d
         for (int j = 2; j < 6; ++j) acc += Bc[j] * K[j][i];
         yn[i] = y[i] + h * acc;
     }
+    if (WIN && outside(*W, F, yn)) { *out = yn[2]; return touched; }
     touched += deriv9<PHASE, AUX64>(F, X, cc, omega, with_phase, yn, K[6]);
     double tot = 0.0;
     for (int i = 0; i < 9; ++i) {
@@ -1157,10 +1159,10 @@ SP_HD int dp5_attempt9(const FieldView<double>& F, const ExtView& X, CellCache<d
     return touched;
 }
 
-template <bool PHASE, bool AUX64>
+template <bool PHASE, bool AUX64, bool WIN = false>
 SP_HD double dp5_initial_step9(const FieldView<double>& F, const ExtView& X, CellCache<double, PHASE>& cc, double omega,
                                bool with_phase, double t_end, double rtol, double atol, const double* y, const double* f0,
-                               int& touched) {
+                               int& touched, const Window* W = nullptr, double* out = nullptr) {
     if (t_end == 0.0) return 0.0;
     double s0 = 0, s1 = 0, sc[9], y1[9], f1[9];
     for (int i = 0; i < 9; ++i) {
@@ -1172,12 +1174,92 @@ SP_HD double dp5_initial_step9(const FieldView<double>& F, const ExtView& X, Cel
     double h0 = (d0 < 1e-5 || d1 < 1e-5) ? 1e-6 : 0.01 * d0 / d1;
     h0 = fmin(h0, t_end);
     for (int i = 0; i < 9; ++i) y1[i] = y[i] + h0 * f0[i];
+    if (WIN && outside(*W, F, y1)) { *out = y1[2]; return 0.0; }
     touched += deriv9<PHASE, AUX64>(F, X, cc, omega, with_phase, y1, f1);
     double s2 = 0;
     for (int i = 0; i < 9; ++i) { const double q = (f1[i] - f0[i]) / sc[i]; s2 += q * q; }
     const double d2 = sqrt(s2 / 9.0) / h0;
     const double h1 = (d1 <= 1e-15 && d2 <= 1e-15) ? fmax(1e-6, h0 * 1e-3) : pow(0.01 / fmax(d1, d2), 0.2);
     return fmin(fmin(100 * h0, h1), t_end);
+}
+
+// The per-ray solve over all nine rows (k_propagate's SP_METHOD_RK45X loop, rk45x_integrate) restricted to a window:
+// the loop of dp5_window with the same record, parking rule and votes.  y (9 rows: p, v in the kernel frame, amp, phase,
+// pol) is read and written -- amp and pol are integrated, so they carry over from slab to slab like the position.  On
+// resume the FSAL derivative is recomputed with deriv9 at the committed state through a fresh CellCache: a fresh lookup
+// is the cached one bit for bit (tests/test_out_of_core_channels.py pins it for ext_eval), so every committed attempt
+// does the in-core arithmetic.
+template <bool PHASE, bool AUX64>
+SP_HD int dp5x_window(const FieldView<double>& F, const ExtView& X, const Window& W, double omega, bool with_phase, double t_end,
+                      double rtol, double atol, unsigned cap, bool early, unsigned lanes, double* y, WinCtl& c, unsigned& acc,
+                      unsigned& capped) {
+    int touched = 0;
+    const bool skip = (c.flags & SP_CTL_FINISHED) != 0;
+    double pw = NAN;
+    if (skip) pw = 0.0;
+    else if (outside(W, F, y)) pw = y[2];
+    double t = c.t, h_abs = c.h;
+    unsigned n_att = c.n_att;
+    bool failed = false, rejected = (c.flags & SP_CTL_PENDING) != 0, fresh = !rejected, started = (c.flags & SP_CTL_STARTED) != 0;
+    double min_step = 10.0 * (nextafter(t, (double)INFINITY) - t);
+    CellCache<double, PHASE> cc;
+    double f[9], yn[9], fn[9];
+    for (int i = 0; i < 9; ++i) f[i] = 0.0;
+    if (pw != pw) {
+        touched += deriv9<PHASE, AUX64>(F, X, cc, omega, with_phase, y, f);
+        if (!started) {
+            const double h0 = dp5_initial_step9<PHASE, AUX64, true>(F, X, cc, omega, with_phase, t_end, rtol, atol, y, f, touched, &W, &pw);
+            if (pw != pw) { h_abs = h0; started = true; }
+        }
+    }
+    for (;;) {
+        bool go = (pw != pw) && (t < t_end) && !failed;
+        const double h_top = h_abs;
+        const bool fresh_top = fresh;
+        if (go && fresh) {
+            bool out = false;
+            if (early) {
+                Ray<double> q;
+                for (int k = 0; k < 3; ++k) { q.p[k] = y[k]; q.v[k] = y[3 + k]; }
+                out = escaped(F, q);
+            }
+            if (out) go = false;
+            else {
+                min_step = 10.0 * (nextafter(t, (double)INFINITY) - t);
+                if (h_abs < min_step) h_abs = min_step;
+                rejected = false; fresh = false;
+            }
+        }
+        if (go && (n_att >= cap || h_abs < min_step)) { failed = true; capped += 1; go = false; }
+        if (!SP_WIN_VOTE(lanes, go)) break;
+        if (go) {
+            double t_new = t + h_abs;
+            if (t_new - t_end > 0.0) t_new = t_end;
+            const double h = t_new - t;
+            h_abs = fabs(h);
+            double esq;
+            touched += dp5_attempt9<PHASE, AUX64, true>(F, X, cc, omega, with_phase, h, rtol, atol, y, f, yn, fn, esq, &W, &pw);
+            if (pw == pw) { h_abs = h_top; fresh = fresh_top; }          // parked: the record as at the top of this iteration
+            else {
+                ++n_att;
+                const double en = sqrt(esq / 9.0);
+                if (!(en == en)) { failed = true; capped += 1; }
+                else if (en < 1.0) {
+                    h_abs *= dp5_factor<double>(en, true, rejected);
+                    t = t_new; acc += 1;
+                    for (int i = 0; i < 9; ++i) { y[i] = yn[i]; f[i] = fn[i]; }
+                    fresh = true;
+                } else {
+                    h_abs *= dp5_factor<double>(en, false, rejected);
+                    rejected = true;
+                }
+            }
+        }
+    }
+    if (skip) return touched;
+    c.t = t; c.h = h_abs; c.n_att = n_att; c.w_park = pw;
+    c.flags = (started ? SP_CTL_STARTED : 0u) | (fresh ? 0u : SP_CTL_PENDING) | (pw != pw ? SP_CTL_FINISHED : 0u) | (failed ? SP_CTL_FAILED : 0u);
+    return touched;
 }
 
 // ---- exit plane ------------------------------------------------------------------------------------------

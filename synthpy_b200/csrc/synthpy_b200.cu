@@ -347,6 +347,7 @@ extern "C" int sp_field_export_gradients(const sp_field* f, float* gx_dev, float
 #define SP_METHOD_RK45B 5     // internal: Dormand-Prince with one step size per 32-ray bundle (SP_FLAG_BUNDLE_STEP)
 #define SP_METHOD_RK45W 7     // internal: per-ray Dormand-Prince restricted to a window along w (sp_propagate_window)
 #define SP_METHOD_TSIT5W 8    // internal: per-ray Tsit5 restricted to a window along w (sp_propagate_window)
+#define SP_METHOD_RK45XW 9    // internal: RK45X restricted to a window along w (sp_propagate_window_channels, float64)
 #define SP_MAX_OPS 16
 #define SP_MAX_CHANNELS 4
 
@@ -453,7 +454,7 @@ struct Epilogue {
     double* sf; double* rf; double* jf; uint32_t* steps;
     int n_channels;
     ChannelDev ch[SP_MAX_CHANNELS];
-    // SP_METHOD_RK45W / SP_METHOD_TSIT5W only: the window, and the controller record (ctl: t, h, w_park rows of n_total
+    // SP_METHOD_RK45W / SP_METHOD_TSIT5W / SP_METHOD_RK45XW only: the window, and the controller record (ctl: t, h, w_park rows of n_total
     // doubles; ctl_flags: SP_CTL_* bits).  sf is then the state itself and steps the attempt count, both read and written.
     Window win; double* ctl; uint32_t* ctl_flags;
 };
@@ -838,6 +839,25 @@ __device__ __noinline__ void rk45x_integrate(const PropArgs<double>& A, Ray<doub
     r.ph = y[7]; amp = y[6]; pol = y[8];
 }
 
+// RK45X restricted to a window (one slab of an out-of-core solve with the channels): ray_core.h dp5x_window on the
+// nine rows, amp and pol read from and written back to the state rows 6 and 8.  Returns the field evaluations.
+template <bool PHASE, bool AUX64, typename T>
+__device__ __forceinline__ int rk45xw_integrate(const PropArgs<T>& A, const Window W, Ray<T>& r, WinCtl& c, bool early, unsigned lanes,
+                                                uint64_t gi, unsigned& acc, unsigned& capped, double& amp, double& pol) { return 0; }
+template <bool PHASE, bool AUX64>
+__device__ __noinline__ int rk45xw_integrate(const PropArgs<double>& A, const Window W, Ray<double>& r, WinCtl& c, bool early,
+                                             unsigned lanes, uint64_t gi, unsigned& acc, unsigned& capped, double& amp, double& pol) {
+    double y[9];
+    for (int k = 0; k < 3; ++k) { y[k] = r.p[k]; y[3 + k] = r.v[k]; }
+    y[6] = A.s0[6 * A.n_total + gi]; y[7] = r.ph; y[8] = A.s0[8 * A.n_total + gi];
+    const unsigned cap = A.n_steps > 0 ? (unsigned)A.n_steps : (1u << 30);
+    const int touched = dp5x_window<PHASE, AUX64>(A.F, A.X, W, A.omega, (A.flags & SP_FLAG_PHASE) != 0, A.t_end, A.rtol, A.atol,
+                                                  cap, early, lanes, y, c, acc, capped);
+    for (int k = 0; k < 3; ++k) { r.p[k] = y[k]; r.v[k] = y[3 + k]; }
+    r.ph = y[7]; amp = y[6]; pol = y[8];
+    return touched;
+}
+
 template <typename T, int METHOD, bool PHASE, bool AUX64>
 __global__ void __launch_bounds__(128, (METHOD == SP_METHOD_RK4 && sizeof(T) == 8) ? SP_RK4_MIN_BLOCKS : (((METHOD == SP_METHOD_RK45 || METHOD == SP_METHOD_RK45B) && sizeof(T) == 8) ? SP_RK45_MIN_BLOCKS : ((METHOD == SP_METHOD_RK4 && sizeof(T) == 4) ? SP_RK4F_MIN_BLOCKS : 1))) k_propagate(const PropArgs<T> A, const Epilogue E) {
     const int lane = threadIdx.x & 31;
@@ -924,7 +944,7 @@ __global__ void __launch_bounds__(128, (METHOD == SP_METHOD_RK4 && sizeof(T) == 
                 r.ph = y[6];
             } else if (METHOD == SP_METHOD_RK45B) {
                 // handled above (whole-warp path)
-            } else if (METHOD == SP_METHOD_RK45W || METHOD == SP_METHOD_TSIT5W) {
+            } else if (METHOD == SP_METHOD_RK45W || METHOD == SP_METHOD_TSIT5W || METHOD == SP_METHOD_RK45XW) {
                 // one slab of an out-of-core solve: resume from the record, park at the window (ray_core.h dp5_window)
                 const uint64_t N = A.n_total;
                 WinCtl c;
@@ -937,6 +957,8 @@ __global__ void __launch_bounds__(128, (METHOD == SP_METHOD_RK4 && sizeof(T) == 
                     ls.evals += dp5_window<T, PHASE, AUX64, StageSmem<T> >(A.F, E.win, A.omega, A.t_end, A.rtol, A.atol, A.n_state,
                                                                           (T)A.s0[6 * N + gi], (T)A.s0[8 * N + gi], cap, early, vmask,
                                                                           r, c, S, acc, capped);
+                } else if (METHOD == SP_METHOD_RK45XW) {
+                    ls.evals += rk45xw_integrate<PHASE, AUX64>(A, E.win, r, c, early, vmask, gi, acc, capped, amp_x, pol_x);
                 } else {
                     const unsigned cap = A.n_steps > 0 ? (unsigned)A.n_steps : 10000u;
                     ls.evals += tsit5_window<T, PHASE, AUX64>(A.F, E.win, A.omega, A.t_end, A.h, A.rtol, A.atol, A.n_state, cap, vmask,
@@ -1011,7 +1033,7 @@ __global__ void __launch_bounds__(128, (METHOD == SP_METHOD_RK4 && sizeof(T) == 
         const uint64_t N = A.n_total;
         double amp = 1.0, pol = 0.0;              // constant along the ray (zero derivative): re-read instead of kept live
         if (valid && !A.use_beam) { amp = A.s0[6 * N + gi]; pol = A.s0[8 * N + gi]; }
-        if (METHOD == SP_METHOD_RK4X || METHOD == SP_METHOD_RK45X) { amp = amp_x; pol = pol_x; }
+        if (METHOD == SP_METHOD_RK4X || METHOD == SP_METHOD_RK45X || METHOD == SP_METHOD_RK45XW) { amp = amp_x; pol = pol_x; }
         if (valid) {
             if (E.sf) {
 #pragma unroll
@@ -1038,7 +1060,7 @@ __global__ void __launch_bounds__(128, (METHOD == SP_METHOD_RK4 && sizeof(T) == 
                 E.jf[2 * (N + gi)] = ey_re; E.jf[2 * (N + gi) + 1] = ey_im;
             }
             // windowed methods: rf / jf of a parked ray are overwritten in the launch it finishes in, but it is binned only there
-            const bool done = (METHOD == SP_METHOD_RK45W || METHOD == SP_METHOD_TSIT5W) ? (valid && fin) : valid;
+            const bool done = (METHOD == SP_METHOD_RK45W || METHOD == SP_METHOD_TSIT5W || METHOD == SP_METHOD_RK45XW) ? (valid && fin) : valid;
             for (int c = 0; c < E.n_channels; ++c) {
                 const ChannelDev& ch = E.ch[c];
                 DetRay d;
@@ -1570,29 +1592,26 @@ template <typename T, int METHOD> static int occupancy_grid(int sm_count, int fl
 static int joint_solve(const sp_field* field, const sp_params* P, sp_workspace* ws, const double* s0_dev, uint64_t n,
                        const Epilogue& E, sp_stats* stats_dev, cudaStream_t st);
 
-// attenuation / Faraday variant: float64, PHASE lane always compiled in (its integration is a run-time flag)
-static int ext_grid(int sm_count, bool adaptive, bool aux64, int& grid) {
+// attenuation / Faraday variants (RK4X, RK45X, RK45XW): float64, PHASE lane always compiled in (its integration is a
+// run-time flag)
+template <int METHOD> static int ext_grid_of(int sm_count, bool aux64, int& grid) {
     int per_sm = 0;
-    if (adaptive) {
-        if (aux64) CU(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, k_propagate<double, SP_METHOD_RK45X, true, true>, 128, 0));
-        else CU(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, k_propagate<double, SP_METHOD_RK45X, true, false>, 128, 0));
-    } else {
-        if (aux64) CU(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, k_propagate<double, SP_METHOD_RK4X, true, true>, 128, 0));
-        else CU(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, k_propagate<double, SP_METHOD_RK4X, true, false>, 128, 0));
-    }
+    if (aux64) CU(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, k_propagate<double, METHOD, true, true>, 128, 0));
+    else CU(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, k_propagate<double, METHOD, true, false>, 128, 0));
     grid = sm_count * (per_sm < 1 ? 1 : per_sm);
     return SP_OK;
 }
-static int launch_ext(const PropArgs<double>& A, const Epilogue& E, bool adaptive, bool aux64, int grid, cudaStream_t st) {
-    if (adaptive) {
-        if (aux64) k_propagate<double, SP_METHOD_RK45X, true, true><<<grid, 128, 0, st>>>(A, E);
-        else k_propagate<double, SP_METHOD_RK45X, true, false><<<grid, 128, 0, st>>>(A, E);
-    } else {
-        if (aux64) k_propagate<double, SP_METHOD_RK4X, true, true><<<grid, 128, 0, st>>>(A, E);
-        else k_propagate<double, SP_METHOD_RK4X, true, false><<<grid, 128, 0, st>>>(A, E);
-    }
+template <int METHOD> static int launch_ext_of(const PropArgs<double>& A, const Epilogue& E, bool aux64, int grid, cudaStream_t st) {
+    if (aux64) k_propagate<double, METHOD, true, true><<<grid, 128, 0, st>>>(A, E);
+    else k_propagate<double, METHOD, true, false><<<grid, 128, 0, st>>>(A, E);
     LAUNCH_CHECK();
     return SP_OK;
+}
+static int ext_grid(int sm_count, bool adaptive, bool aux64, int& grid) {
+    return adaptive ? ext_grid_of<SP_METHOD_RK45X>(sm_count, aux64, grid) : ext_grid_of<SP_METHOD_RK4X>(sm_count, aux64, grid);
+}
+static int launch_ext(const PropArgs<double>& A, const Epilogue& E, bool adaptive, bool aux64, int grid, cudaStream_t st) {
+    return adaptive ? launch_ext_of<SP_METHOD_RK45X>(A, E, aux64, grid, st) : launch_ext_of<SP_METHOD_RK4X>(A, E, aux64, grid, st);
 }
 
 extern "C" int sp_propagate(const sp_field* field, const sp_params* P, sp_workspace* ws, const double* s0_dev,
@@ -1734,18 +1753,28 @@ extern "C" int sp_propagate(const sp_field* field, const sp_params* P, sp_worksp
     return SP_OK;
 }
 
-extern "C" int sp_propagate_window(const sp_field* field, const sp_params* P, sp_workspace* ws, double* state_dev, uint64_t n,
-                                   const uint32_t* idx_dev, uint64_t n_idx, double* ctl_dev, uint32_t* ctl_flags_dev,
-                                   uint32_t* steps_dev, double w_lo, double w_hi, double g_lo, double g_hi, double* rf_dev, double* jf_dev,
-                                   const sp_channel* channels_host, int n_channels, sp_stats* stats_dev, void* stream) {
+// sp_propagate_window (ext = false) and sp_propagate_window_channels (ext = true): one implementation
+static int propagate_window(bool ext, const sp_field* field, const sp_params* P, sp_workspace* ws, double* state_dev, uint64_t n,
+                            const uint32_t* idx_dev, uint64_t n_idx, double* ctl_dev, uint32_t* ctl_flags_dev, uint32_t* steps_dev,
+                            double w_lo, double w_hi, double g_lo, double g_hi, double* rf_dev, double* jf_dev,
+                            const sp_channel* channels_host, int n_channels, sp_stats* stats_dev, void* stream) {
     if (!field || !P || !ws) return fail(SP_EINVAL, "null field / params / workspace");
     if (!state_dev || !ctl_dev || !ctl_flags_dev || !steps_dev) return fail(SP_EINVAL, "null state / controller record / steps");
     if (!(w_lo <= w_hi)) return fail(SP_EINVAL, "window needs w_lo <= w_hi");
     if (!(g_lo <= g_hi)) return fail(SP_EINVAL, "grid range needs g_lo <= g_hi");
-    if (P->method != SP_METHOD_RK45 && P->method != SP_METHOD_TSIT5)
-        return fail(SP_EINVAL, "sp_propagate_window takes SP_METHOD_RK45 (per ray) or SP_METHOD_TSIT5");
-    if (P->flags & (SP_FLAG_BUNDLE_STEP | SP_FLAG_ATTEN | SP_FLAG_FARADAY))
-        return fail(SP_EINVAL, "sp_propagate_window: no bundle-step RK45 and no attenuation / Faraday channels");
+    if (!ext) {
+        if (P->method != SP_METHOD_RK45 && P->method != SP_METHOD_TSIT5)
+            return fail(SP_EINVAL, "sp_propagate_window takes SP_METHOD_RK45 (per ray) or SP_METHOD_TSIT5");
+        if (P->flags & (SP_FLAG_BUNDLE_STEP | SP_FLAG_ATTEN | SP_FLAG_FARADAY))
+            return fail(SP_EINVAL, "sp_propagate_window: no bundle-step RK45 and no attenuation / Faraday channels");
+    } else {
+        if (P->method != SP_METHOD_RK45)
+            return fail(SP_EINVAL, "sp_propagate_window_channels takes SP_METHOD_RK45 (per ray)");
+        if (!(P->flags & (SP_FLAG_ATTEN | SP_FLAG_FARADAY)))
+            return fail(SP_EINVAL, "sp_propagate_window_channels needs SP_FLAG_ATTEN and / or SP_FLAG_FARADAY (else sp_propagate_window)");
+        if (P->flags & (SP_FLAG_FP32 | SP_FLAG_BUNDLE_STEP))
+            return fail(SP_EINVAL, "sp_propagate_window_channels: float64 per-ray RK45 only (no SP_FLAG_FP32, no SP_FLAG_BUNDLE_STEP)");
+    }
     if (n_channels < 0 || n_channels > SP_MAX_CHANNELS) return fail(SP_EINVAL, "at most 4 detector channels");
     if (P->probing_axis < 0 || P->probing_axis > 2 || P->out_axis_a < 0 || P->out_axis_a > 2 || P->out_axis_b < 0 ||
         P->out_axis_b > 2)
@@ -1753,6 +1782,11 @@ extern "C" int sp_propagate_window(const sp_field* field, const sp_params* P, sp
     if (kernel_index_of(field, P->probing_axis) != 2) return fail(SP_EINVAL, "the field must march along the probing axis (the window is along it)");
     if (P->method == SP_METHOD_TSIT5 && (!(P->h > 0) || !(P->t_end > 0))) return fail(SP_EINVAL, "tsit5 needs h = dt0 > 0 (units of t_end) and t_end > 0");
     if ((P->flags & SP_FLAG_PHASE_F64) && !field->aux64) return fail(SP_ESTATE, "field was built without SP_FIELD_PHASE_F64");
+    if (ext) {
+        if ((P->flags & SP_FLAG_ATTEN) && !field->ext[0]) return fail(SP_ESTATE, "SP_FLAG_ATTEN without a kappa grid (sp_field_attach_channels)");
+        if ((P->flags & SP_FLAG_FARADAY) && !(field->ext[1] && field->ext[2] && field->ext[3] && field->ext[4]))
+            return fail(SP_ESTATE, "SP_FLAG_FARADAY without ne and B grids (sp_field_attach_channels)");
+    }
     const uint64_t m = idx_dev ? n_idx : n;
     if (m == 0) return SP_OK;
     cudaStream_t st = (cudaStream_t)stream;
@@ -1764,8 +1798,10 @@ extern "C" int sp_propagate_window(const sp_field* field, const sp_params* P, sp
         if (rc) return rc;
     }
     const bool fp32 = (P->flags & SP_FLAG_FP32) != 0, tsit = P->method == SP_METHOD_TSIT5;
+    const bool ext_aux64 = (P->flags & SP_FLAG_PHASE) && (P->flags & SP_FLAG_PHASE_F64);
     int grid = 0, rc;
-    if (tsit) rc = fp32 ? occupancy_grid<float, SP_METHOD_TSIT5W>(ws->sm_count, P->flags, grid) : occupancy_grid<double, SP_METHOD_TSIT5W>(ws->sm_count, P->flags, grid);
+    if (ext) rc = ext_grid_of<SP_METHOD_RK45XW>(ws->sm_count, ext_aux64, grid);
+    else if (tsit) rc = fp32 ? occupancy_grid<float, SP_METHOD_TSIT5W>(ws->sm_count, P->flags, grid) : occupancy_grid<double, SP_METHOD_TSIT5W>(ws->sm_count, P->flags, grid);
     else rc = fp32 ? occupancy_grid<float, SP_METHOD_RK45W>(ws->sm_count, P->flags, grid) : occupancy_grid<double, SP_METHOD_RK45W>(ws->sm_count, P->flags, grid);
     if (rc) return rc;
     const uint64_t CHUNK = 1ull << 25;
@@ -1789,7 +1825,11 @@ extern "C" int sp_propagate_window(const sp_field* field, const sp_params* P, sp
         A.extent = (T)P->extent; A.stats = stats_dev;
         rc = ws_event(ws, st);
         if (rc) return rc;
-        if (fp32) {
+        if (ext) {
+            FILL(double)
+            A.X = make_ext(field, P->verdet, P->flags);
+            rc = launch_ext_of<SP_METHOD_RK45XW>(A, E, ext_aux64, g, st);
+        } else if (fp32) {
             FILL(float)
             rc = tsit ? launch_propagate<float, SP_METHOD_TSIT5W>(A, E, g, st) : launch_propagate<float, SP_METHOD_RK45W>(A, E, g, st);
         } else {
@@ -1802,6 +1842,23 @@ extern "C" int sp_propagate_window(const sp_field* field, const sp_params* P, sp
         if (rc) return rc;
     }
     return SP_OK;
+}
+
+extern "C" int sp_propagate_window(const sp_field* field, const sp_params* P, sp_workspace* ws, double* state_dev, uint64_t n,
+                                   const uint32_t* idx_dev, uint64_t n_idx, double* ctl_dev, uint32_t* ctl_flags_dev,
+                                   uint32_t* steps_dev, double w_lo, double w_hi, double g_lo, double g_hi, double* rf_dev, double* jf_dev,
+                                   const sp_channel* channels_host, int n_channels, sp_stats* stats_dev, void* stream) {
+    return propagate_window(false, field, P, ws, state_dev, n, idx_dev, n_idx, ctl_dev, ctl_flags_dev, steps_dev, w_lo, w_hi, g_lo,
+                            g_hi, rf_dev, jf_dev, channels_host, n_channels, stats_dev, stream);
+}
+
+extern "C" int sp_propagate_window_channels(const sp_field* field, const sp_params* P, sp_workspace* ws, double* state_dev, uint64_t n,
+                                            const uint32_t* idx_dev, uint64_t n_idx, double* ctl_dev, uint32_t* ctl_flags_dev,
+                                            uint32_t* steps_dev, double w_lo, double w_hi, double g_lo, double g_hi, double* rf_dev,
+                                            double* jf_dev, const sp_channel* channels_host, int n_channels, sp_stats* stats_dev,
+                                            void* stream) {
+    return propagate_window(true, field, P, ws, state_dev, n, idx_dev, n_idx, ctl_dev, ctl_flags_dev, steps_dev, w_lo, w_hi, g_lo,
+                            g_hi, rf_dev, jf_dev, channels_host, n_channels, stats_dev, stream);
 }
 
 // Host controller of the joint solve: a line-for-line counterpart of scipy's RK45._step_impl loop, with the

@@ -374,7 +374,9 @@ def propagate_window(field, params, state, record, w_lo, w_hi, grid_range, *, id
                      stats=None):
     """One call of ``sp_propagate_window``: advance the rays ``idx`` (int32 CUDA tensor of indices, None = all) of the
     (9, N) CUDA float64 ``state`` in place, each until it finishes or parks at the window [w_lo, w_hi] of the probing
-    axis (``grid_range``: the whole grid's extent along it).  ``record`` from ``controller_record``; ``rf`` (4, N) / ``jf`` (2, N) complex128 receive the rays that finish;
+    axis (``grid_range``: the whole grid's extent along it).  With a channel flag in ``params`` (attenuation / Faraday, RK45
+    only) this is ``sp_propagate_window_channels``: amp and pol (rows 6, 8) are integrated too, and ``field`` needs the
+    grids (``attach_channels``).  ``record`` from ``controller_record``; ``rf`` (4, N) / ``jf`` (2, N) complex128 receive the rays that finish;
     ``stats`` an int64 (6,) CUDA tensor accumulated into.  No sync."""
     require_cuda()
     if not (isinstance(state, torch.Tensor) and state.is_cuda and state.dtype == torch.float64 and state.is_contiguous()
@@ -391,7 +393,8 @@ def propagate_window(field, params, state, record, w_lo, w_hi, grid_range, *, id
         structs.append(ch)
         keep.append(k)
     ch_arr = (L.Channel * max(1, len(structs)))(*structs)
-    L.check(L.lib.sp_propagate_window(field._h, C.byref(params), workspace(), _ptr(state), n, _ptr(idx),
+    fn = L.lib.sp_propagate_window_channels if params.flags & (L.FLAG_ATTEN | L.FLAG_FARADAY) else L.lib.sp_propagate_window
+    L.check(fn(field._h, C.byref(params), workspace(), _ptr(state), n, _ptr(idx),
                                       0 if idx is None else idx.numel(), _ptr(record["ctl"]), _ptr(record["flags"]),
                                       _ptr(record["steps"]), float(w_lo), float(w_hi), float(grid_range[0]),
                                       float(grid_range[1]), _ptr(rf), _ptr(jf), ch_arr,

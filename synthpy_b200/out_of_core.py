@@ -27,6 +27,13 @@ raw dump, or CUDA tensor): ``array_source`` wraps an array-like; ``field_generat
 turbulent field on the device slab by slab.  One slab is resident at a time; the next is packed after
 the rays have left the current one.  ``PrefetchingSource`` overlaps the host-side read of the next slab with the tracing;
 upload and packing are not overlapped yet.
+
+The attenuation and Faraday channels (``solve_out_of_core(..., inv_brems=True, B_on=True, B=..., Te=..., Z=...)``) stream
+with the density: ``channel_source`` composes the ne source with slab sources of B, Te and Z into one that returns a
+``ChannelSlab`` per slab -- the ne planes and the channel grids of the same planes, converted as ``ScalarDomain.device_field``
+converts the whole grids (Te clamped to Te_min, kappa from ``engine.kappa_grid`` on the host: elementwise, so a slab's
+kappa is the whole grid's kappa sliced).  The backends attach them to each slab's field; RK4 then runs sp_propagate's
+RK4X kernel and RK45 sp_propagate_window_channels, with amp and pol carried in the (9, N) state.
 """
 from time import time
 
@@ -108,6 +115,82 @@ class PrefetchingSource:
             self._job = None
 
 
+class ChannelSlab:
+    """One slab of ``channel_source``: the ne planes and the channel grids of the same planes (None where a channel is off):
+    ``kappa`` (host float64), ``ne_faraday`` (the ne planes, for the Faraday term) and ``B`` (planes x 3)."""
+    __slots__ = ("ne", "kappa", "ne_faraday", "B")
+
+    def __init__(self, ne, kappa=None, ne_faraday=None, B=None):
+        self.ne, self.kappa, self.ne_faraday, self.B = ne, kappa, ne_faraday, B
+
+    def attach(self, field):
+        if self.kappa is not None or self.B is not None:
+            field.attach_channels(kappa=self.kappa, ne=self.ne_faraday, B=self.B)
+        return field
+
+
+def _host(a):
+    return a.cpu().numpy() if hasattr(a, "cpu") else a
+
+
+def _slab_source(a, axis):
+    """``f(k0, k1)`` over a slab callable (returned as is), an array-like over the whole grid (sliced along ``axis`` as
+    ``array_source`` slices it; trailing axes kept) or a scalar (the same value for every slab)."""
+    if callable(a):
+        return a
+    if getattr(a, "ndim", 0) == 0:
+        return lambda k0, k1: a
+
+    def source(k0, k1):
+        idx = [slice(None)] * 3
+        idx[axis] = slice(k0, k1)
+        return a[tuple(idx)]
+    return source
+
+
+def _is_host_source(a):
+    """Whether ``PrefetchingSource`` may wrap the slab source of ``a``: callables (refused later if they return CUDA tensors)
+    and host arrays, not CUDA tensors or scalars."""
+    return callable(a) or (getattr(a, "ndim", 0) > 0 and not getattr(a, "is_cuda", False))
+
+
+def channel_source(source, probing_direction, omega, *, inv_brems=False, B_on=False, B=None, Te=None, Z=None, Te_min=1.0):
+    """The slab source of a solve with the attenuation (``inv_brems``) and / or Faraday (``B_on``) channels: ``f(k0, k1)``
+    returns a ``ChannelSlab`` of ``source(k0, k1)`` and the channel grids of those planes.  ``B`` ((..., 3) per point),
+    ``Te`` and ``Z`` are slab callables or array-likes over the whole grid (NumPy, memmap, CUDA tensor); ``Te`` and ``Z``
+    may be scalars.  Each slab is converted as ``ScalarDomain`` converts the whole grids: ``Te`` clamped with
+    ``np.maximum(Te_min, Te)``, kappa = ``engine.kappa_grid(ne, Te, Z, omega)`` on the host, the ne planes themselves for
+    the Faraday term.  A channel slab whose shape is not the ne slab's raises ``ValueError``."""
+    axis = engine.AXIS[probing_direction]
+    b_src = _slab_source(B, axis) if B_on else None
+    te_src = _slab_source(Te, axis) if inv_brems else None
+    z_src = _slab_source(Z, axis) if inv_brems else None
+
+    def slab(k0, k1):
+        ne = source(k0, k1)
+        shape = tuple(ne.shape)
+        kappa = b = None
+        if inv_brems:
+            te, z = te_src(k0, k1), z_src(k0, k1)
+            for name, a in (("Te", te), ("Z", z)):
+                if getattr(a, "ndim", 0) and tuple(a.shape) != shape:
+                    raise ValueError(f"{name} slab has shape {tuple(a.shape)}, the ne slab {shape}")
+            kappa = engine.kappa_grid(_host(ne), np.maximum(Te_min, _host(te)), _host(z), omega)
+        if B_on:
+            b = b_src(k0, k1)
+            if tuple(b.shape) != shape + (3,):
+                raise ValueError(f"B slab has shape {tuple(b.shape)}, expected {shape + (3,)} (the ne slab's, plus 3)")
+        return ChannelSlab(ne, kappa, ne if B_on else None, b)
+    return slab
+
+
+def _field_of(backend, slab, axes):
+    ne = slab.ne if isinstance(slab, ChannelSlab) else slab
+    field = engine.DeviceField.from_ne(ne, axes[0], axes[1], axes[2], engine.omega_of(backend.lwl), march_axis=backend.p,
+                                       phase=backend.phase, phase_f64=backend.phase_f64)
+    return slab.attach(field) if isinstance(slab, ChannelSlab) else field
+
+
 def axis_is_uniform(a32):
     """The test field_prep.h / np.gradient make on an axis: every float32 spacing equal to the first."""
     d = np.diff(np.asarray(a32, dtype=np.float32))
@@ -153,11 +236,12 @@ def plan_slab(zc, zmin, zmax, vmax, h, steps_left, slab_planes):
 class _DeviceBackend:
     """The product path: packed slab field in HBM, ``sp_propagate`` per slab."""
 
-    def __init__(self, lwl, probing_direction, phase, phase_f64, out_axes, extent, sort):
+    def __init__(self, lwl, probing_direction, phase, phase_f64, out_axes, extent, sort, atten=False, faraday=False):
         import torch
         self.torch = torch
         self.lwl, self.pd, self.phase, self.phase_f64 = lwl, probing_direction, phase, phase_f64
         self.out_axes, self.extent, self.sort = out_axes, extent, sort
+        self.atten, self.faraday = atten, faraday
         self.p = engine.AXIS[probing_direction]
 
     def to_state(self, s0):
@@ -175,13 +259,13 @@ class _DeviceBackend:
         return float(z.min()), float(z.max()), float(vz.abs().max())
 
     def field(self, ne_slab, axes):
-        return engine.DeviceField.from_ne(ne_slab, axes[0], axes[1], axes[2], engine.omega_of(self.lwl), march_axis=self.p,
-                                          phase=self.phase, phase_f64=self.phase_f64)
+        return _field_of(self, ne_slab, axes)
 
     def steps(self, field, s, m, h, last, want_jf, channels):
         P = engine.make_params("rk4", probing_direction=self.pd, extent=self.extent, omega=engine.omega_of(self.lwl), n_steps=m,
                                h=h, phase=self.phase, phase_f64=self.phase_f64, early_exit=True, sort=self.sort,
-                               out_axes=self.out_axes)
+                               out_axes=self.out_axes, atten=self.atten, faraday=self.faraday,
+                               verdet=2.62e-13 * self.lwl ** 2 if self.faraday else 0.0)      # as propagator._solver_params
         out = engine.propagate(field, P, s0=s, want_sf=True, want_rf=last, want_jf=last and want_jf, want_steps=True,
                                channels=channels if last else (), with_stats=True)
         return out["sf"], out["steps"].to(self.torch.int64), out["rf"], out["jf"], out["stats_dev"]
@@ -199,7 +283,7 @@ class _DeviceBackend:
 def trace_slabs(backend, s0, source, axes, probing_direction, n_steps, h, slab_planes, *, want_jf=False, channels=()):
     """The slab loop, independent of where the arithmetic runs (``backend``: the device, or the host build of the same ray
     code in the tests).  Returns (state, steps per ray, rf, jf, log, stats) with ``log`` one dict per slab (planes, steps taken,
-    range of the live rays before it) and ``stats`` the launch counters summed over the slabs (None on the host build)."""
+    range of the live rays before it, bytes of the slab's device field) and ``stats`` the launch counters summed over the slabs (None on the host build)."""
     p = engine.AXIS[probing_direction]
     ax64 = [np.asarray(np.float32(a), dtype=np.float64) for a in axes]
     zc = ax64[p]
@@ -222,6 +306,7 @@ def trace_slabs(backend, s0, source, axes, probing_direction, n_steps, h, slab_p
         slab_axes = list(axes)
         slab_axes[p] = np.asarray(axes[p])[a:b + 1]
         field = backend.field(source(a, b + 1), slab_axes)
+        nbytes = getattr(field, "nbytes", None)
         while True:
             s_new, st, rf, jf, stats = backend.steps(field, s, m, h, last, want_jf, channels)
             after = None if last else backend.live_range(s_new, lo, hi)
@@ -231,7 +316,7 @@ def trace_slabs(backend, s0, source, axes, probing_direction, n_steps, h, slab_p
                 raise RuntimeError("a ray crossed the slab margin in a single step: increase slab_planes")
             m = max(1, m // 2)                                # a ray got further than planned: redo with fewer steps
         backend.release(field)
-        log.append(dict(planes=(a, b), steps=m, z_live=(zmin, zmax)))
+        log.append(dict(planes=(a, b), steps=m, z_live=(zmin, zmax), field_bytes=nbytes))
         s, done = s_new, done + m
         steps_total = st if steps_total is None else steps_total + st
         if stats is not None:
@@ -284,8 +369,7 @@ class _AdaptiveDeviceBackend:
                     clip=int((parked & (c[0] + c[1] - t_stop > 0)).sum()))
 
     def field(self, ne_slab, axes):
-        return engine.DeviceField.from_ne(ne_slab, axes[0], axes[1], axes[2], engine.omega_of(self.lwl), march_axis=self.p,
-                                          phase=self.phase, phase_f64=self.phase_f64)
+        return _field_of(self, ne_slab, axes)
 
     def launch(self, field, s, rec, idx, w_lo, w_hi, grid_range, channels):
         engine.propagate_window(field, self.P, s, rec, w_lo, w_hi, grid_range, idx=idx, rf=self.rf, jf=self.jf, channels=channels,
@@ -304,7 +388,8 @@ def trace_slabs_adaptive(backend, s0, source, axes, probing_direction, slab_plan
     and launches once over the unfinished rays inside its window; a ray runs until it finishes or parks at the window, and
     resumes in a later slab from its controller record.  Returns (state, record, log): ``log`` one dict per slab with its
     planes, window, rays launched, finished, parked, parked with a pending rejection ('parked_pending'), parked right
-    before their final step, the one clipped to the end of the interval ('parked_clip'), and committed attempts.
+    before their final step, the one clipped to the end of the interval ('parked_clip'), committed attempts, and the bytes
+    of the slab's device field ('field_bytes', channel grids included).
     ``t_stop`` is where that clip happens in the record's time (t_end for RK45, 1 for Tsit5's normalised time).
 
     A launch in which no ray commits an attempt or finishes leaves the state as it was: some attempt spans more planes than
@@ -334,12 +419,13 @@ def trace_slabs_adaptive(backend, s0, source, axes, probing_direction, slab_plan
         slab_axes = list(axes)
         slab_axes[p] = np.asarray(axes[p])[a:b + 1]
         field = backend.field(source(a, b + 1), slab_axes)
+        nbytes = getattr(field, "nbytes", None)
         backend.launch(field, s, rec, idx, w_lo, w_hi, grid_range, channels)
         backend.release(field)
         after = backend.summary(rec, idx, t_stop)
         done, att = after["finished"] - before["finished"], after["attempts"] - before["attempts"]
         log.append(dict(planes=(a, b), window=(w_lo, w_hi), launched=len(idx), finished=done, parked=len(idx) - done,
-                        parked_pending=after["pending"], parked_clip=after["clip"], attempts=att))
+                        parked_pending=after["pending"], parked_clip=after["clip"], attempts=att, field_bytes=nbytes))
         # Nothing committed and nothing finished: the state is what it was, so the next window is this one or (once) the
         # one that holds the point a ray parked at below it.  Grow the slab; at the largest, a second such launch means an
         # attempt wider than the window.
@@ -359,7 +445,7 @@ def solve_out_of_core(s0_import, source, lengths, dims, probing_depth, *, slab_p
                       return_E=False, phaseshift=False, phase_f64=False, n_steps=None, ds=None, sort=True,
                       axis_convention="current", diagnostics=(), return_state=False, prefetch=False, method="rk4",
                       rtol=None, atol=None, max_steps=None, precision="fp64", early_exit=True, save_steps=2,
-                      max_slab_planes=None):
+                      max_slab_planes=None, inv_brems=False, B_on=False, B=None, Te=None, Z=None):
     """``propagator.solve(..., method=...)`` for a grid delivered in slabs of ``slab_planes`` planes of the probing axis
     by ``source(k0, k1)``.  ``lengths`` / ``dims`` describe the whole grid as ``ScalarDomain`` takes them (axes
     ``linspace(-L/2, L/2, n)`` rounded to float32).  Same outputs as ``solve``: ``(rf, Jf, duration)`` (+ a dict with
@@ -371,8 +457,16 @@ def solve_out_of_core(s0_import, source, lengths, dims, probing_depth, *, slab_p
     ``method='rk4'`` (default; ``n_steps`` / ``ds``) or the per-ray adaptive solves ``'rk45'`` and ``'tsit5'`` with
     ``rtol`` / ``atol`` / ``max_steps`` / ``precision`` / ``early_exit`` / ``save_steps`` as ``propagator.solve`` takes
     them; every result equals the in-core solve's bit for bit.  'rk45_joint' and 'rk45_bundle' are not available out of
-    core (one step size per batch / per bundle), nor are the attenuation and Faraday channels.  ``max_slab_planes`` lets
-    an adaptive solve grow a slab while no ray can take its next attempt inside it (``trace_slabs_adaptive``)."""
+    core (one step size per batch / per bundle).  ``max_slab_planes`` lets an adaptive solve grow a slab while no ray can
+    take its next attempt inside it (``trace_slabs_adaptive``).
+
+    The attenuation (``inv_brems``, with ``Te`` and ``Z``) and Faraday (``B_on``, with ``B``) channels are those of
+    ``ScalarDomain(inv_brems=..., B_on=...)`` with ``external_Te`` / ``external_Z`` / ``external_B``: each of ``B`` ((..., 3)
+    per point), ``Te`` and ``Z`` is an array-like over the whole grid (NumPy, memmap, CUDA tensor; sliced along the probing
+    axis) or a slab callable ``f(k0, k1)`` like ``source``; ``Te`` and ``Z`` may be scalars (``channel_source``).  With
+    the channels, RK4 and RK45 ('rk4', 'rk45') in float64; Tsit5 does not integrate them, in core or out of core.  RK45
+    with the channels saves memory only when ``max_slab_planes`` covers SciPy's first attempts, which span about half the
+    box (DESIGN.md section 6)."""
     import torch
     from . import propagator
     if method in ("rk45_joint", "rk45_bundle"):
@@ -382,14 +476,20 @@ def solve_out_of_core(s0_import, source, lengths, dims, probing_depth, *, slab_p
         raise ValueError(f"unknown method {method!r}")
     if method == "rk4" and (precision != "fp64" or not early_exit):
         raise ValueError("out-of-core RK4 runs in float64 with early exit (precision='fp64', early_exit=True)")
+    inv_brems, B_on = bool(inv_brems), bool(B_on)
+    if inv_brems or B_on:
+        _check_channels(dims, probing_direction, method, precision, inv_brems, B_on, B, Te, Z)
     engine.require_cuda()
+    if inv_brems or B_on:
+        source = _channels_from(source, dims, probing_direction, lwl, prefetch, inv_brems, B_on, B, Te, Z)
+        prefetch = False                          # each host source got its own PrefetchingSource
     if method in ("rk45", "tsit5"):
         return _solve_adaptive(s0_import, source, lengths, dims, probing_depth, slab_planes=slab_planes,
                                probing_direction=probing_direction, lwl=lwl, return_E=return_E, phaseshift=phaseshift,
                                phase_f64=phase_f64, axis_convention=axis_convention, diagnostics=diagnostics,
                                return_state=return_state, prefetch=prefetch, method=method, rtol=rtol, atol=atol,
                                max_steps=max_steps, precision=precision, early_exit=early_exit, save_steps=save_steps,
-                               sort=sort, max_slab_planes=max_slab_planes)
+                               sort=sort, max_slab_planes=max_slab_planes, atten=inv_brems, faraday=B_on)
     lengths, dims, axes = _grid_axes(lengths, dims)
     extent = float(probing_depth)
     t_end = np.sqrt(8.0) * extent / C_LIGHT
@@ -404,7 +504,7 @@ def solve_out_of_core(s0_import, source, lengths, dims, probing_depth, *, slab_p
     need_phase = any(d.image.kind == "interferogram" for d in diagnostics)
     phase = bool(phaseshift) or need_phase
     backend = _DeviceBackend(lwl, probing_direction, phase, phase_f64, propagator._out_axes(probing_direction, axis_convention),
-                             extent, sort)
+                             extent, sort, atten=inv_brems, faraday=B_on)
     chans = [(d.ops, d.image, d.wavelength if d.wavelength else lwl) for d in diagnostics]
     as_numpy = not isinstance(s0_import, torch.Tensor)
     if prefetch:
@@ -416,8 +516,7 @@ def solve_out_of_core(s0_import, source, lengths, dims, probing_depth, *, slab_p
         sf, steps, rf, jf, log, stats = trace_slabs(backend, s0_import, source, axes, probing_direction, n_steps, h, slab_planes,
                                                     want_jf=return_E, channels=chans)
     finally:
-        if prefetch:
-            source.close()
+        _close(source)
     torch.cuda.synchronize()
     duration = time() - start
     if as_numpy:
@@ -427,6 +526,45 @@ def solve_out_of_core(s0_import, source, lengths, dims, probing_depth, *, slab_p
                      stats=engine.stats_dict(stats))
         return rf, jf, duration, extra
     return rf, jf, duration
+
+
+def _check_channels(dims, probing_direction, method, precision, inv_brems, B_on, B, Te, Z):
+    """The refusals of a solve with channels, before anything touches the GPU."""
+    if B_on and B is None:
+        raise ValueError("B_on=True needs B (an array over the grid, (..., 3) per point, or a slab callable)")
+    if inv_brems and (Te is None or Z is None):
+        raise ValueError("inv_brems=True needs Te and Z (arrays over the grid, scalars or slab callables)")
+    if method == "tsit5":
+        raise ValueError("method='tsit5' does not integrate the attenuation / Faraday channels (in core neither): use 'rk4' "
+                         "or 'rk45'")
+    if precision != "fp64":
+        raise ValueError("the attenuation / Faraday channels are float64 only (precision='fp64')")
+    shape = tuple(int(n) for n in (dims if np.ndim(dims) else [dims] * 3))
+    for name, a, want in (("B", B if B_on else None, shape + (3,)), ("Te", Te if inv_brems else None, shape),
+                          ("Z", Z if inv_brems else None, shape)):
+        if a is not None and not callable(a) and getattr(a, "ndim", 0) and tuple(a.shape) != want:
+            raise ValueError(f"{name} has shape {tuple(a.shape)}, the grid needs {want}")
+
+
+def _channels_from(source, dims, probing_direction, lwl, prefetch, inv_brems, B_on, B, Te, Z):
+    """``channel_source`` over ``source`` and the channel inputs; with ``prefetch`` every host source (ne, B, Te, Z) is
+    wrapped in its own ``PrefetchingSource`` first."""
+    pa = engine.AXIS[probing_direction]
+    n = int(dims[pa]) if np.ndim(dims) else int(dims)
+    if prefetch:
+        source = PrefetchingSource(source, n, pa)
+        B, Te, Z = (PrefetchingSource(_slab_source(a, pa), n, pa) if (on and _is_host_source(a)) else a
+                    for a, on in ((B, B_on), (Te, inv_brems), (Z, inv_brems)))
+    slab = channel_source(source, probing_direction, engine.omega_of(lwl), inv_brems=inv_brems, B_on=B_on, B=B, Te=Te, Z=Z)
+    slab.parts = [a for a in (source, B, Te, Z) if isinstance(a, PrefetchingSource)]
+    return slab
+
+
+def _close(source):
+    """Stop the worker threads of the ``PrefetchingSource`` objects behind ``source``."""
+    for s in [source] + list(getattr(source, "parts", ())):
+        if isinstance(s, PrefetchingSource):
+            s.close()
 
 
 def _grid_axes(lengths, dims):
@@ -440,14 +578,14 @@ def _grid_axes(lengths, dims):
 
 def _solve_adaptive(s0_import, source, lengths, dims, probing_depth, *, slab_planes, probing_direction, lwl, return_E,
                     phaseshift, phase_f64, axis_convention, diagnostics, return_state, prefetch, method, rtol, atol,
-                    max_steps, precision, early_exit, save_steps, sort, max_slab_planes):
+                    max_steps, precision, early_exit, save_steps, sort, max_slab_planes, atten=False, faraday=False):
     import torch
     from . import propagator
     lengths, dims, axes = _grid_axes(lengths, dims)
     pa = engine.AXIS[probing_direction]
     need_phase = any(d.image.kind == "interferogram" for d in diagnostics)
     phase = bool(phaseshift) or need_phase
-    P = propagator._solver_params(probing_direction, float(lengths[pa]) / (int(dims[pa]) - 1), False, False, probing_depth,
+    P = propagator._solver_params(probing_direction, float(lengths[pa]) / (int(dims[pa]) - 1), atten, faraday, probing_depth,
                                   lwl, method, None, None, rtol, atol, precision, early_exit, phase, phase_f64, sort,
                                   axis_convention, max_steps, save_steps)
     backend = _AdaptiveDeviceBackend(P, lwl, probing_direction, phase, phase_f64, return_E)
@@ -462,8 +600,7 @@ def _solve_adaptive(s0_import, source, lengths, dims, probing_depth, *, slab_pla
                                             1.0 if method == "tsit5" else P.t_end, max_slab_planes=max_slab_planes,
                                             channels=chans)
     finally:
-        if prefetch:
-            source.close()
+        _close(source)
     torch.cuda.synchronize()
     duration = time() - start
     rf, jf, steps = backend.rf, backend.jf, rec["steps"]
