@@ -306,6 +306,34 @@ int sp_propagate_window_channels(const sp_field* field, const sp_params* params,
                                  uint32_t* steps_dev, double w_lo, double w_hi, double g_lo, double g_hi, double* rf_dev,
                                  double* jf_dev, const sp_channel* channels_host, int n_channels, sp_stats* stats_dev, void* stream);
 
+/* sp_propagate_window / sp_propagate_window_channels (chosen by the channel flags) PARKING BETWEEN STAGE EVALUATIONS: a ray
+ * parks right before the first point of its attempt (or of RK45's initial-step probe) that lies outside the window, and
+ * keeps K1 (the FSAL derivative at its committed state; for the probe f0) and the stage values evaluated so far in
+ * stage_dev.  It resumes, in a launch whose window holds that point, with that evaluation: nothing is evaluated at its own
+ * position, so a ray is served by any window that holds its NEXT point, and no window ever needs to hold a whole attempt.
+ * Every evaluation runs exactly once: rhs_evals equals sp_propagate's.  Same arguments, record and stats as the other two,
+ * plus:
+ *   ctl_flags_dev: SP_CTL_STAGED when the stage store holds the ray's attempt in progress, and in bits SP_CTL_ROW_SHIFT..
+ *           (4 bits) the row of the stage matrix its next evaluation fills (1 .. 6; 0 = RK45's initial-step probe);
+ *           ctl_dev row 2 (w of the point that parked the ray) is that point's w.
+ *   stage_dev  the stage store, zeroed before the first launch: SP_STAGE_RK45 / SP_STAGE_TSIT5 / SP_STAGE_RK45X values per
+ *           ray (method, channel flags), value j of ray i at [j * n + i], float64 -- float32 (and 4 bytes per value) with
+ *           SP_FLAG_FP32.  RK45: K1's velocity rows and phase row (4), then K2..K6's velocity rows (15) and the phase stage
+ *           values n3..n6 (4): 184 B per ray.  Tsit5: stage matrix rows K1..K6 of 7 (336 B).  RK45 with the channels: rows
+ *           K1..K6 of 9 (432 B).
+ * SP_EINVAL before any CUDA call: a null stage_dev, and everything sp_propagate_window (no channel flag) or
+ * sp_propagate_window_channels (a channel flag) refuses.  SP_ESTATE as they return it. */
+#define SP_CTL_STAGED 16u
+#define SP_CTL_ROW_SHIFT 8
+#define SP_STAGE_RK45 23
+#define SP_STAGE_TSIT5 42
+#define SP_STAGE_RK45X 54
+int sp_propagate_window_staged(const sp_field* field, const sp_params* params, sp_workspace* ws, double* state_dev, uint64_t n,
+                               const uint32_t* idx_dev, uint64_t n_idx, double* ctl_dev, uint32_t* ctl_flags_dev,
+                               uint32_t* steps_dev, double* stage_dev, double w_lo, double w_hi, double g_lo, double g_hi,
+                               double* rf_dev, double* jf_dev, const sp_channel* channels_host, int n_channels, sp_stats* stats_dev,
+                               void* stream);
+
 /* Device time of the k_propagate launches issued through `ws` since the last call (CUDA events recorded
  * around each launch on its stream; this call waits for the last one).  bench.py's roofline figure. */
 int sp_workspace_propagate_ms(sp_workspace* ws, double* total_ms, int* n_launches);

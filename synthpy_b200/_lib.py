@@ -19,6 +19,8 @@ STOKES_FRAC_BITS = 32         # SP_STOKES_FRAC_BITS: Stokes I, Q, U planes are i
 METHOD_RK4, METHOD_RK45, METHOD_RK45_JOINT, METHOD_TSIT5 = 0, 1, 2, 6
 FLAG_PHASE, FLAG_EARLY_EXIT, FLAG_FP32, FLAG_PHASE_F64, FLAG_NO_SORT, FLAG_ATTEN, FLAG_FARADAY, FLAG_BUNDLE_STEP = 1, 2, 4, 8, 16, 32, 64, 128
 CTL_STARTED, CTL_PENDING, CTL_FINISHED, CTL_FAILED = 1, 2, 4, 8     # SP_CTL_*: controller record of sp_propagate_window
+CTL_STAGED, CTL_ROW_SHIFT = 16, 8     # SP_CTL_STAGED, SP_CTL_ROW_SHIFT: a ray of sp_propagate_window_staged parked mid-attempt
+STAGE_RK45, STAGE_TSIT5, STAGE_RK45X = 23, 42, 54     # SP_STAGE_*: stage-store values per ray
 
 
 class Beam(C.Structure):
@@ -88,6 +90,10 @@ EXPORTS = {
                                                C.c_uint64, C.c_void_p, C.c_void_p, C.c_void_p, C.c_double, C.c_double, C.c_double,
                                                C.c_double, C.c_void_p, C.c_void_p, C.POINTER(Channel), C.c_int, C.c_void_p,
                                                C.c_void_p]),
+    "sp_propagate_window_staged": (C.c_int, [C.c_void_p, C.POINTER(Params), C.c_void_p, C.c_void_p, C.c_uint64, C.c_void_p,
+                                             C.c_uint64, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_double, C.c_double,
+                                             C.c_double, C.c_double, C.c_void_p, C.c_void_p, C.POINTER(Channel), C.c_int,
+                                             C.c_void_p, C.c_void_p]),
     "sp_exit_plane": (C.c_int, [C.c_void_p, C.c_uint64, C.c_int, C.c_int, C.c_int, C.c_double, C.c_int, C.c_void_p, C.c_void_p,
                                 C.c_void_p, C.c_void_p]),
     "sp_scatter_to_grid": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_uint64, C.c_void_p, C.c_uint64, C.c_void_p,

@@ -724,9 +724,12 @@ template <typename T> SP_HD bool outside(const Window& W, const FieldView<T>& F,
     return !(p[0] < F.ax[0].lo || p[0] > F.ax[0].hi || p[1] < F.ax[1].lo || p[1] > F.ax[1].hi);
 }
 
-template <typename T, bool PHASE, bool AUX64, typename Store, bool WIN = false>
+// STAGED (stage parking): the attempt starts at stage `s_first` (2 .. 7) with the stage values of the stages before it
+// already in S, and a park reports its stage in *s_park; the stage points are the same instructions on both paths.
+template <typename T, bool PHASE, bool AUX64, typename Store, bool WIN = false, bool STAGED = false>
 SP_HD int dp5_attempt(const FieldView<T>& F, T omega, T h, T rtol, T atol, const Ray<T>& r, const Deriv<T>& k1,
-                      Ray<T>& rn, Deriv<T>& k7, T& err_sq, Store& S, const Window* W = nullptr, double* out = nullptr) {
+                      Ray<T>& rn, Deriv<T>& k7, T& err_sq, Store& S, const Window* W = nullptr, double* out = nullptr,
+                      int s_first = 2, int* s_park = nullptr) {
     T n7 = (T)0;
     const T* K1 = k1.dv;
     const T h2 = h * h;
@@ -739,7 +742,7 @@ SP_HD int dp5_attempt(const FieldView<T>& F, T omega, T h, T rtol, T atol, const
 #if defined(__CUDA_ARCH__)
 #pragma unroll 1
 #endif
-    for (int s = 2; s <= 7; ++s) {
+    for (int s = STAGED ? s_first : 2; s <= 7; ++s) {
         T p[3] = {0, 0, 0};
         switch (s) {
         case 2:
@@ -776,7 +779,11 @@ SP_HD int dp5_attempt(const FieldView<T>& F, T omega, T h, T rtol, T atol, const
                 rn.ph = r.ph + h * ((T)DP::b1 * k1.dph + omega * ((T)DP::b3 * S.N(0) + (T)DP::b4 * S.N(1) + (T)DP::b5 * S.N(2) + (T)DP::b6 * S.N(3)));
             break;
         }
-        if (WIN && outside(*W, F, p)) { *out = (double)p[2]; return touched; }
+        if (WIN && outside(*W, F, p)) {
+            *out = (double)p[2];
+            if constexpr (STAGED) *s_park = s;
+            return touched;
+        }
         T a0, a1, a2, nn;
         touched += rhs_direct<T, PHASE, AUX64>(F, p[0], p[1], p[2], a0, a1, a2, nn);
         switch (s) {
@@ -907,9 +914,11 @@ SP_HD int tsit5_f(const FieldView<T>& F, T omega, const T* y, T* f) {
     return t;
 }
 
-template <typename T, bool PHASE, bool AUX64, bool WIN = false>
+// STAGED: the stage matrix is the caller's Ks ([7][7], rows 1 .. s_first - 1 filled), the attempt starts with the evaluation
+// that fills row s_first (1 .. 6; 6 = the one at yn), and a park reports the row it was about to fill in *s_park.
+template <typename T, bool PHASE, bool AUX64, bool WIN = false, bool STAGED = false>
 SP_HD int tsit5_attempt(const FieldView<T>& F, T omega, T h, T rtol, T atol, const T* y, const T* k1, T* yn, T* k7, T& err_sq,
-                        const Window* W = nullptr, double* out = nullptr) {
+                        const Window* W = nullptr, double* out = nullptr, int s_first = 1, int* s_park = nullptr, T* Ks = nullptr) {
     const double A[5][5] = {{0.161, 0, 0, 0, 0},
                             {-0.008480655492356989, 0.335480655492357, 0, 0, 0},
                             {2.8971530571054935, -6.359448489975075, 4.3622954328695815, 0, 0},
@@ -918,16 +927,22 @@ SP_HD int tsit5_attempt(const FieldView<T>& F, T omega, T h, T rtol, T atol, con
     const double B[6] = {0.09646076681806523, 0.01, 0.4798896504144996, 1.379008574103742, -3.290069515436081, 2.324710524099774};
     const double Bt[7] = {-0.00178001105222577714, -0.0008164344596567469, 0.007880878010261995, -0.1447110071732629,
                           0.5823571654525552, -0.45808210592918697, 0.015151515151515152};
-    T K[7][7], ys[7];
+    T Kl[STAGED ? 1 : 7][7], ys[7];
+    T (*K)[7] = STAGED ? reinterpret_cast<T (*)[7]>(Ks) : Kl;
     int touched = 0;
     for (int i = 0; i < 7; ++i) K[0][i] = k1[i];
     for (int s = 1; s < 6; ++s) {
+        if (STAGED && s < s_first) continue;           // the same loop as in core, so the compiler contracts it alike
         for (int i = 0; i < 7; ++i) {
             T acc = (T)A[s - 1][0] * K[0][i];
             for (int j = 1; j < s; ++j) acc += (T)A[s - 1][j] * K[j][i];
             ys[i] = y[i] + acc * h;
         }
-        if (WIN && outside(*W, F, ys)) { *out = (double)ys[2]; return touched; }
+        if (WIN && outside(*W, F, ys)) {
+            *out = (double)ys[2];
+            if constexpr (STAGED) *s_park = s;
+            return touched;
+        }
         touched += tsit5_f<T, PHASE, AUX64>(F, omega, ys, K[s]);
     }
     for (int i = 0; i < 7; ++i) {
@@ -935,7 +950,11 @@ SP_HD int tsit5_attempt(const FieldView<T>& F, T omega, T h, T rtol, T atol, con
         for (int j = 1; j < 6; ++j) acc += (T)B[j] * K[j][i];
         yn[i] = y[i] + h * acc;
     }
-    if (WIN && outside(*W, F, yn)) { *out = (double)yn[2]; return touched; }
+    if (WIN && outside(*W, F, yn)) {
+        *out = (double)yn[2];
+        if constexpr (STAGED) *s_park = 6;
+        return touched;
+    }
     touched += tsit5_f<T, PHASE, AUX64>(F, omega, yn, K[6]);
     T tot = (T)0;
     for (int i = 0; i < 7; ++i) {
@@ -978,20 +997,67 @@ struct WinCtl {
     unsigned n_att, flags;
 };
 
+// ---- stage parking (sp_propagate_window_staged, out_of_core park='stage') ----------------------------------------------
+// The loops above park a ray a whole attempt at a time, so a window must hold the ray's position and every stage point of
+// its next attempt.  With STAGED they park between stage evaluations instead: a ray parks right before the first point of
+// its attempt (or of RK45's initial-step probe) that lies outside the window, and the per-ray STAGE STORE in HBM keeps
+//   * K1, the FSAL derivative at the committed state (for the probe: f0),
+//   * the stage values evaluated so far in this attempt,
+// while the record flags get SP_CTL_STAGED and, in bits SP_CTL_ROW_SHIFT.., the row of the stage matrix the next evaluation
+// fills (1 .. 6; 0 = RK45's initial-step probe).  The record's t / h / PENDING are as at the top of the loop iteration, as
+// for an attempt park, so the resumed attempt recomputes its h with the same instructions.  On resume nothing is evaluated
+// at the ray's own position: the next evaluation is the stage point, in whichever slab holds it.  Every stage derivative is
+// a pure function of its point (rhs_direct has no cache; deriv9's fresh cell lookup is the cached one), so the committed
+// arithmetic and the evaluation count are the in-core ones.  Store layout: value j of ray i at stg[j * stride + i]
+// (stride = the rays of the state), in the solve's precision (float32 for float32 instantiations):
+//   RK45  (SP_STAGE_RK45,  23 values, 184 B per ray in float64): K1 dv[3], K1 dph, StageSmem's 19 values (K2..K6 dv, n3..n6)
+//   Tsit5 (SP_STAGE_TSIT5, 42 values, 336 B): the stage matrix rows K[0..5][7]
+//   RK45X (SP_STAGE_RK45X, 54 values, 432 B): the stage matrix rows K[0..5][9]
+#define SP_CTL_STAGED 16u
+#define SP_CTL_ROW_SHIFT 8
+#define SP_STAGE_RK45 23
+#define SP_STAGE_TSIT5 42
+#define SP_STAGE_RK45X 54
+template <typename T> struct StageStore {
+    T* p; unsigned long long stride;
+    SP_HD T get(int j) const { return p[(unsigned long long)j * stride]; }
+    SP_HD void set(int j, T v) const { p[(unsigned long long)j * stride] = v; }
+};
+SP_HD int staged_row(unsigned flags) { return (int)((flags >> SP_CTL_ROW_SHIFT) & 15u); }
+
+// escaped() for stage parking.  A resumed ray's position may lie outside the slab (only its next point has to be inside the
+// window), so along w the test takes the whole grid's bounds, not the slab's: the slab's own where the window reaches a
+// grid edge (w_lo / w_hi infinite: the slab starts / ends with the grid), [g_lo, g_hi] elsewhere.  Both are the grid's
+// float32-rounded end planes, so the decision is the in-core one.
+template <typename T> SP_HD bool escaped_grid(const FieldView<T>& F, const Window& W, const Ray<T>& r) {
+    const double lo = W.lo == -(double)INFINITY ? (double)F.ax[2].lo : W.g_lo;
+    const double hi = W.hi == (double)INFINITY ? (double)F.ax[2].hi : W.g_hi;
+    const double w = (double)r.p[2];
+    bool e = (w > hi && r.v[2] >= (T)0) || (w < lo && r.v[2] <= (T)0);
+#pragma unroll
+    for (int k = 0; k < 2; ++k)
+        e = e || (r.p[k] > F.ax[k].hi && r.v[k] >= (T)0) || (r.p[k] < F.ax[k].lo && r.v[k] <= (T)0);
+    return e;
+}
+
 #if defined(__CUDA_ARCH__)
 #define SP_WIN_VOTE(lanes, go) __any_sync(lanes, go)
 #else
 #define SP_WIN_VOTE(lanes, go) (go)
 #endif
 
-template <typename T, bool PHASE, bool AUX64, typename Store>
+template <typename T, bool PHASE, bool AUX64, typename Store, bool STAGED = false>
 SP_HD int dp5_window(const FieldView<T>& F, const Window& W, T omega, T t_end, T rtol, T atol, int n_state, T amp, T pol,
-                     unsigned cap, bool early, unsigned lanes, Ray<T>& r, WinCtl& c, Store& S, unsigned& acc, unsigned& capped) {
+                     unsigned cap, bool early, unsigned lanes, Ray<T>& r, WinCtl& c, Store& S, unsigned& acc, unsigned& capped,
+                     StageStore<T> G = StageStore<T>()) {
     int touched = 0;
     const bool skip = (c.flags & SP_CTL_FINISHED) != 0;   // finished in an earlier launch: takes part in the votes only
+    const bool held = STAGED && !skip && (c.flags & SP_CTL_STAGED) != 0;   // K1 and the first stages are in the stage store
+    const int row = held ? staged_row(c.flags) : 0;
+    int s_first = row >= 1 ? row + 1 : 2, s_park = 0, park_row = -1;
     double pw = NAN;                                       // set (not NaN) once the ray parks
     if (skip) pw = 0.0;
-    else if (outside(W, F, r.p)) pw = (double)r.p[2];   // before the escape test: the slab's w bounds are not the grid's
+    else if (!held && outside(W, F, r.p)) pw = (double)r.p[2];   // before the escape test: the slab's w bounds are not the grid's
     T t = (T)c.t, h_abs = (T)c.h;
     unsigned n_att = c.n_att;
     bool failed = false, rejected = (c.flags & SP_CTL_PENDING) != 0, fresh = !rejected, started = (c.flags & SP_CTL_STARTED) != 0;
@@ -1000,10 +1066,24 @@ SP_HD int dp5_window(const FieldView<T>& F, const Window& W, T omega, T t_end, T
     Deriv<T> f;
     f.dp[0] = f.dp[1] = f.dp[2] = f.dv[0] = f.dv[1] = f.dv[2] = f.dph = (T)0;
     if (pw != pw) {
-        touched += deriv_direct<T, PHASE, AUX64>(F, omega, r.p, r.v, f);
+        if constexpr (STAGED) {
+            if (held) {
+#pragma unroll
+                for (int k = 0; k < 3; ++k) { f.dp[k] = r.v[k]; f.dv[k] = G.get(k); }
+                f.dph = G.get(3);
+                for (int j = 0; j < row - 1; ++j)              // K2 .. K(row): S.K(j) is stage j + 2, S.N(j) stage j + 3
+                    for (int k = 0; k < 3; ++k) S.setK(j, k, G.get(4 + 3 * j + k));
+                for (int j = 0; j < row - 2; ++j) S.setN(j, G.get(19 + j));
+            } else {
+                touched += deriv_direct<T, PHASE, AUX64>(F, omega, r.p, r.v, f);
+            }
+        } else {
+            touched += deriv_direct<T, PHASE, AUX64>(F, omega, r.p, r.v, f);
+        }
         if (!started) {
             const T h0 = dp5_initial_step<T, PHASE, AUX64, true>(F, omega, t_end, rtol, atol, n_state, amp, pol, r, f, touched, &W, &pw);
             if (pw != pw) { h_abs = h0; started = true; }
+            if constexpr (STAGED) if (pw == pw) park_row = 0;
         }
     }
     for (;;) {
@@ -1011,7 +1091,7 @@ SP_HD int dp5_window(const FieldView<T>& F, const Window& W, T omega, T t_end, T
         const T h_top = h_abs;
         const bool fresh_top = fresh;
         if (go && fresh) {
-            if (early && escaped(F, r)) go = false;
+            if (early && (STAGED ? escaped_grid(F, W, r) : escaped(F, r))) go = false;
             else {
                 min_step = (T)10 * (nextafter(t, (T)INFINITY) - t);
                 if (h_abs < min_step) h_abs = min_step;
@@ -1026,7 +1106,14 @@ SP_HD int dp5_window(const FieldView<T>& F, const Window& W, T omega, T t_end, T
             const T h = t_new - t;
             h_abs = fabs(h);
             Ray<T> rn; Deriv<T> fn; T esq;
-            touched += dp5_attempt<T, PHASE, AUX64, Store, true>(F, omega, h, rtol, atol, r, f, rn, fn, esq, S, &W, &pw);
+            if constexpr (STAGED) {
+                touched += dp5_attempt<T, PHASE, AUX64, Store, true, true>(F, omega, h, rtol, atol, r, f, rn, fn, esq, S, &W, &pw,
+                                                                           s_first, &s_park);
+                s_first = 2;
+                if (pw == pw) park_row = s_park - 1;
+            } else {
+                touched += dp5_attempt<T, PHASE, AUX64, Store, true>(F, omega, h, rtol, atol, r, f, rn, fn, esq, S, &W, &pw);
+            }
             if (pw == pw) { h_abs = h_top; fresh = fresh_top; }          // parked: the record as at the top of this iteration
             else {
                 ++n_att;
@@ -1044,25 +1131,49 @@ SP_HD int dp5_window(const FieldView<T>& F, const Window& W, T omega, T t_end, T
     if (skip) return touched;
     c.t = (double)t; c.h = (double)h_abs; c.n_att = n_att; c.w_park = pw;
     c.flags = (started ? SP_CTL_STARTED : 0u) | (fresh ? 0u : SP_CTL_PENDING) | (pw != pw ? SP_CTL_FINISHED : 0u) | (failed ? SP_CTL_FAILED : 0u);
+    if constexpr (STAGED) if (pw == pw && park_row >= 0) {
+        c.flags |= SP_CTL_STAGED | ((unsigned)park_row << SP_CTL_ROW_SHIFT);
+#pragma unroll
+        for (int k = 0; k < 3; ++k) G.set(k, f.dv[k]);
+        G.set(3, f.dph);
+        for (int j = 0; j < park_row - 1; ++j)
+            for (int k = 0; k < 3; ++k) G.set(4 + 3 * j + k, S.K(j, k));
+        for (int j = 0; j < park_row - 2; ++j) G.set(19 + j, S.N(j));
+    }
     return touched;
 }
 
 // Tsit5 + PID per ray (k_propagate's SP_METHOD_TSIT5 branch), resumable in the same way; dt0 is taken when !STARTED.
-template <typename T, bool PHASE, bool AUX64>
+template <typename T, bool PHASE, bool AUX64, bool STAGED = false>
 SP_HD int tsit5_window(const FieldView<T>& F, const Window& W, T omega, T t_end, T dt0, T rtol, T atol, int n_state,
-                       unsigned cap, unsigned lanes, Ray<T>& r, WinCtl& c, unsigned& acc, unsigned& capped) {
+                       unsigned cap, unsigned lanes, Ray<T>& r, WinCtl& c, unsigned& acc, unsigned& capped,
+                       StageStore<T> G = StageStore<T>()) {
     int touched = 0;
     const bool skip = (c.flags & SP_CTL_FINISHED) != 0;
+    const bool held = STAGED && !skip && (c.flags & SP_CTL_STAGED) != 0;
+    const int row = held ? staged_row(c.flags) : 0;
+    int s_first = row >= 1 ? row : 1, s_park = 0, park_row = -1;
     double pw = NAN;
     if (skip) pw = 0.0;
-    else if (outside(W, F, r.p)) pw = (double)r.p[2];
+    else if (!held && outside(W, F, r.p)) pw = (double)r.p[2];
     T y[7], f[7], yn[7], fn[7];
+    T K[STAGED ? 7 : 1][7];                                // STAGED: the attempt's stage matrix, saved at a park
 #pragma unroll
     for (int k = 0; k < 3; ++k) { y[k] = r.p[k]; y[3 + k] = r.v[k]; }
     y[6] = r.ph;
 #pragma unroll
     for (int k = 0; k < 7; ++k) f[k] = (T)0;
-    if (pw != pw) touched += tsit5_f<T, PHASE, AUX64>(F, omega, y, f);
+    if constexpr (STAGED) {
+        if (held) {
+            for (int j = 0; j < row; ++j)
+                for (int i = 0; i < 7; ++i) K[j][i] = G.get(7 * j + i);
+            for (int i = 0; i < 7; ++i) f[i] = K[0][i];
+        } else if (pw != pw) {
+            touched += tsit5_f<T, PHASE, AUX64>(F, omega, y, f);
+        }
+    } else {
+        if (pw != pw) touched += tsit5_f<T, PHASE, AUX64>(F, omega, y, f);
+    }
     T tau = (T)c.t, dt = (c.flags & SP_CTL_STARTED) ? (T)c.h : dt0;
     unsigned n_att = c.n_att;
     const T inv_n = (T)1 / (T)n_state;
@@ -1075,7 +1186,14 @@ SP_HD int tsit5_window(const FieldView<T>& F, const Window& W, T omega, T t_end,
             const bool last = tau + dt >= (T)1;
             const T d = last ? (T)1 - tau : dt;
             T esq;
-            touched += tsit5_attempt<T, PHASE, AUX64, true>(F, omega, d * t_end, rtol, atol, y, f, yn, fn, esq, &W, &pw);
+            if constexpr (STAGED) {
+                touched += tsit5_attempt<T, PHASE, AUX64, true, true>(F, omega, d * t_end, rtol, atol, y, f, yn, fn, esq, &W, &pw,
+                                                                      s_first, &s_park, &K[0][0]);
+                s_first = 1;
+                if (pw == pw) park_row = s_park;
+            } else {
+                touched += tsit5_attempt<T, PHASE, AUX64, true>(F, omega, d * t_end, rtol, atol, y, f, yn, fn, esq, &W, &pw);
+            }
             if (pw != pw) {
                 ++n_att;
                 const T en = sqrt(esq * inv_n);
@@ -1098,6 +1216,11 @@ SP_HD int tsit5_window(const FieldView<T>& F, const Window& W, T omega, T t_end,
     r.ph = y[6];
     c.t = (double)tau; c.h = (double)dt; c.n_att = n_att; c.w_park = pw;
     c.flags = SP_CTL_STARTED | (pw != pw ? SP_CTL_FINISHED : 0u) | (failed ? SP_CTL_FAILED : 0u);
+    if constexpr (STAGED) if (pw == pw && park_row >= 1) {
+        c.flags |= SP_CTL_STAGED | ((unsigned)park_row << SP_CTL_ROW_SHIFT);
+        for (int j = 0; j < park_row; ++j)
+            for (int i = 0; i < 7; ++i) G.set(7 * j + i, K[j][i]);
+    }
     return touched;
 }
 
@@ -1118,24 +1241,32 @@ SP_HD int deriv9(const FieldView<double>& F, const ExtView& X, CellCache<double,
     return in;
 }
 
-template <bool PHASE, bool AUX64, bool WIN = false>
+// STAGED: as tsit5_attempt, with the caller's [7][9] stage matrix Ks.
+template <bool PHASE, bool AUX64, bool WIN = false, bool STAGED = false>
 SP_HD int dp5_attempt9(const FieldView<double>& F, const ExtView& X, CellCache<double, PHASE>& cc, double omega, bool with_phase,
                        double h, double rtol, double atol, const double* y, const double* k1, double* yn, double* k7,
-                       double& err_sq, const Window* W = nullptr, double* out = nullptr) {
+                       double& err_sq, const Window* W = nullptr, double* out = nullptr, int s_first = 1, int* s_park = nullptr,
+                       double* Ks = nullptr) {
     const double A[5][5] = {{DP::a21, 0, 0, 0, 0}, {DP::a31, DP::a32, 0, 0, 0}, {DP::a41, DP::a42, DP::a43, 0, 0},
                             {DP::a51, DP::a52, DP::a53, DP::a54, 0}, {DP::a61, DP::a62, DP::a63, DP::a64, DP::a65}};
     const double Bc[6] = {DP::b1, 0.0, DP::b3, DP::b4, DP::b5, DP::b6};
     const double Ec[7] = {DP::e1, 0.0, DP::e3, DP::e4, DP::e5, DP::e6, DP::e7};
-    double K[7][9], ys[9];
+    double Kl[STAGED ? 1 : 7][9], ys[9];
+    double (*K)[9] = STAGED ? reinterpret_cast<double (*)[9]>(Ks) : Kl;
     int touched = 0;
     for (int i = 0; i < 9; ++i) K[0][i] = k1[i];
     for (int s = 1; s < 6; ++s) {
+        if (STAGED && s < s_first) continue;           // the same loop as in core, so the compiler contracts it alike
         for (int i = 0; i < 9; ++i) {
             double acc = A[s - 1][0] * K[0][i];
             for (int j = 1; j < s; ++j) acc += A[s - 1][j] * K[j][i];
             ys[i] = y[i] + acc * h;
         }
-        if (WIN && outside(*W, F, ys)) { *out = ys[2]; return touched; }
+        if (WIN && outside(*W, F, ys)) {
+            *out = ys[2];
+            if constexpr (STAGED) *s_park = s;
+            return touched;
+        }
         touched += deriv9<PHASE, AUX64>(F, X, cc, omega, with_phase, ys, K[s]);
     }
     for (int i = 0; i < 9; ++i) {
@@ -1143,7 +1274,11 @@ SP_HD int dp5_attempt9(const FieldView<double>& F, const ExtView& X, CellCache<d
         for (int j = 2; j < 6; ++j) acc += Bc[j] * K[j][i];
         yn[i] = y[i] + h * acc;
     }
-    if (WIN && outside(*W, F, yn)) { *out = yn[2]; return touched; }
+    if (WIN && outside(*W, F, yn)) {
+        *out = yn[2];
+        if constexpr (STAGED) *s_park = 6;
+        return touched;
+    }
     touched += deriv9<PHASE, AUX64>(F, X, cc, omega, with_phase, yn, K[6]);
     double tot = 0.0;
     for (int i = 0; i < 9; ++i) {
@@ -1189,15 +1324,19 @@ SP_HD double dp5_initial_step9(const FieldView<double>& F, const ExtView& X, Cel
 // resume the FSAL derivative is recomputed with deriv9 at the committed state through a fresh CellCache: a fresh lookup
 // is the cached one bit for bit (tests/test_out_of_core_channels.py pins it for ext_eval), so every committed attempt
 // does the in-core arithmetic.
-template <bool PHASE, bool AUX64>
+template <bool PHASE, bool AUX64, bool STAGED = false>
 SP_HD int dp5x_window(const FieldView<double>& F, const ExtView& X, const Window& W, double omega, bool with_phase, double t_end,
                       double rtol, double atol, unsigned cap, bool early, unsigned lanes, double* y, WinCtl& c, unsigned& acc,
-                      unsigned& capped) {
+                      unsigned& capped, StageStore<double> G = StageStore<double>()) {
     int touched = 0;
     const bool skip = (c.flags & SP_CTL_FINISHED) != 0;
+    const bool held = STAGED && !skip && (c.flags & SP_CTL_STAGED) != 0;
+    const int row = held ? staged_row(c.flags) : 0;
+    int s_first = row >= 1 ? row : 1, s_park = 0, park_row = -1;
     double pw = NAN;
     if (skip) pw = 0.0;
-    else if (outside(W, F, y)) pw = y[2];
+    else if (!held && outside(W, F, y)) pw = y[2];
+    double K[STAGED ? 7 : 1][9];                           // STAGED: the attempt's stage matrix, saved at a park
     double t = c.t, h_abs = c.h;
     unsigned n_att = c.n_att;
     bool failed = false, rejected = (c.flags & SP_CTL_PENDING) != 0, fresh = !rejected, started = (c.flags & SP_CTL_STARTED) != 0;
@@ -1206,10 +1345,21 @@ SP_HD int dp5x_window(const FieldView<double>& F, const ExtView& X, const Window
     double f[9], yn[9], fn[9];
     for (int i = 0; i < 9; ++i) f[i] = 0.0;
     if (pw != pw) {
-        touched += deriv9<PHASE, AUX64>(F, X, cc, omega, with_phase, y, f);
+        if constexpr (STAGED) {
+            if (held) {
+                for (int j = 0; j < (row > 1 ? row : 1); ++j)
+                    for (int i = 0; i < 9; ++i) K[j][i] = G.get(9 * j + i);
+                for (int i = 0; i < 9; ++i) f[i] = K[0][i];
+            } else {
+                touched += deriv9<PHASE, AUX64>(F, X, cc, omega, with_phase, y, f);
+            }
+        } else {
+            touched += deriv9<PHASE, AUX64>(F, X, cc, omega, with_phase, y, f);
+        }
         if (!started) {
             const double h0 = dp5_initial_step9<PHASE, AUX64, true>(F, X, cc, omega, with_phase, t_end, rtol, atol, y, f, touched, &W, &pw);
             if (pw != pw) { h_abs = h0; started = true; }
+            if constexpr (STAGED) if (pw == pw) park_row = 0;
         }
     }
     for (;;) {
@@ -1221,7 +1371,7 @@ SP_HD int dp5x_window(const FieldView<double>& F, const ExtView& X, const Window
             if (early) {
                 Ray<double> q;
                 for (int k = 0; k < 3; ++k) { q.p[k] = y[k]; q.v[k] = y[3 + k]; }
-                out = escaped(F, q);
+                out = STAGED ? escaped_grid(F, W, q) : escaped(F, q);
             }
             if (out) go = false;
             else {
@@ -1238,7 +1388,14 @@ SP_HD int dp5x_window(const FieldView<double>& F, const ExtView& X, const Window
             const double h = t_new - t;
             h_abs = fabs(h);
             double esq;
-            touched += dp5_attempt9<PHASE, AUX64, true>(F, X, cc, omega, with_phase, h, rtol, atol, y, f, yn, fn, esq, &W, &pw);
+            if constexpr (STAGED) {
+                touched += dp5_attempt9<PHASE, AUX64, true, true>(F, X, cc, omega, with_phase, h, rtol, atol, y, f, yn, fn, esq, &W,
+                                                                  &pw, s_first, &s_park, &K[0][0]);
+                s_first = 1;
+                if (pw == pw) park_row = s_park;
+            } else {
+                touched += dp5_attempt9<PHASE, AUX64, true>(F, X, cc, omega, with_phase, h, rtol, atol, y, f, yn, fn, esq, &W, &pw);
+            }
             if (pw == pw) { h_abs = h_top; fresh = fresh_top; }          // parked: the record as at the top of this iteration
             else {
                 ++n_att;
@@ -1259,6 +1416,12 @@ SP_HD int dp5x_window(const FieldView<double>& F, const ExtView& X, const Window
     if (skip) return touched;
     c.t = t; c.h = h_abs; c.n_att = n_att; c.w_park = pw;
     c.flags = (started ? SP_CTL_STARTED : 0u) | (fresh ? 0u : SP_CTL_PENDING) | (pw != pw ? SP_CTL_FINISHED : 0u) | (failed ? SP_CTL_FAILED : 0u);
+    if constexpr (STAGED) if (pw == pw && park_row >= 0) {
+        c.flags |= SP_CTL_STAGED | ((unsigned)park_row << SP_CTL_ROW_SHIFT);
+        for (int i = 0; i < 9; ++i) G.set(i, f[i]);        // K1 (for the probe: f0)
+        for (int j = 1; j < park_row; ++j)
+            for (int i = 0; i < 9; ++i) G.set(9 * j + i, K[j][i]);
+    }
     return touched;
 }
 

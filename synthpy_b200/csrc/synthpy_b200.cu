@@ -348,6 +348,15 @@ extern "C" int sp_field_export_gradients(const sp_field* f, float* gx_dev, float
 #define SP_METHOD_RK45W 7     // internal: per-ray Dormand-Prince restricted to a window along w (sp_propagate_window)
 #define SP_METHOD_TSIT5W 8    // internal: per-ray Tsit5 restricted to a window along w (sp_propagate_window)
 #define SP_METHOD_RK45XW 9    // internal: RK45X restricted to a window along w (sp_propagate_window_channels, float64)
+#define SP_METHOD_RK45WS 10   // internal: SP_METHOD_RK45W parking between stage evaluations (sp_propagate_window_staged)
+#define SP_METHOD_TSIT5WS 11  // internal: SP_METHOD_TSIT5W parking between stage evaluations
+#define SP_METHOD_RK45XWS 12  // internal: SP_METHOD_RK45XW parking between stage evaluations
+// the methods that resume from the controller record (one slab of an out-of-core solve), and those with a stage store
+__host__ __device__ static constexpr bool windowed_method(int m) {
+    return m == SP_METHOD_RK45W || m == SP_METHOD_TSIT5W || m == SP_METHOD_RK45XW || m == SP_METHOD_RK45WS ||
+           m == SP_METHOD_TSIT5WS || m == SP_METHOD_RK45XWS;
+}
+__host__ __device__ static constexpr bool staged_method(int m) { return m == SP_METHOD_RK45WS || m == SP_METHOD_TSIT5WS || m == SP_METHOD_RK45XWS; }
 #define SP_MAX_OPS 16
 #define SP_MAX_CHANNELS 4
 
@@ -840,26 +849,44 @@ __device__ __noinline__ void rk45x_integrate(const PropArgs<double>& A, Ray<doub
 }
 
 // RK45X restricted to a window (one slab of an out-of-core solve with the channels): ray_core.h dp5x_window on the
-// nine rows, amp and pol read from and written back to the state rows 6 and 8.  Returns the field evaluations.
+// nine rows, amp and pol read from and written back to the state rows 6 and 8.  Returns the field evaluations.  STAGED:
+// stage parking, the ray's stage store at G (rk45xws_integrate).
+template <bool PHASE, bool AUX64, bool STAGED>
+__device__ __forceinline__ int rk45xw_body(const PropArgs<double>& A, const Window W, Ray<double>& r, WinCtl& c, bool early,
+                                           unsigned lanes, uint64_t gi, unsigned& acc, unsigned& capped, double& amp, double& pol,
+                                           StageStore<double> G) {
+    double y[9];
+    for (int k = 0; k < 3; ++k) { y[k] = r.p[k]; y[3 + k] = r.v[k]; }
+    y[6] = A.s0[6 * A.n_total + gi]; y[7] = r.ph; y[8] = A.s0[8 * A.n_total + gi];
+    const unsigned cap = A.n_steps > 0 ? (unsigned)A.n_steps : (1u << 30);
+    const int touched = dp5x_window<PHASE, AUX64, STAGED>(A.F, A.X, W, A.omega, (A.flags & SP_FLAG_PHASE) != 0, A.t_end, A.rtol,
+                                                          A.atol, cap, early, lanes, y, c, acc, capped, G);
+    for (int k = 0; k < 3; ++k) { r.p[k] = y[k]; r.v[k] = y[3 + k]; }
+    r.ph = y[7]; amp = y[6]; pol = y[8];
+    return touched;
+}
 template <bool PHASE, bool AUX64, typename T>
 __device__ __forceinline__ int rk45xw_integrate(const PropArgs<T>& A, const Window W, Ray<T>& r, WinCtl& c, bool early, unsigned lanes,
                                                 uint64_t gi, unsigned& acc, unsigned& capped, double& amp, double& pol) { return 0; }
 template <bool PHASE, bool AUX64>
 __device__ __noinline__ int rk45xw_integrate(const PropArgs<double>& A, const Window W, Ray<double>& r, WinCtl& c, bool early,
                                              unsigned lanes, uint64_t gi, unsigned& acc, unsigned& capped, double& amp, double& pol) {
-    double y[9];
-    for (int k = 0; k < 3; ++k) { y[k] = r.p[k]; y[3 + k] = r.v[k]; }
-    y[6] = A.s0[6 * A.n_total + gi]; y[7] = r.ph; y[8] = A.s0[8 * A.n_total + gi];
-    const unsigned cap = A.n_steps > 0 ? (unsigned)A.n_steps : (1u << 30);
-    const int touched = dp5x_window<PHASE, AUX64>(A.F, A.X, W, A.omega, (A.flags & SP_FLAG_PHASE) != 0, A.t_end, A.rtol, A.atol,
-                                                  cap, early, lanes, y, c, acc, capped);
-    for (int k = 0; k < 3; ++k) { r.p[k] = y[k]; r.v[k] = y[3 + k]; }
-    r.ph = y[7]; amp = y[6]; pol = y[8];
-    return touched;
+    return rk45xw_body<PHASE, AUX64, false>(A, W, r, c, early, lanes, gi, acc, capped, amp, pol, StageStore<double>());
+}
+template <bool PHASE, bool AUX64, typename T>
+__device__ __forceinline__ int rk45xws_integrate(const PropArgs<T>& A, const Window W, Ray<T>& r, WinCtl& c, bool early, unsigned lanes,
+                                                 uint64_t gi, unsigned& acc, unsigned& capped, double& amp, double& pol,
+                                                 StageStore<T> G) { return 0; }
+template <bool PHASE, bool AUX64>
+__device__ __noinline__ int rk45xws_integrate(const PropArgs<double>& A, const Window W, Ray<double>& r, WinCtl& c, bool early,
+                                              unsigned lanes, uint64_t gi, unsigned& acc, unsigned& capped, double& amp, double& pol,
+                                              StageStore<double> G) {
+    return rk45xw_body<PHASE, AUX64, true>(A, W, r, c, early, lanes, gi, acc, capped, amp, pol, G);
 }
 
+// The body of k_propagate and k_propagate_staged: stg is the stage store of the staged methods (nullptr otherwise).
 template <typename T, int METHOD, bool PHASE, bool AUX64>
-__global__ void __launch_bounds__(128, (METHOD == SP_METHOD_RK4 && sizeof(T) == 8) ? SP_RK4_MIN_BLOCKS : (((METHOD == SP_METHOD_RK45 || METHOD == SP_METHOD_RK45B) && sizeof(T) == 8) ? SP_RK45_MIN_BLOCKS : ((METHOD == SP_METHOD_RK4 && sizeof(T) == 4) ? SP_RK4F_MIN_BLOCKS : 1))) k_propagate(const PropArgs<T> A, const Epilogue E) {
+__device__ __forceinline__ void propagate_rays(const PropArgs<T>& A, const Epilogue E, T* stg) {
     const int lane = threadIdx.x & 31;
     const bool early = (A.flags & SP_FLAG_EARLY_EXIT) != 0;
     extern __shared__ double sp_dyn_smem[];     // adaptive methods only: SP_STAGE_DOUBLES values per thread (see StageSmem)
@@ -944,9 +971,10 @@ __global__ void __launch_bounds__(128, (METHOD == SP_METHOD_RK4 && sizeof(T) == 
                 r.ph = y[6];
             } else if (METHOD == SP_METHOD_RK45B) {
                 // handled above (whole-warp path)
-            } else if (METHOD == SP_METHOD_RK45W || METHOD == SP_METHOD_TSIT5W || METHOD == SP_METHOD_RK45XW) {
+            } else if (windowed_method(METHOD)) {
                 // one slab of an out-of-core solve: resume from the record, park at the window (ray_core.h dp5_window)
                 const uint64_t N = A.n_total;
+                StageStore<T> G; G.p = staged_method(METHOD) ? stg + gi : nullptr; G.stride = N;
                 WinCtl c;
                 c.t = E.ctl[gi]; c.h = E.ctl[N + gi]; c.w_park = E.ctl[2 * N + gi]; c.n_att = E.steps[gi]; c.flags = E.ctl_flags[gi];
                 n_att0 = c.n_att;
@@ -957,8 +985,19 @@ __global__ void __launch_bounds__(128, (METHOD == SP_METHOD_RK4 && sizeof(T) == 
                     ls.evals += dp5_window<T, PHASE, AUX64, StageSmem<T> >(A.F, E.win, A.omega, A.t_end, A.rtol, A.atol, A.n_state,
                                                                           (T)A.s0[6 * N + gi], (T)A.s0[8 * N + gi], cap, early, vmask,
                                                                           r, c, S, acc, capped);
+                } else if (METHOD == SP_METHOD_RK45WS) {
+                    const unsigned cap = A.n_steps > 0 ? (unsigned)A.n_steps : (1u << 30);
+                    ls.evals += dp5_window<T, PHASE, AUX64, StageSmem<T>, true>(A.F, E.win, A.omega, A.t_end, A.rtol, A.atol, A.n_state,
+                                                                                (T)A.s0[6 * N + gi], (T)A.s0[8 * N + gi], cap, early,
+                                                                                vmask, r, c, S, acc, capped, G);
                 } else if (METHOD == SP_METHOD_RK45XW) {
                     ls.evals += rk45xw_integrate<PHASE, AUX64>(A, E.win, r, c, early, vmask, gi, acc, capped, amp_x, pol_x);
+                } else if (METHOD == SP_METHOD_RK45XWS) {
+                    ls.evals += rk45xws_integrate<PHASE, AUX64>(A, E.win, r, c, early, vmask, gi, acc, capped, amp_x, pol_x, G);
+                } else if (METHOD == SP_METHOD_TSIT5WS) {
+                    const unsigned cap = A.n_steps > 0 ? (unsigned)A.n_steps : 10000u;
+                    ls.evals += tsit5_window<T, PHASE, AUX64, true>(A.F, E.win, A.omega, A.t_end, A.h, A.rtol, A.atol, A.n_state, cap,
+                                                                    vmask, r, c, acc, capped, G);
                 } else {
                     const unsigned cap = A.n_steps > 0 ? (unsigned)A.n_steps : 10000u;
                     ls.evals += tsit5_window<T, PHASE, AUX64>(A.F, E.win, A.omega, A.t_end, A.h, A.rtol, A.atol, A.n_state, cap, vmask,
@@ -1033,7 +1072,9 @@ __global__ void __launch_bounds__(128, (METHOD == SP_METHOD_RK4 && sizeof(T) == 
         const uint64_t N = A.n_total;
         double amp = 1.0, pol = 0.0;              // constant along the ray (zero derivative): re-read instead of kept live
         if (valid && !A.use_beam) { amp = A.s0[6 * N + gi]; pol = A.s0[8 * N + gi]; }
-        if (METHOD == SP_METHOD_RK4X || METHOD == SP_METHOD_RK45X || METHOD == SP_METHOD_RK45XW) { amp = amp_x; pol = pol_x; }
+        if (METHOD == SP_METHOD_RK4X || METHOD == SP_METHOD_RK45X || METHOD == SP_METHOD_RK45XW || METHOD == SP_METHOD_RK45XWS) {
+            amp = amp_x; pol = pol_x;
+        }
         if (valid) {
             if (E.sf) {
 #pragma unroll
@@ -1060,7 +1101,7 @@ __global__ void __launch_bounds__(128, (METHOD == SP_METHOD_RK4 && sizeof(T) == 
                 E.jf[2 * (N + gi)] = ey_re; E.jf[2 * (N + gi) + 1] = ey_im;
             }
             // windowed methods: rf / jf of a parked ray are overwritten in the launch it finishes in, but it is binned only there
-            const bool done = (METHOD == SP_METHOD_RK45W || METHOD == SP_METHOD_TSIT5W || METHOD == SP_METHOD_RK45XW) ? (valid && fin) : valid;
+            const bool done = windowed_method(METHOD) ? (valid && fin) : valid;
             for (int c = 0; c < E.n_channels; ++c) {
                 const ChannelDev& ch = E.ch[c];
                 DetRay d;
@@ -1085,6 +1126,17 @@ __global__ void __launch_bounds__(128, (METHOD == SP_METHOD_RK4 && sizeof(T) == 
         }
         }
     }
+}
+
+template <typename T, int METHOD, bool PHASE, bool AUX64>
+__global__ void __launch_bounds__(128, (METHOD == SP_METHOD_RK4 && sizeof(T) == 8) ? SP_RK4_MIN_BLOCKS : (((METHOD == SP_METHOD_RK45 || METHOD == SP_METHOD_RK45B) && sizeof(T) == 8) ? SP_RK45_MIN_BLOCKS : ((METHOD == SP_METHOD_RK4 && sizeof(T) == 4) ? SP_RK4F_MIN_BLOCKS : 1))) k_propagate(const PropArgs<T> A, const Epilogue E) {
+    propagate_rays<T, METHOD, PHASE, AUX64>(A, E, nullptr);
+}
+
+// The staged methods (sp_propagate_window_staged): stg is the stage store (ray_core.h, StageStore), in T.
+template <typename T, int METHOD, bool PHASE, bool AUX64>
+__global__ void __launch_bounds__(128, 1) k_propagate_staged(const PropArgs<T> A, const Epilogue E, T* stg) {
+    propagate_rays<T, METHOD, PHASE, AUX64>(A, E, stg);
 }
 
 // ------------------------------------------------------------------------------------------- joint RK45
@@ -1563,16 +1615,29 @@ static int kernel_index_of(const sp_field* f, int caller_axis) {
 }
 
 template <typename T, int METHOD> static constexpr size_t stage_smem_bytes() {
-    return (METHOD == SP_METHOD_RK45 || METHOD == SP_METHOD_RK45B || METHOD == SP_METHOD_RK45W) ? (size_t)SP_STAGE_DOUBLES * 128 * sizeof(T) : 0;
+    return (METHOD == SP_METHOD_RK45 || METHOD == SP_METHOD_RK45B || METHOD == SP_METHOD_RK45W || METHOD == SP_METHOD_RK45WS)
+               ? (size_t)SP_STAGE_DOUBLES * 128 * sizeof(T) : 0;
+}
+
+// one instantiation of k_propagate (k_propagate_staged for the staged methods, with the stage store stg)
+template <typename T, int METHOD, bool PHASE, bool AUX64>
+static void launch_one(const PropArgs<T>& A, const Epilogue& E, T* stg, int grid, size_t sm, cudaStream_t st) {
+    if constexpr (staged_method(METHOD)) k_propagate_staged<T, METHOD, PHASE, AUX64><<<grid, 128, sm, st>>>(A, E, stg);
+    else k_propagate<T, METHOD, PHASE, AUX64><<<grid, 128, sm, st>>>(A, E);
+}
+template <typename T, int METHOD, bool PHASE, bool AUX64> static cudaError_t occupancy_one(int* per_sm, size_t sm) {
+    if constexpr (staged_method(METHOD))
+        return cudaOccupancyMaxActiveBlocksPerMultiprocessor(per_sm, k_propagate_staged<T, METHOD, PHASE, AUX64>, 128, sm);
+    else return cudaOccupancyMaxActiveBlocksPerMultiprocessor(per_sm, k_propagate<T, METHOD, PHASE, AUX64>, 128, sm);
 }
 
 template <typename T, int METHOD>
-static int launch_propagate(const PropArgs<T>& A, const Epilogue& E, int grid, cudaStream_t st) {
+static int launch_propagate(const PropArgs<T>& A, const Epilogue& E, int grid, cudaStream_t st, T* stg = nullptr) {
     const bool phase = (A.flags & SP_FLAG_PHASE) != 0, aux64 = phase && (A.flags & SP_FLAG_PHASE_F64) != 0;
     const size_t sm = stage_smem_bytes<T, METHOD>();
-    if (!phase) k_propagate<T, METHOD, false, false><<<grid, 128, sm, st>>>(A, E);
-    else if (!aux64) k_propagate<T, METHOD, true, false><<<grid, 128, sm, st>>>(A, E);
-    else k_propagate<T, METHOD, true, true><<<grid, 128, sm, st>>>(A, E);
+    if (!phase) launch_one<T, METHOD, false, false>(A, E, stg, grid, sm, st);
+    else if (!aux64) launch_one<T, METHOD, true, false>(A, E, stg, grid, sm, st);
+    else launch_one<T, METHOD, true, true>(A, E, stg, grid, sm, st);
     LAUNCH_CHECK();
     return SP_OK;
 }
@@ -1581,9 +1646,9 @@ template <typename T, int METHOD> static int occupancy_grid(int sm_count, int fl
     int per_sm = 0;
     const bool phase = (flags & SP_FLAG_PHASE) != 0, aux64 = phase && (flags & SP_FLAG_PHASE_F64) != 0;
     const size_t sm = stage_smem_bytes<T, METHOD>();
-    if (!phase) CU(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, k_propagate<T, METHOD, false, false>, 128, sm));
-    else if (!aux64) CU(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, k_propagate<T, METHOD, true, false>, 128, sm));
-    else CU(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, k_propagate<T, METHOD, true, true>, 128, sm));
+    if (!phase) CU((occupancy_one<T, METHOD, false, false>(&per_sm, sm)));
+    else if (!aux64) CU((occupancy_one<T, METHOD, true, false>(&per_sm, sm)));
+    else CU((occupancy_one<T, METHOD, true, true>(&per_sm, sm)));
     if (per_sm < 1) per_sm = 1;
     grid = sm_count * per_sm;
     return SP_OK;
@@ -1596,14 +1661,15 @@ static int joint_solve(const sp_field* field, const sp_params* P, sp_workspace* 
 // run-time flag)
 template <int METHOD> static int ext_grid_of(int sm_count, bool aux64, int& grid) {
     int per_sm = 0;
-    if (aux64) CU(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, k_propagate<double, METHOD, true, true>, 128, 0));
-    else CU(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, k_propagate<double, METHOD, true, false>, 128, 0));
+    if (aux64) CU((occupancy_one<double, METHOD, true, true>(&per_sm, 0)));
+    else CU((occupancy_one<double, METHOD, true, false>(&per_sm, 0)));
     grid = sm_count * (per_sm < 1 ? 1 : per_sm);
     return SP_OK;
 }
-template <int METHOD> static int launch_ext_of(const PropArgs<double>& A, const Epilogue& E, bool aux64, int grid, cudaStream_t st) {
-    if (aux64) k_propagate<double, METHOD, true, true><<<grid, 128, 0, st>>>(A, E);
-    else k_propagate<double, METHOD, true, false><<<grid, 128, 0, st>>>(A, E);
+template <int METHOD> static int launch_ext_of(const PropArgs<double>& A, const Epilogue& E, bool aux64, int grid, cudaStream_t st,
+                                               double* stg = nullptr) {
+    if (aux64) launch_one<double, METHOD, true, true>(A, E, stg, grid, 0, st);
+    else launch_one<double, METHOD, true, false>(A, E, stg, grid, 0, st);
     LAUNCH_CHECK();
     return SP_OK;
 }
@@ -1753,11 +1819,13 @@ extern "C" int sp_propagate(const sp_field* field, const sp_params* P, sp_worksp
     return SP_OK;
 }
 
-// sp_propagate_window (ext = false) and sp_propagate_window_channels (ext = true): one implementation
+// sp_propagate_window (ext = false), sp_propagate_window_channels (ext = true) and, with a stage store (stage_dev non-null),
+// sp_propagate_window_staged: one implementation
 static int propagate_window(bool ext, const sp_field* field, const sp_params* P, sp_workspace* ws, double* state_dev, uint64_t n,
                             const uint32_t* idx_dev, uint64_t n_idx, double* ctl_dev, uint32_t* ctl_flags_dev, uint32_t* steps_dev,
                             double w_lo, double w_hi, double g_lo, double g_hi, double* rf_dev, double* jf_dev,
-                            const sp_channel* channels_host, int n_channels, sp_stats* stats_dev, void* stream) {
+                            const sp_channel* channels_host, int n_channels, sp_stats* stats_dev, void* stream,
+                            double* stage_dev = nullptr) {
     if (!field || !P || !ws) return fail(SP_EINVAL, "null field / params / workspace");
     if (!state_dev || !ctl_dev || !ctl_flags_dev || !steps_dev) return fail(SP_EINVAL, "null state / controller record / steps");
     if (!(w_lo <= w_hi)) return fail(SP_EINVAL, "window needs w_lo <= w_hi");
@@ -1799,8 +1867,11 @@ static int propagate_window(bool ext, const sp_field* field, const sp_params* P,
     }
     const bool fp32 = (P->flags & SP_FLAG_FP32) != 0, tsit = P->method == SP_METHOD_TSIT5;
     const bool ext_aux64 = (P->flags & SP_FLAG_PHASE) && (P->flags & SP_FLAG_PHASE_F64);
+    const bool staged = stage_dev != nullptr;
     int grid = 0, rc;
-    if (ext) rc = ext_grid_of<SP_METHOD_RK45XW>(ws->sm_count, ext_aux64, grid);
+    if (ext) rc = staged ? ext_grid_of<SP_METHOD_RK45XWS>(ws->sm_count, ext_aux64, grid) : ext_grid_of<SP_METHOD_RK45XW>(ws->sm_count, ext_aux64, grid);
+    else if (staged && tsit) rc = fp32 ? occupancy_grid<float, SP_METHOD_TSIT5WS>(ws->sm_count, P->flags, grid) : occupancy_grid<double, SP_METHOD_TSIT5WS>(ws->sm_count, P->flags, grid);
+    else if (staged) rc = fp32 ? occupancy_grid<float, SP_METHOD_RK45WS>(ws->sm_count, P->flags, grid) : occupancy_grid<double, SP_METHOD_RK45WS>(ws->sm_count, P->flags, grid);
     else if (tsit) rc = fp32 ? occupancy_grid<float, SP_METHOD_TSIT5W>(ws->sm_count, P->flags, grid) : occupancy_grid<double, SP_METHOD_TSIT5W>(ws->sm_count, P->flags, grid);
     else rc = fp32 ? occupancy_grid<float, SP_METHOD_RK45W>(ws->sm_count, P->flags, grid) : occupancy_grid<double, SP_METHOD_RK45W>(ws->sm_count, P->flags, grid);
     if (rc) return rc;
@@ -1825,13 +1896,25 @@ static int propagate_window(bool ext, const sp_field* field, const sp_params* P,
         A.extent = (T)P->extent; A.stats = stats_dev;
         rc = ws_event(ws, st);
         if (rc) return rc;
-        if (ext) {
+        if (ext && staged) {
+            FILL(double)
+            A.X = make_ext(field, P->verdet, P->flags);
+            rc = launch_ext_of<SP_METHOD_RK45XWS>(A, E, ext_aux64, g, st, stage_dev);
+        } else if (ext) {
             FILL(double)
             A.X = make_ext(field, P->verdet, P->flags);
             rc = launch_ext_of<SP_METHOD_RK45XW>(A, E, ext_aux64, g, st);
+        } else if (fp32 && staged) {
+            FILL(float)
+            float* sg = reinterpret_cast<float*>(stage_dev);
+            rc = tsit ? launch_propagate<float, SP_METHOD_TSIT5WS>(A, E, g, st, sg) : launch_propagate<float, SP_METHOD_RK45WS>(A, E, g, st, sg);
         } else if (fp32) {
             FILL(float)
             rc = tsit ? launch_propagate<float, SP_METHOD_TSIT5W>(A, E, g, st) : launch_propagate<float, SP_METHOD_RK45W>(A, E, g, st);
+        } else if (staged) {
+            FILL(double)
+            rc = tsit ? launch_propagate<double, SP_METHOD_TSIT5WS>(A, E, g, st, stage_dev)
+                      : launch_propagate<double, SP_METHOD_RK45WS>(A, E, g, st, stage_dev);
         } else {
             FILL(double)
             rc = tsit ? launch_propagate<double, SP_METHOD_TSIT5W>(A, E, g, st) : launch_propagate<double, SP_METHOD_RK45W>(A, E, g, st);
@@ -1859,6 +1942,17 @@ extern "C" int sp_propagate_window_channels(const sp_field* field, const sp_para
                                             void* stream) {
     return propagate_window(true, field, P, ws, state_dev, n, idx_dev, n_idx, ctl_dev, ctl_flags_dev, steps_dev, w_lo, w_hi, g_lo,
                             g_hi, rf_dev, jf_dev, channels_host, n_channels, stats_dev, stream);
+}
+
+extern "C" int sp_propagate_window_staged(const sp_field* field, const sp_params* P, sp_workspace* ws, double* state_dev, uint64_t n,
+                                          const uint32_t* idx_dev, uint64_t n_idx, double* ctl_dev, uint32_t* ctl_flags_dev,
+                                          uint32_t* steps_dev, double* stage_dev, double w_lo, double w_hi, double g_lo, double g_hi,
+                                          double* rf_dev, double* jf_dev, const sp_channel* channels_host, int n_channels,
+                                          sp_stats* stats_dev, void* stream) {
+    if (!stage_dev) return fail(SP_EINVAL, "sp_propagate_window_staged needs a stage store (stage_dev)");
+    const bool ext = P && (P->flags & (SP_FLAG_ATTEN | SP_FLAG_FARADAY)) != 0;
+    return propagate_window(ext, field, P, ws, state_dev, n, idx_dev, n_idx, ctl_dev, ctl_flags_dev, steps_dev, w_lo, w_hi, g_lo,
+                            g_hi, rf_dev, jf_dev, channels_host, n_channels, stats_dev, stream, stage_dev);
 }
 
 // Host controller of the joint solve: a line-for-line counterpart of scipy's RK45._step_impl loop, with the

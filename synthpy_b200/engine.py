@@ -370,14 +370,30 @@ def controller_record(n):
                 flags=torch.zeros(n, dtype=torch.int32, device="cuda"), steps=torch.zeros(n, dtype=torch.int32, device="cuda"))
 
 
+def stage_store(n, params):
+    """Zeroed stage store of ``propagate_window(..., stages=...)`` for n rays solved with ``params``: (values, n) CUDA,
+    float32 with ``FLAG_FP32`` and float64 otherwise, values = ``STAGE_RK45`` (23), ``STAGE_TSIT5`` (42) or, with a channel
+    flag, ``STAGE_RK45X`` (54) -- the layout of sp_propagate_window_staged in include/synthpy_b200.h."""
+    require_cuda()
+    dtype = torch.float32 if params.flags & L.FLAG_FP32 else torch.float64
+    return torch.zeros((_stage_values(params), n), dtype=dtype, device="cuda")
+
+
+def _stage_values(params):
+    if params.flags & (L.FLAG_ATTEN | L.FLAG_FARADAY):
+        return L.STAGE_RK45X
+    return L.STAGE_TSIT5 if params.method == L.METHOD_TSIT5 else L.STAGE_RK45
+
+
 def propagate_window(field, params, state, record, w_lo, w_hi, grid_range, *, idx=None, rf=None, jf=None, channels=(),
-                     stats=None):
+                     stats=None, stages=None):
     """One call of ``sp_propagate_window``: advance the rays ``idx`` (int32 CUDA tensor of indices, None = all) of the
     (9, N) CUDA float64 ``state`` in place, each until it finishes or parks at the window [w_lo, w_hi] of the probing
     axis (``grid_range``: the whole grid's extent along it).  With a channel flag in ``params`` (attenuation / Faraday, RK45
     only) this is ``sp_propagate_window_channels``: amp and pol (rows 6, 8) are integrated too, and ``field`` needs the
     grids (``attach_channels``).  ``record`` from ``controller_record``; ``rf`` (4, N) / ``jf`` (2, N) complex128 receive the rays that finish;
-    ``stats`` an int64 (6,) CUDA tensor accumulated into.  No sync."""
+    ``stats`` an int64 (6,) CUDA tensor accumulated into.  With ``stages`` (from ``stage_store``) this is
+    ``sp_propagate_window_staged``: rays park between stage evaluations and keep their attempt in progress there.  No sync."""
     require_cuda()
     if not (isinstance(state, torch.Tensor) and state.is_cuda and state.dtype == torch.float64 and state.is_contiguous()
             and state.ndim == 2 and state.shape[0] == 9):
@@ -393,6 +409,17 @@ def propagate_window(field, params, state, record, w_lo, w_hi, grid_range, *, id
         structs.append(ch)
         keep.append(k)
     ch_arr = (L.Channel * max(1, len(structs)))(*structs)
+    if stages is not None:
+        dtype = torch.float32 if params.flags & L.FLAG_FP32 else torch.float64
+        if not (isinstance(stages, torch.Tensor) and stages.is_cuda and stages.dtype == dtype and stages.is_contiguous()
+                and tuple(stages.shape) == (_stage_values(params), n)):
+            raise TypeError("stages must be the contiguous CUDA tensor of stage_store(n, params) for this state")
+        L.check(L.lib.sp_propagate_window_staged(field._h, C.byref(params), workspace(), _ptr(state), n, _ptr(idx),
+                                                 0 if idx is None else idx.numel(), _ptr(record["ctl"]), _ptr(record["flags"]),
+                                                 _ptr(record["steps"]), _ptr(stages), float(w_lo), float(w_hi),
+                                                 float(grid_range[0]), float(grid_range[1]), _ptr(rf), _ptr(jf), ch_arr,
+                                                 len(structs), _ptr(stats), _stream()))
+        return
     fn = L.lib.sp_propagate_window_channels if params.flags & (L.FLAG_ATTEN | L.FLAG_FARADAY) else L.lib.sp_propagate_window
     L.check(fn(field._h, C.byref(params), workspace(), _ptr(state), n, _ptr(idx),
                                       0 if idx is None else idx.numel(), _ptr(record["ctl"]), _ptr(record["flags"]),

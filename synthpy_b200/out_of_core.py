@@ -11,7 +11,10 @@ that nothing about the result depends on it:
   * the per-ray adaptive solves (method='rk45', 'tsit5'; ``trace_slabs_adaptive`` over ``sp_propagate_window``): a ray
     parks when its next attempt would evaluate the field inside the grid but outside the slab's window, with its
     controller record as at the top of that loop iteration, and resumes in a later slab; every committed attempt is the
-    in-core arithmetic (see ray_core.h dp5_window).  Joint and bundle-step RK45 stay in core;
+    in-core arithmetic (see ray_core.h dp5_window).  With ``park='stage'`` (``sp_propagate_window_staged``) a ray parks
+    between stage evaluations instead, its attempt in progress kept in a per-ray stage store, so a window only has to
+    hold the next point it evaluates: fixed-size slabs then serve SciPy's box-sized first attempts too, without growing,
+    and every evaluation runs once, as in core.  Joint and bundle-step RK45 stay in core;
   * a slab holds the planes [a, b] of the probing axis.  The float32 gradient stencil (field_prep.h) at plane k reads
     planes k-1 and k+1, so the edge planes of a slab carry one-sided differences that the whole grid would not: the
     planner keeps every RK stage of every live ray at least two planes inside (``plan_slab``), checks it afterwards on
@@ -326,14 +329,16 @@ def trace_slabs(backend, s0, source, axes, probing_direction, n_steps, h, slab_p
 
 
 class _AdaptiveDeviceBackend:
-    """The product path of the adaptive solves: packed slab field in HBM, ``sp_propagate_window`` per slab."""
+    """The product path of the adaptive solves: packed slab field in HBM, ``sp_propagate_window`` per slab
+    (``sp_propagate_window_staged`` with ``park='stage'``)."""
 
-    def __init__(self, params, lwl, probing_direction, phase, phase_f64, want_jf):
+    def __init__(self, params, lwl, probing_direction, phase, phase_f64, want_jf, park="attempt"):
         import torch
         self.torch, self.P, self.lwl, self.phase, self.phase_f64 = torch, params, lwl, phase, phase_f64
         self.p = engine.AXIS[probing_direction]
-        self.want_jf = want_jf
+        self.want_jf, self.staged = want_jf, park == "stage"
         self.stats = torch.zeros(6, dtype=torch.int64, device="cuda")
+        self.stages = None
 
     def to_state(self, s0):
         s = engine.to_device(s0, self.torch.float64)
@@ -345,18 +350,25 @@ class _AdaptiveDeviceBackend:
         rec["ctl"][2].fill_(np.inf)
         self.rf = t.empty((4, n), dtype=t.float64, device="cuda")
         self.jf = t.empty((2, n), dtype=t.complex128, device="cuda") if self.want_jf else None
+        if self.staged:
+            self.stages = engine.stage_store(n, self.P)
         return rec
+
+    def _needed(self, s, rec):
+        """Stage parking: the point a ray needs next -- where it parked, or its position before its first launch."""
+        w = rec["ctl"][2]
+        return self.torch.where(self.torch.isfinite(w), w, s[self.p])
 
     def slowest(self, s, rec):
         todo = (rec["flags"] & engine.L.CTL_FINISHED) == 0
         if not bool(todo.any()):
             return None
-        z = self.torch.minimum(s[self.p][todo], rec["ctl"][2][todo])
+        z = self._needed(s, rec)[todo] if self.staged else self.torch.minimum(s[self.p][todo], rec["ctl"][2][todo])
         z = z[self.torch.isfinite(z)]
         return float(z.min()) if z.numel() else -np.inf
 
     def select(self, s, rec, w_lo, w_hi):
-        w = s[self.p]
+        w = self._needed(s, rec) if self.staged else s[self.p]
         ok = ((rec["flags"] & engine.L.CTL_FINISHED) == 0) & ~(w < w_lo) & ~(w > w_hi)      # NaN positions are inside
         return self.torch.nonzero(ok).squeeze(1).to(self.torch.int32)
 
@@ -364,16 +376,20 @@ class _AdaptiveDeviceBackend:
         f, c = rec["flags"][idx.long()], rec["ctl"][:, idx.long()]
         L = engine.L
         parked = (f & L.CTL_FINISHED) == 0
-        return dict(attempts=int(rec["steps"].sum()), finished=int(((rec["flags"] & L.CTL_FINISHED) != 0).sum()),
-                    pending=int((parked & ((f & L.CTL_PENDING) != 0)).sum()),
-                    clip=int((parked & (c[0] + c[1] - t_stop > 0)).sum()))
+        out = dict(attempts=int(rec["steps"].sum()), finished=int(((rec["flags"] & L.CTL_FINISHED) != 0).sum()),
+                   pending=int((parked & ((f & L.CTL_PENDING) != 0)).sum()),
+                   clip=int((parked & (c[0] + c[1] - t_stop > 0)).sum()))
+        if self.staged:
+            mid = parked & ((f & L.CTL_STAGED) != 0) & (((f >> L.CTL_ROW_SHIFT) & 15) >= 1)
+            out.update(evals=int(self.stats[5]), mid=int(mid.sum()))
+        return out
 
     def field(self, ne_slab, axes):
         return _field_of(self, ne_slab, axes)
 
     def launch(self, field, s, rec, idx, w_lo, w_hi, grid_range, channels):
         engine.propagate_window(field, self.P, s, rec, w_lo, w_hi, grid_range, idx=idx, rf=self.rf, jf=self.jf, channels=channels,
-                                stats=self.stats)
+                                stats=self.stats, stages=self.stages)
 
     def release(self, field):
         self.torch.cuda.current_stream().synchronize()
@@ -382,7 +398,7 @@ class _AdaptiveDeviceBackend:
 
 
 def trace_slabs_adaptive(backend, s0, source, axes, probing_direction, slab_planes, t_stop, *, max_slab_planes=None,
-                         channels=()):
+                         channels=(), park="attempt"):
     """The slab loop of the adaptive solves (``backend``: the device, or the host build of the same ray code in the tests).
     Each pass loads the slab from MARGIN planes behind the slowest unfinished ray (or the lowest point a parked ray needs)
     and launches once over the unfinished rays inside its window; a ray runs until it finishes or parks at the window, and
@@ -396,7 +412,20 @@ def trace_slabs_adaptive(backend, s0, source, axes, probing_direction, slab_plan
     the window.  The slab then doubles, up to ``max_slab_planes`` (default ``slab_planes``: no growth), and returns to
     ``slab_planes`` after the next launch that makes progress.  SciPy's initial step is one such attempt: 100 h0 is of
     the order of the distance from the origin, so the first (rejected) attempts of RK45 span much of the box.  A second
-    launch without progress at the largest slab raises ``ValueError`` instead of looping."""
+    launch without progress at the largest slab raises ``ValueError`` instead of looping.
+
+    ``park='stage'`` (a backend built for it: ``sp_propagate_window_staged``): rays park between stage evaluations and carry
+    their attempt in progress in a stage store, so a window only has to hold the NEXT point a ray evaluates -- where it
+    parked, or its position before its first launch (the ray's needed point).  ``slowest`` and ``select`` go by the needed
+    point, and the window starts MARGIN planes behind the lowest one, so every launch evaluates at least that point: the
+    slab never grows (``max_slab_planes`` is refused).  Each slab's log adds the field evaluations ('evals') and the rays
+    parked mid-attempt ('parked_mid').  Two launches in a row that neither evaluate, commit nor finish anything raise
+    ``RuntimeError`` (the first launch can evaluate only points outside the grid, which are not counted)."""
+    if park not in ("attempt", "stage"):
+        raise ValueError(f"park must be 'attempt' or 'stage', not {park!r}")
+    staged = park == "stage"
+    if staged and max_slab_planes is not None:
+        raise ValueError("park='stage' never grows the slab: max_slab_planes does not apply")
     p = engine.AXIS[probing_direction]
     zc = np.asarray(np.float32(axes[p]), dtype=np.float64)
     n = len(zc)
@@ -426,6 +455,14 @@ def trace_slabs_adaptive(backend, s0, source, axes, probing_direction, slab_plan
         done, att = after["finished"] - before["finished"], after["attempts"] - before["attempts"]
         log.append(dict(planes=(a, b), window=(w_lo, w_hi), launched=len(idx), finished=done, parked=len(idx) - done,
                         parked_pending=after["pending"], parked_clip=after["clip"], attempts=att, field_bytes=nbytes))
+        if staged:
+            evals = after["evals"] - before["evals"]
+            log[-1].update(evals=evals, parked_mid=after["mid"])
+            stalls = 0 if (evals > 0 or att > 0 or done > 0) else stalls + 1
+            if stalls >= 2:
+                raise RuntimeError(f"stage parking: two launches over the window ({w_lo:.4g} .. {w_hi:.4g} m) evaluated "
+                                   "nothing although it holds the lowest point a ray needs")
+            continue
         # Nothing committed and nothing finished: the state is what it was, so the next window is this one or (once) the
         # one that holds the point a ray parked at below it.  Grow the slab; at the largest, a second such launch means an
         # attempt wider than the window.
@@ -445,7 +482,7 @@ def solve_out_of_core(s0_import, source, lengths, dims, probing_depth, *, slab_p
                       return_E=False, phaseshift=False, phase_f64=False, n_steps=None, ds=None, sort=True,
                       axis_convention="current", diagnostics=(), return_state=False, prefetch=False, method="rk4",
                       rtol=None, atol=None, max_steps=None, precision="fp64", early_exit=True, save_steps=2,
-                      max_slab_planes=None, inv_brems=False, B_on=False, B=None, Te=None, Z=None):
+                      max_slab_planes=None, inv_brems=False, B_on=False, B=None, Te=None, Z=None, park="attempt"):
     """``propagator.solve(..., method=...)`` for a grid delivered in slabs of ``slab_planes`` planes of the probing axis
     by ``source(k0, k1)``.  ``lengths`` / ``dims`` describe the whole grid as ``ScalarDomain`` takes them (axes
     ``linspace(-L/2, L/2, n)`` rounded to float32).  Same outputs as ``solve``: ``(rf, Jf, duration)`` (+ a dict with
@@ -465,8 +502,14 @@ def solve_out_of_core(s0_import, source, lengths, dims, probing_depth, *, slab_p
     per point), ``Te`` and ``Z`` is an array-like over the whole grid (NumPy, memmap, CUDA tensor; sliced along the probing
     axis) or a slab callable ``f(k0, k1)`` like ``source``; ``Te`` and ``Z`` may be scalars (``channel_source``).  With
     the channels, RK4 and RK45 ('rk4', 'rk45') in float64; Tsit5 does not integrate them, in core or out of core.  RK45
-    with the channels saves memory only when ``max_slab_planes`` covers SciPy's first attempts, which span about half the
-    box (DESIGN.md section 6)."""
+    with ``park='attempt'`` saves memory only when ``max_slab_planes`` covers SciPy's first attempts, which span about half
+    the box (DESIGN.md section 6).
+
+    ``park`` (adaptive solves): 'attempt' (default) parks a ray a whole attempt at a time, so a window must hold the ray and
+    every stage point of its next attempt (the slab grows up to ``max_slab_planes``); 'stage' parks it between stage
+    evaluations with the attempt in progress kept in a per-ray stage store on the device (184 B per ray for RK45, 336 B
+    for Tsit5, 432 B with the channels), so slabs of ``slab_planes`` planes serve every ray and the slab never grows --
+    the same results, bit for bit, and the in-core evaluation count."""
     import torch
     from . import propagator
     if method in ("rk45_joint", "rk45_bundle"):
@@ -474,6 +517,12 @@ def solve_out_of_core(s0_import, source, lengths, dims, probing_depth, *, slab_p
                          "bundle of rays; use 'rk45' (per ray), 'tsit5' or 'rk4'")
     if method not in ("rk4", "rk45", "tsit5"):
         raise ValueError(f"unknown method {method!r}")
+    if park not in ("attempt", "stage"):
+        raise ValueError(f"park must be 'attempt' or 'stage', not {park!r}")
+    if park == "stage" and method == "rk4":
+        raise ValueError("park='stage' is for the adaptive solves ('rk45', 'tsit5'): RK4 never parks mid-step")
+    if park == "stage" and max_slab_planes is not None:
+        raise ValueError("park='stage' never grows the slab: max_slab_planes does not apply")
     if method == "rk4" and (precision != "fp64" or not early_exit):
         raise ValueError("out-of-core RK4 runs in float64 with early exit (precision='fp64', early_exit=True)")
     inv_brems, B_on = bool(inv_brems), bool(B_on)
@@ -489,7 +538,7 @@ def solve_out_of_core(s0_import, source, lengths, dims, probing_depth, *, slab_p
                                phase_f64=phase_f64, axis_convention=axis_convention, diagnostics=diagnostics,
                                return_state=return_state, prefetch=prefetch, method=method, rtol=rtol, atol=atol,
                                max_steps=max_steps, precision=precision, early_exit=early_exit, save_steps=save_steps,
-                               sort=sort, max_slab_planes=max_slab_planes, atten=inv_brems, faraday=B_on)
+                               sort=sort, max_slab_planes=max_slab_planes, atten=inv_brems, faraday=B_on, park=park)
     lengths, dims, axes = _grid_axes(lengths, dims)
     extent = float(probing_depth)
     t_end = np.sqrt(8.0) * extent / C_LIGHT
@@ -578,7 +627,8 @@ def _grid_axes(lengths, dims):
 
 def _solve_adaptive(s0_import, source, lengths, dims, probing_depth, *, slab_planes, probing_direction, lwl, return_E,
                     phaseshift, phase_f64, axis_convention, diagnostics, return_state, prefetch, method, rtol, atol,
-                    max_steps, precision, early_exit, save_steps, sort, max_slab_planes, atten=False, faraday=False):
+                    max_steps, precision, early_exit, save_steps, sort, max_slab_planes, atten=False, faraday=False,
+                    park="attempt"):
     import torch
     from . import propagator
     lengths, dims, axes = _grid_axes(lengths, dims)
@@ -588,7 +638,7 @@ def _solve_adaptive(s0_import, source, lengths, dims, probing_depth, *, slab_pla
     P = propagator._solver_params(probing_direction, float(lengths[pa]) / (int(dims[pa]) - 1), atten, faraday, probing_depth,
                                   lwl, method, None, None, rtol, atol, precision, early_exit, phase, phase_f64, sort,
                                   axis_convention, max_steps, save_steps)
-    backend = _AdaptiveDeviceBackend(P, lwl, probing_direction, phase, phase_f64, return_E)
+    backend = _AdaptiveDeviceBackend(P, lwl, probing_direction, phase, phase_f64, return_E, park=park)
     chans = [(d.ops, d.image, d.wavelength if d.wavelength else lwl) for d in diagnostics]
     as_numpy = not isinstance(s0_import, torch.Tensor)
     if prefetch:
@@ -598,7 +648,7 @@ def _solve_adaptive(s0_import, source, lengths, dims, probing_depth, *, slab_pla
     try:
         sf, rec, log = trace_slabs_adaptive(backend, s0_import, source, axes, probing_direction, slab_planes,
                                             1.0 if method == "tsit5" else P.t_end, max_slab_planes=max_slab_planes,
-                                            channels=chans)
+                                            channels=chans, park=park)
     finally:
         _close(source)
     torch.cuda.synchronize()
